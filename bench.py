@@ -57,6 +57,30 @@ def bytes_per_solve(n, m, N):
     return 4 * (n + n * N + m * (N - 1)) + 4 * (n * N + m * (N - 1)) + 8
 
 
+DUMP_PROBLEMS = 1 << 16      # --dump-outputs sample: 2^16 problems of the largest shape (quadrotor) are 41 MB of float32
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, outputs, B):
+    """Writes the per-problem outputs of a step (dict name -> device tensor with the problem index first) as
+    out_dir/<name>.npy in float32, restricted to a fixed sample of the batch: every problem up to DUMP_PROBLEMS, otherwise
+    DUMP_PROBLEMS indices drawn with seed 0, in increasing order.  Iteration counts and status codes are exact in float32."""
+    import torch
+    if B <= DUMP_PROBLEMS:
+        idx = np.arange(B)
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(B, DUMP_PROBLEMS, replace=False))
+    arrays = {}
+    for name, t in outputs.items():
+        arrays[name] = t[torch.from_numpy(idx).to(t.device)].to(torch.float32).cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs: {total} bytes exceed {DUMP_MAX_BYTES}"
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", a)
+
+
 def fp32_peak_tflops():
     """FP32 CUDA-core peak: measured by profiles/microbench/ffma_bench.cu on this pool (see
     profiles/microbench/RESULTS.md); MEASURED_PEAKS.json carries no FP32 figure."""
@@ -227,7 +251,12 @@ def main():
     ap.add_argument("--order", type=int, default=-1, help="option order of the library (claim the hardest problems first); -1 = library default (1), 0 = index order")
     ap.add_argument("--e2e-mode", dest="e2e_mode", default="compact", choices=["compact", "full"],
                     help="I/O mode of the headline end-to-end number (the other one is reported as e2e_other)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write x, u, iter and status of the last one as DIR/<name>.npy (float32) for a fixed sample "
+                         f"of at most {DUMP_PROBLEMS} problems of rank 0's shard, so that two builds can be compared on identical inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3   # timing rule: at least 3 warm-up steps
 
@@ -352,6 +381,8 @@ def main():
     marked = solver.cuda.last_marked if band > 0 else 0
     iters_one = int(it.sum().item())                 # identical every step (same inputs)
     unsolved = float((st == 11).float().mean().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"x": x, "u": u, "iter": it, "status": st}, B)
     ms_all, (iters_all, launches_all) = S.reduce_report(ms, [iters_one, launches], dist, dev)   # max of times, sum of work
     launches_all = int(launches_all)
     value = world * B * args.steps / (ms_all * 1e-3)
