@@ -181,7 +181,7 @@ int  tinympc_cuda_session_set_u_ref(tinympc_cuda_session *ss, const double *Uref
 /* tiny_solve on every solver, warm start (tiny_api.cpp:321-323 -> admm.cpp:274-389) */
 int  tinympc_cuda_session_solve(tinympc_cuda_session *ss);
 /* x0 <- Adyn x0 + Bdyn u0 + fdyn on the device; u0 = work->u.col(0) (use_solution 0, quadrotor_hovering.cpp:91) or
- * solution->u.col(0) (use_solution 1, cartpole_example_mpc.m:40-41) */
+ * solution->u.col(0) (use_solution 1, cartpole_example_mpc.m:40-41).  TINYMPC_CUDA_EUNSUPPORTED for nx > 32, x0 untouched. */
 int  tinympc_cuda_session_step(tinympc_cuda_session *ss, int use_solution);
 /* read one member of every solver into host memory (doubles; iter/status as doubles too):
  * "x0" batch*nx | "x", "sol_x" batch*nx*N (work->x, solution->x) | "u", "sol_u" batch*nu*(N-1) |

@@ -1730,16 +1730,17 @@ int tinympc_cuda_session_step(tinympc_cuda_session* ss, int use_solution) {
     if (!ss) return TINYMPC_CUDA_EINVAL;
     tinympc_cuda_solver* s = ss->s;
     if (!s) return TINYMPC_CUDA_ENOTREADY;   // the solver was destroyed under the session
+    if (ss->fam.nx > 32)                     // the step kernel gives each state row one lane of a warp
+        return fail(s, TINYMPC_CUDA_EUNSUPPORTED, "session step needs nx <= 32 (one lane per state); the session has nx = " +
+                                                      std::to_string(ss->fam.nx));
     DeviceCtx& d = s->devs[ss->dev];
-    int prev = 0;
-    cudaGetDevice(&prev);
+    DeviceGuard guard;                       // restores the caller's current device on every return path
     CU(s, cudaSetDevice(d.device));
     cudaStream_t st = d.streams[0];
     CU(s, ss->bits == 64 ? wpp_session_step<double>(ss->fam.L, ss->pack.p, ss->W, ss->ws.p, ss->batch, use_solution, st)
                          : wpp_session_step<float>(ss->fam.L, ss->pack.p, ss->W, ss->ws.p, ss->batch, use_solution, st));
     s->launches += 1;
     CU(s, cudaStreamSynchronize(st));
-    cudaSetDevice(prev);
     return TINYMPC_CUDA_OK;
 }
 

@@ -238,7 +238,6 @@ extern "C" int tinympc_cuda_precompute_batch(const tinympc_cuda_precompute_in* i
     const size_t smem = sizeof(double) * WarpMem::size(nx, nu) * warps_per_cta;
     cudaFuncSetAttribute(precompute_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     int sms = 0;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, 0);
     int dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -247,8 +246,8 @@ extern "C" int tinympc_cuda_precompute_batch(const tinympc_cuda_precompute_in* i
     ok(cudaGetLastError());
     ok(cudaDeviceSynchronize());
     if (e != cudaSuccess) return TINYMPC_CUDA_ECUDA;
-    // back to the host, column-major per problem
-    double* h = new double[B * nxx];
+    // back to the host, column-major per problem; the staging buffer holds the largest block fetched (nu x nx or nu x nu when nu > nx)
+    double* h = new double[B * std::max({nxx, nxu, nuu})];
     auto fetch = [&](const Dev& d, double* dst, int rows, int cols) {
         if (!dst) return;
         ok(cudaMemcpy(h, d.p, sizeof(double) * B * rows * cols, cudaMemcpyDeviceToHost));
