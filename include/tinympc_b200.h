@@ -125,6 +125,37 @@ int  tinympc_cuda_solve_batch(tinympc_cuda_solver *s, const tinympc_cuda_batch_i
 int  tinympc_cuda_solve_batch_device(tinympc_cuda_solver *s, int dev_index, const tinympc_cuda_batch_in *in,
                                      const tinympc_cuda_batch_out *out, void *stream);
 
+/* ---- batches in which every problem brings its own model ---------------------------------------- */
+/* Per-problem models: double, one contiguous COLUMN-MAJOR chunk per problem (the layout of tinympc_cuda_family and of
+ * tinympc_cuda_precompute_out, so precompute results plug in unchanged).  HOST pointers for _solve_batch_models, DEVICE
+ * pointers (16-byte aligned) for _solve_batch_models_device. */
+typedef struct {
+    const double *Adyn, *Bdyn;            /* batch*nx*nx, batch*nx*nu */
+    const double *fdyn;                   /* batch*nx or NULL = 0 */
+    const double *Q, *R;                  /* batch*nx, batch*nu: work->Q, work->R (diag + rho), exactly as tinympc_cuda_family */
+    const double *rho;                    /* batch: cache->rho */
+    const double *Kinf, *Pinf, *Quu_inv, *AmBKt;   /* batch*(nu*nx | nx*nx | nu*nu | nx*nx) */
+    const double *APf, *BPf;              /* batch*nx, batch*nu, or NULL = 0 */
+    const double *dKinf_drho, *dPinf_drho;   /* batch*(nu*nx | nx*nx); required when the family has adaptive_rho */
+} tinympc_cuda_models;
+/* replaces a loop of { tiny_setup(A_b, B_b, Q_b, R_b, rho_b); tiny_set_x0; tiny_set_x_ref; tiny_set_u_ref; tiny_solve } over
+ * `batch` solvers whose models differ.  The family set by tinympc_cuda_set_family still supplies nx, nu, N, the settings, the
+ * shared bounds, the cones, the linear rows and the adaptive-rho flags; its matrices and cache are not read.  Each problem gets a
+ * cold start with ITS OWN model and pristine cache, i.e. what a fresh tiny_setup with that model produces.  Per-problem bounds,
+ * compact I/O (xref_const, u0), residuals and rho work as in tinympc_cuda_solve_batch.
+ * The host entry shards contiguously over the solver's devices like tinympc_cuda_solve_batch and runs the chunked H2D -> kernel
+ * -> D2H pipeline, the model arrays of each chunk travelling with its inputs; the streamed pipeline, the compact launch chain and
+ * the claim order (option "order") do not apply to model batches.  The device entry has the rule of
+ * tinympc_cuda_solve_batch_device: ONE call in flight per (solver, dev_index).
+ * Kernels: with "precision" 64, a box family without adaptive rho, shared bounds and a shape that has a compiled lane-group fp64
+ * kernel, its model form; otherwise the warp-per-problem kernel in the arithmetic "precision" selects.  The exact-count mode
+ * ("precision" 32 with "mixed" > 0) has no model form: TINYMPC_CUDA_EUNSUPPORTED ("precision" 64 is exact for model batches).
+ * A missing required array, adaptive rho without the two sensitivities or (device entry) a misaligned pointer: TINYMPC_CUDA_EINVAL. */
+int  tinympc_cuda_solve_batch_models(tinympc_cuda_solver *s, const tinympc_cuda_models *m, const tinympc_cuda_batch_in *in,
+                                     const tinympc_cuda_batch_out *out);
+int  tinympc_cuda_solve_batch_models_device(tinympc_cuda_solver *s, int dev_index, const tinympc_cuda_models *m,
+                                            const tinympc_cuda_batch_in *in, const tinympc_cuda_batch_out *out, void *stream);
+
 /* Full-workspace solve of ONE problem with the reference's warm-start semantics: replaces
  * tiny_solve(solver) on a live TinySolver (tiny_api.cpp:321-323 -> admm.cpp:274-389).  All arrays are HOST,
  * column-major double, exactly the TinyWorkspace members (types.hpp:92-160); the solve starts from whatever

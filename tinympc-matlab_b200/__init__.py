@@ -178,12 +178,15 @@ class TinyMPC:
         return u0
 
     # ------------------------------------------------------------------ NEW: batched entry point
-    def solve_batch(self, X0, Xref=None, Uref=None, x_min=None, x_max=None, u_min=None, u_max=None):
+    def solve_batch(self, X0, Xref=None, Uref=None, x_min=None, x_max=None, u_min=None, u_max=None, models=None):
         """Solve B independent problems of this family that differ in x0 / references / bounds (cold start each).
 
         MATLAB shapes: X0 nx x B; Xref nx x N x B (or nx x N / nx x 1: shared, expanded like set_x_ref); Uref likewise;
         optional per-problem bounds nx x N x B / nu x (N-1) x B.  Returns dict(states nx x N x B, controls nu x (N-1) x B,
         iter B, status B, residuals 4 x B, rho B).
+        models: every problem's own dynamics, costs and cache (the dict of capi.pack_models, e.g. capi.precompute_batch's
+        output merged with A, B, f, Q, R, rho), as a loop of setup + solve over solvers with different models would use them;
+        this object then supplies the horizon, settings and constraints only.
         """
         self._check_setup()
         X0 = np.asarray(X0, np.float64)
@@ -208,7 +211,11 @@ class TinyMPC:
         out = dict(x=np.empty((B, N, nx), np.float32), u=np.empty((B, N - 1, nu), np.float32), iter=np.empty(B, np.int32),
                    status=np.empty(B, np.int32), residuals=np.empty((B, 4), np.float32), rho=np.empty(B, np.float32))
         co = capi.CBatchOut(*[out[k].ctypes.data for k in ("x", "u", "iter", "status", "residuals", "rho")])
-        rc = self._L.tinympc_host_solve_batch(self._h, C.byref(cin), C.byref(co))
+        if models is None:
+            rc = self._L.tinympc_host_solve_batch(self._h, C.byref(cin), C.byref(co))
+        else:
+            arrays = capi.pack_models(models, B, nx, nu)
+            rc = self._L.tinympc_host_solve_batch_models(self._h, C.byref(capi.models_struct(arrays)), C.byref(cin), C.byref(co))
         if rc:
             raise TinympcCudaError(rc, self._L.tinympc_host_last_error(self._h).decode())
         return dict(states=np.transpose(out["x"], (2, 1, 0)).astype(np.float64), controls=np.transpose(out["u"], (2, 1, 0)).astype(np.float64),

@@ -97,12 +97,14 @@ def inst4(nx, nu, N, refs=True, fb=False, variant=0, aff=None, cones=(0, 0, 0, 0
                 opq=False, tib=False, tm=True, minb=1, ntm=0, cones=cones, ttm=-1)
 
 
-def instg(nx, nu, N, variant=0, adapt=False, cones=None, rolled=False):
-    """lane-group-per-problem fp64 kernel (tmpc_gpp.cuh): one lane per state row and per input row, groups of 8 / 16 / 32 lanes"""
+def instg(nx, nu, N, variant=0, adapt=False, cones=None, rolled=False, models=False):
+    """lane-group-per-problem fp64 kernel (tmpc_gpp.cuh): one lane per state row and per input row, groups of 8 / 16 / 32 lanes;
+    models: its model-batch form (gen 6, box only: gpp_kernel MODE 3), whose rows come from each problem's own model"""
     gs = 8 if nx + nu <= 8 else (16 if nx + nu <= 16 else 32)
     assert nx + nu <= 32
-    return dict(gen=5, bits=64, nx=nx, nu=nu, N=N, feat=CON if cones else (ADP if adapt else BOX), refs=2, ppb=False, fb=False, variant=variant, block=128,
-                aff=True, gs=gs, cones=cones, rolled=rolled)
+    assert not (models and (adapt or cones))
+    return dict(gen=6 if models else 5, bits=64, nx=nx, nu=nu, N=N, feat=CON if cones else (ADP if adapt else BOX), refs=2, ppb=False, fb=False,
+                variant=variant, block=128, aff=True, gs=gs, cones=cones, rolled=rolled)
 
 
 def cols_per_thread(nx, nu, N, feat, refs, ntm=0):
@@ -175,6 +177,9 @@ def default_instances():
     for (nx, nu, N) in shapes:
         out.append(instg(nx, nu, N))
     out.append(instg(12, 4, 10, adapt=True))     # adaptive rho: the fp64 path of BASELINE config 5
+    # model batches (tinympc_cuda_solve_batch_models) of fp64 box families with shared bounds: every problem its own model
+    for (nx, nu, N) in shapes:
+        out.append(instg(nx, nu, N, models=True))
     # rocket family (one cone per side, with and without the two linear rows): fp64 batches and the second pass of its exact-count mode
     out.append(instg(6, 3, 10, cones=(0, 3, 0, 3, 1, 1)))
     out.append(instg(6, 3, 10, cones=(0, 3, 0, 3, 0, 0)))
@@ -213,9 +218,9 @@ def default_instances():
 
 def name_of(i):
     t = "f32" if i["bits"] == 32 else "f64"
-    if i["gen"] == 5:
+    if i["gen"] in (5, 6):
         cn = ("_c" + "".join(str(c) for c in i["cones"])) if i.get("cones") else ""
-        return f"gpp_f64_{i['nx']}x{i['nu']}x{i['N']}_{FEAT_NAME[i['feat']]}{cn}_g{i['gs']}_v{i['variant']}"
+        return f"gpp_f64_{i['nx']}x{i['nu']}x{i['N']}_{FEAT_NAME[i['feat']]}{cn}_g{i['gs']}_v{i['variant']}{'_mdl' if i['gen'] == 6 else ''}"
     if i["gen"] == 4:
         cn = "_c" + "".join(str(c) for c in i["cones"])
         return f"tpp4_mix_{i['nx']}x{i['nu']}x{i['N']}_con{cn}{'' if i['refs'] else '_noref'}{'_fb' if i['fb'] else ''}{'_aff' if i['aff'] else ''}_v{i['variant']}"
@@ -244,6 +249,15 @@ def gen_sources(instances):
                 f"using Cfg_{n} = GppCfg<{i['nx']}, {i['nu']}, {i['N']}, {i['gs']}, {i['block']}, {b(i['feat'] == ADP)}"
                 + (f", {', '.join(str(c) for c in i['cones'])}, true" if i.get("cones") else (", 0, 0, 0, 0, 0, 0, false, true" if i.get("rolled") else "")) + ">;\n"
                 f"TMPC_DEFINE_GPP_ENTRY({n}, Cfg_{n}, {i['variant']})\n"
+            )
+        elif i["gen"] == 6:
+            # gpp_kernel<Cfg, 3> next to the family instance's gpp_kernel<Cfg, 0>: the same configuration type, a different kernel
+            # symbol.  The configuration is spelled with every template argument.
+            src = (
+                "// generated by tinympc-matlab_b200/build.py -- do not edit\n"
+                '#include "../tmpc_gpp.cuh"\n#include "../tmpc_registry.h"\nusing namespace tmpc;\n'
+                f"using Cfg_{n} = GppCfg<{i['nx']}, {i['nu']}, {i['N']}, {i['gs']}, {i['block']}, false, 0, 0, 0, 0, 0, 0, false, false>;\n"
+                f"TMPC_DEFINE_GPP_MDL_ENTRY({n}, Cfg_{n}, {i['variant']})\n"
             )
         elif i["gen"] == 4:
             src = (

@@ -25,7 +25,7 @@ HOST_EXPORTS = [
     "tinympc_host_set_linear_constraints", "tinympc_host_update_settings", "tinympc_host_set_x0", "tinympc_host_set_x_ref",
     "tinympc_host_set_u_ref", "tinympc_host_solve", "tinympc_host_get_solution", "tinympc_host_get_stats", "tinympc_host_get_cache",
     "tinympc_host_set_cache_terms", "tinympc_host_init_sensitivity", "tinympc_host_set_sensitivity", "tinympc_host_reset_workspace",
-    "tinympc_host_solve_batch", "tinympc_host_set_devices", "tinympc_host_set_option", "tinympc_host_cuda_handle", "tinympc_host_codegen",
+    "tinympc_host_solve_batch", "tinympc_host_solve_batch_models", "tinympc_host_set_devices", "tinympc_host_set_option", "tinympc_host_cuda_handle", "tinympc_host_codegen",
     "tiny_codegen", "tiny_codegen_with_sensitivity",
     # the C++ API mirror itself (extern "C" names of the reference, tiny_api.hpp:10-50)
     "tiny_setup", "tiny_set_bound_constraints", "tiny_set_cone_constraints", "tiny_set_linear_constraints",
@@ -40,7 +40,7 @@ EXPORTS = [
     "tinympc_cuda_version", "tinympc_cuda_host_alloc", "tinympc_cuda_host_free",
     "tinympc_cuda_session_create", "tinympc_cuda_session_destroy", "tinympc_cuda_session_set_x0", "tinympc_cuda_session_set_x_ref",
     "tinympc_cuda_session_set_u_ref", "tinympc_cuda_session_solve", "tinympc_cuda_session_step", "tinympc_cuda_session_read",
-    "tinympc_cuda_precompute_batch",
+    "tinympc_cuda_precompute_batch", "tinympc_cuda_solve_batch_models", "tinympc_cuda_solve_batch_models_device",
 ]
 
 
@@ -79,6 +79,48 @@ class CBatchIn(C.Structure):
 class CBatchOut(C.Structure):
     _fields_ = [("x", C.c_void_p), ("u", C.c_void_p), ("iter", C.c_void_p), ("status", C.c_void_p),
                 ("residuals", C.c_void_p), ("rho", C.c_void_p), ("u0", C.c_void_p)]
+
+
+class CModels(C.Structure):
+    """tinympc_cuda_models: per-problem model arrays, double, one column-major chunk per problem"""
+    _fields_ = [("Adyn", C.c_void_p), ("Bdyn", C.c_void_p), ("fdyn", C.c_void_p), ("Q", C.c_void_p), ("R", C.c_void_p), ("rho", C.c_void_p),
+                ("Kinf", C.c_void_p), ("Pinf", C.c_void_p), ("Quu_inv", C.c_void_p), ("AmBKt", C.c_void_p), ("APf", C.c_void_p), ("BPf", C.c_void_p),
+                ("dKinf_drho", C.c_void_p), ("dPinf_drho", C.c_void_p)]
+
+
+# models dict key -> (CModels field, math shape per problem given (nx, nu)); matrices are stored column-major per problem
+MODEL_FIELDS = (("A", "Adyn", lambda nx, nu: (nx, nx)), ("B", "Bdyn", lambda nx, nu: (nx, nu)), ("f", "fdyn", lambda nx, nu: (nx,)),
+                ("Q", "Q", lambda nx, nu: (nx,)), ("R", "R", lambda nx, nu: (nu,)), ("rho", "rho", lambda nx, nu: ()),
+                ("Kinf", "Kinf", lambda nx, nu: (nu, nx)), ("Pinf", "Pinf", lambda nx, nu: (nx, nx)), ("Quu_inv", "Quu_inv", lambda nx, nu: (nu, nu)),
+                ("AmBKt", "AmBKt", lambda nx, nu: (nx, nx)), ("APf", "APf", lambda nx, nu: (nx,)), ("BPf", "BPf", lambda nx, nu: (nu,)),
+                ("dKinf", "dKinf_drho", lambda nx, nu: (nu, nx)), ("dPinf", "dPinf_drho", lambda nx, nu: (nx, nx)))
+
+
+def pack_models(models: dict, batch: int, nx: int, nu: int) -> dict:
+    """Math-shaped per-problem models -> the column-major float64 arrays of tinympc_cuda_models.
+
+    models: A (B, nx, nx), B (B, nx, nu), f (B, nx), Q (B, nx), R (B, nu) (work->Q / work->R: diagonal + rho), rho (B,), Kinf (B, nu, nx),
+    Pinf (B, nx, nx), Quu_inv (B, nu, nu), AmBKt (B, nx, nx), APf (B, nx), BPf (B, nu), dKinf, dPinf (adaptive rho) -- the shapes
+    precompute_batch returns, so its output merges in directly.  Keys that are absent or None stay NULL.  Returns {CModels field: array}."""
+    out = {}
+    for key, field, shape in MODEL_FIELDS:
+        a = models.get(key)
+        if a is None:
+            continue
+        a = np.asarray(a, np.float64)
+        want = (batch,) + shape(nx, nu)
+        if a.shape != want:
+            raise ValueError(f"models[{key!r}]: expected shape {want}, got {a.shape}")
+        out[field] = np.ascontiguousarray(np.swapaxes(a, 1, 2) if a.ndim == 3 else a)
+    return out
+
+
+def models_struct(arrays: dict) -> CModels:
+    """CModels over host numpy arrays (pack_models) or device pointers (ints)"""
+    m = CModels()
+    for field, a in arrays.items():
+        setattr(m, field, a if isinstance(a, int) else a.ctypes.data)
+    return m
 
 
 class CPrecomputeIn(C.Structure):
@@ -163,6 +205,9 @@ def load():
         L.tinympc_cuda_session_step.argtypes = [C.c_void_p, C.c_int]
         L.tinympc_cuda_session_read.argtypes = [C.c_void_p, C.c_char_p, c_dp]
         L.tinympc_cuda_precompute_batch.argtypes = [C.POINTER(CPrecomputeIn), C.POINTER(CPrecomputeOut)]
+        L.tinympc_cuda_solve_batch_models.argtypes = [C.c_void_p, C.POINTER(CModels), C.POINTER(CBatchIn), C.POINTER(CBatchOut)]
+        L.tinympc_cuda_solve_batch_models_device.argtypes = [C.c_void_p, C.c_int, C.POINTER(CModels), C.POINTER(CBatchIn), C.POINTER(CBatchOut),
+                                                             C.c_void_p]
         # plain-C shim over the host C++ API mirror (csrc/host/tiny_capi_shim.cpp)
         dp, ip, vp = c_dp, c_ip, C.c_void_p
         L.tinympc_host_setup.argtypes = [dp, dp, dp, dp, dp, C.c_double, C.c_int, C.c_int, C.c_int, C.c_int, ip]
@@ -186,6 +231,7 @@ def load():
         L.tinympc_host_set_sensitivity.argtypes = [vp, dp, dp, dp, dp]
         L.tinympc_host_reset_workspace.argtypes = [vp]
         L.tinympc_host_solve_batch.argtypes = [vp, C.POINTER(CBatchIn), C.POINTER(CBatchOut)]
+        L.tinympc_host_solve_batch_models.argtypes = [vp, C.POINTER(CModels), C.POINTER(CBatchIn), C.POINTER(CBatchOut)]
         L.tinympc_host_set_devices.argtypes = [vp, ip, C.c_int]
         L.tinympc_host_set_option.argtypes = [vp, C.c_char_p, C.c_double]
         L.tinympc_host_last_error.argtypes = [vp]
@@ -323,9 +369,10 @@ class CudaSolver:
 
     # ---- host buffers (numpy) ---------------------------------------------------------------
     def solve_batch(self, x0, Xref=None, Uref=None, x_min=None, x_max=None, u_min=None, u_max=None,
-                    want_residuals=True, want_rho=True, out=None, xref_const=None, compact_out=False) -> dict:
+                    want_residuals=True, want_rho=True, out=None, xref_const=None, compact_out=False, models=None) -> dict:
         """xref_const (B, nx): one reference state per problem held over the horizon (instead of Xref);
-        compact_out: return only u0 (B, nu), iter, status -- the trajectories stay on the device."""
+        compact_out: return only u0 (B, nu), iter, status -- the trajectories stay on the device.
+        models: every problem's own model (see pack_models), tinympc_cuda_solve_batch_models; None: the family's."""
         nx, nu, N = self.dims
         keep = []
 
@@ -355,8 +402,17 @@ class CudaSolver:
                     out["rho"] = np.empty(B, np.float32)
         opt = lambda k: out[k].ctypes.data if k in out else None
         co = CBatchOut(opt("x"), opt("u"), out["iter"].ctypes.data, out["status"].ctypes.data, opt("residuals"), opt("rho"), opt("u0"))
-        self._check(self.L.tinympc_cuda_solve_batch(self.h, C.byref(cin), C.byref(co)))
+        if models is None:
+            self._check(self.L.tinympc_cuda_solve_batch(self.h, C.byref(cin), C.byref(co)))
+        else:
+            arrays = pack_models(models, B, nx, nu)
+            self._check(self.L.tinympc_cuda_solve_batch_models(self.h, C.byref(models_struct(arrays)), C.byref(cin), C.byref(co)))
         return out
+
+    def solve_batch_models(self, models: dict, x0, **kw) -> dict:
+        """Problems that each bring their own model (tinympc_cuda_solve_batch_models); `models` as for pack_models, the rest as for
+        solve_batch."""
+        return self.solve_batch(x0, models=models, **kw)
 
     def session(self, batch: int, dev_index: int = 0) -> "CudaSession":
         """`batch` warm-started solvers of the family, resident on the device (tinympc_cuda_session_*)."""
@@ -368,6 +424,15 @@ class CudaSolver:
         cin = CBatchIn(batch, x0, Xref, Uref, x_min, x_max, u_min, u_max, xref_const)
         co = CBatchOut(x, u, iters, status, residuals, rho, u0)
         self._check(self.L.tinympc_cuda_solve_batch_device(self.h, dev_index, C.byref(cin), C.byref(co), stream))
+
+    def solve_batch_models_device(self, models: dict, batch: int, x0, Xref, Uref, x, u, iters, status, residuals=None, rho=None,
+                                  x_min=None, x_max=None, u_min=None, u_max=None, stream=None, dev_index=0, xref_const=None, u0=None):
+        """tinympc_cuda_solve_batch_models_device: models maps CModels field names (Adyn, Bdyn, fdyn, Q, R, rho, Kinf, Pinf, Quu_inv,
+        AmBKt, APf, BPf, dKinf_drho, dPinf_drho) to device pointers of the column-major float64 arrays (pack_models' layout)."""
+        cin = CBatchIn(batch, x0, Xref, Uref, x_min, x_max, u_min, u_max, xref_const)
+        co = CBatchOut(x, u, iters, status, residuals, rho, u0)
+        self._check(self.L.tinympc_cuda_solve_batch_models_device(self.h, dev_index, C.byref(models_struct(models)), C.byref(cin), C.byref(co),
+                                                                  stream))
 
 
 class CudaSession:

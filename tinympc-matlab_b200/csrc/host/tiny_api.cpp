@@ -397,7 +397,8 @@ void tiny_initialize_sensitivity_matrices(TinySolver* solver) {
     for (int i = 0; i < 144; ++i) { c->dPinf_drho.data()[i] = (double)tmpc_tables::dPinf_flat[i]; c->dC2_drho.data()[i] = (double)tmpc_tables::dC2_flat[i]; }
 }
 
-int tiny_solve_batch(TinySolver* solver, const TinyBatchIn* in, const TinyBatchOut* out) {
+namespace {
+int solve_batch_impl(TinySolver* solver, const TinyModelBatch* models, const TinyBatchIn* in, const TinyBatchOut* out) {
     if (!solver || !in || !out) return TINYMPC_CUDA_EINVAL;
     int rc = sync_family(solver);
     if (rc) return rc;
@@ -406,9 +407,17 @@ int tiny_solve_batch(TinySolver* solver, const TinyBatchIn* in, const TinyBatchO
     ci.x_min = in->x_min; ci.x_max = in->x_max; ci.u_min = in->u_min; ci.u_max = in->u_max; ci.xref_const = in->xref_const;
     tinympc_cuda_batch_out co{};
     co.x = out->x; co.u = out->u; co.iter = out->iter; co.status = out->status; co.residuals = out->residuals; co.rho = out->rho; co.u0 = out->u0;
-    rc = tinympc_cuda_solve_batch(solver->backend->cuda, &ci, &co);
+    rc = models ? tinympc_cuda_solve_batch_models(solver->backend->cuda, models, &ci, &co) : tinympc_cuda_solve_batch(solver->backend->cuda, &ci, &co);
     if (rc) solver->backend->err = tinympc_cuda_last_error(solver->backend->cuda);
     return rc;
+}
+}  // namespace
+
+int tiny_solve_batch(TinySolver* solver, const TinyBatchIn* in, const TinyBatchOut* out) { return solve_batch_impl(solver, nullptr, in, out); }
+
+int tiny_solve_batch_models(TinySolver* solver, const TinyModelBatch* models, const TinyBatchIn* in, const TinyBatchOut* out) {
+    if (!models) return TINYMPC_CUDA_EINVAL;
+    return solve_batch_impl(solver, models, in, out);
 }
 
 int tiny_b200_set_devices(TinySolver* solver, const int* devices, int n_devices) {

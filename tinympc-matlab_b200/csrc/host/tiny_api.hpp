@@ -44,6 +44,10 @@ void tiny_initialize_sensitivity_matrices(TinySolver* solver);
 // taken from `solver` as it is NOW) that differ in x0 / Xref / Uref / bounds; cold start per problem.
 // 0 on success, a TINYMPC_CUDA_E* code otherwise.  Validates its arguments (unlike quirk Q8).
 int tiny_solve_batch(TinySolver* solver, const TinyBatchIn* in, const TinyBatchOut* out);
+// The same for problems that each bring their OWN model (dynamics, costs, cache, rho: TinyModelBatch, e.g. from
+// tinympc_cuda_precompute_batch): replaces a loop of { tiny_setup(A_b, B_b, Q_b, R_b, rho_b); tiny_set_x0; tiny_solve } over solvers.
+// `solver` supplies the shape, settings, shared bounds, cones and linear rows; its own matrices and cache are not used.
+int tiny_solve_batch_models(TinySolver* solver, const TinyModelBatch* models, const TinyBatchIn* in, const TinyBatchOut* out);
 // devices to shard batches over (default: the current CUDA device); precision 32 / 64 and other knobs of
 // tinympc_cuda_set_option
 int tiny_b200_set_devices(TinySolver* solver, const int* devices, int n_devices);

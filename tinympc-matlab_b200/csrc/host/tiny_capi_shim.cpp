@@ -129,6 +129,11 @@ int tinympc_host_solve_batch(void* h, const tinympc_cuda_batch_in* in, const tin
     TinyBatchOut bo{out->x, out->u, out->iter, out->status, out->residuals, out->rho};
     return tiny_solve_batch(S(h), &bi, &bo);
 }
+int tinympc_host_solve_batch_models(void* h, const tinympc_cuda_models* m, const tinympc_cuda_batch_in* in, const tinympc_cuda_batch_out* out) {
+    TinyBatchIn bi{in->batch, in->x0, in->Xref, in->Uref, in->x_min, in->x_max, in->u_min, in->u_max, in->xref_const};
+    TinyBatchOut bo{out->x, out->u, out->iter, out->status, out->residuals, out->rho, out->u0};
+    return tiny_solve_batch_models(S(h), m, &bi, &bo);
+}
 int tinympc_host_set_devices(void* h, const int* devices, int n) { return tiny_b200_set_devices(S(h), devices, n); }
 int tinympc_host_set_option(void* h, const char* name, double value) { return tiny_b200_set_option(S(h), name, value); }
 const char* tinympc_host_last_error(void* h) { return tiny_b200_last_error(S(h)); }

@@ -6,6 +6,7 @@
 // T/examples/quadrotor_hovering.cpp:54,66, rocket_landing_mpc.cpp:97-134).  One member is added at the
 // END of TinySolver: the opaque B200 backend that tiny_solve / tiny_solve_batch run on.
 #pragma once
+#include "../../../include/tinympc_b200.h"
 #include "tiny_linalg.hpp"
 
 struct TinySolution {
@@ -108,3 +109,5 @@ struct TinyBatchOut {
     float* rho;           // batch or NULL
     float* u0 = nullptr;  // batch x nu: first control only; with it x and u may be NULL (the trajectories stay on the device)
 };
+// per-problem models of tiny_solve_batch_models: the C ABI's struct itself (double, one column-major chunk per problem)
+typedef tinympc_cuda_models TinyModelBatch;

@@ -69,6 +69,7 @@ struct DeviceCtx {
     DevBuf ref_scratch64[kStreams + 1]; // mixed mode: reference terms of the fp64 re-solve pass
     DevBuf marked[kStreams + 1];        // mixed mode: indices of the problems the fp32 pass marked ambiguous (two-pass form) / the queue
     DevBuf order_buf;                   // claim order of the device-resident entry: 256 histogram words, n list words, n bucket bytes
+    DevBuf models[14];                  // model batches through the host entry: one buffer per field of tinympc_cuda_models (model_fields)
     cudaEvent_t ev_pass = nullptr, ev_copied = nullptr;   // compact streamed pipeline: end of the first pass / of the early result copies
     // exact-count mode, concurrent form: per slot {q_tail, producer CTAs done, consumer ticket counter, pad}
     int* qctl = nullptr;                // 4 * kMaxChunks ints, indexed like the work counters (chunk index; the last one = device entry)
@@ -185,6 +186,7 @@ const KernelEntry* find_kernel(const Family& f, int bits, bool ppb, bool refs, i
     for (int pass = 0; pass < 2; ++pass) {   // pass 1: a reference-storing kernel also serves a reference-free batch
         for (int i = 0; i < n; ++i) {
             const KernelEntry* e = tab[i];
+            if (e->models) continue;                               // model-batch instances: model_kernel()
             if (e->fastbox && (!f.fastbox || ppb)) continue;      // table order puts the fast-box instances first
             if (f.affine && !e->affine) continue;
             if (e->cone_fixed) {   // cones compiled into the instance: the family's cone list must be exactly that
@@ -202,6 +204,36 @@ const KernelEntry* find_kernel(const Family& f, int bits, bool ppb, bool refs, i
     }
     if (variant != 0) return find_kernel(f, bits, ppb, refs, 0);
     return nullptr;
+}
+
+// Model batches (tinympc_cuda_solve_batch_models): the model form of the lane-group fp64 kernel where it applies -- precision 64, a box
+// family without adaptive rho, shared bounds, a compiled shape -- else nullptr: the warp-per-problem kernel in the solver's precision.
+// max_iter <= 0 also takes the warp-per-problem kernel, which runs the reference's zero iterations (the lane-group kernel runs one).
+const KernelEntry* model_kernel(const tinympc_cuda_solver* s, const Family& f, bool ppb) {
+    if (s->force_wpp || s->precision != 64 || f.feat != kFeatBox || ppb || !f.shared_bounds_ok || f.base.max_iter <= 0) return nullptr;
+    int n = 0;
+    const KernelEntry* const* tab = kernel_table(&n);
+    for (int i = 0; i < n; ++i)
+        if (tab[i]->models && tab[i]->nx == f.nx && tab[i]->nu == f.nu && tab[i]->N == f.N) return tab[i];
+    return nullptr;
+}
+
+// the arrays of tinympc_cuda_models and their doubles per problem
+struct ModelField {
+    const double* tinympc_cuda_models::*field;
+    const char* name;
+    int per_problem;
+    bool required;        // dKinf_drho, dPinf_drho: required with adaptive rho
+};
+constexpr int kModelFields = 14;
+void model_fields(int nx, int nu, bool adaptive, ModelField out[kModelFields]) {
+    using M = tinympc_cuda_models;
+    const ModelField f[kModelFields] = {
+        {&M::Adyn, "Adyn", nx * nx, true}, {&M::Bdyn, "Bdyn", nx * nu, true}, {&M::fdyn, "fdyn", nx, false}, {&M::Q, "Q", nx, true},
+        {&M::R, "R", nu, true}, {&M::rho, "rho", 1, true}, {&M::Kinf, "Kinf", nu * nx, true}, {&M::Pinf, "Pinf", nx * nx, true},
+        {&M::Quu_inv, "Quu_inv", nu * nu, true}, {&M::AmBKt, "AmBKt", nx * nx, true}, {&M::APf, "APf", nx, false}, {&M::BPf, "BPf", nu, false},
+        {&M::dKinf_drho, "dKinf_drho", nu * nx, adaptive}, {&M::dPinf_drho, "dPinf_drho", nx * nx, adaptive}};
+    for (int k = 0; k < kModelFields; ++k) out[k] = f[k];
 }
 
 // mixed mode: gather the indices of the problems whose status carries kAmbiguousBit (order is irrelevant)
@@ -392,7 +424,7 @@ const KernelEntry* pick_kernel(const tinympc_cuda_solver* s, const DeviceCtx& d,
 }
 
 int launch_tpp(tinympc_cuda_solver* s, DeviceCtx& d, const KernelEntry* ke, SolveParams& p, DevBuf& rb, int bits, int* counter, cudaStream_t st,
-               int reserve_sms = 0, int* grid_out = nullptr, int max_sms = 0) {
+               int reserve_sms = 0, int* grid_out = nullptr, int max_sms = 0, const tinympc_cuda_models* models = nullptr) {
     const Family& f = s->fam;
     const size_t smem = ke->smem_bytes(f.L.cold_size);
     if (smem > 227u * 1024u) return fail(s, TINYMPC_CUDA_EUNSUPPORTED, std::string("kernel ") + ke->name + " needs more shared memory than an SM has");
@@ -415,7 +447,7 @@ int launch_tpp(tinympc_cuda_solver* s, DeviceCtx& d, const KernelEntry* ke, Solv
     p.work_counter = counter;
     p.refill_min = s->refill_min;
     CU(s, cudaMemsetAsync(counter, 0, sizeof(int), st));
-    CU(s, ke->launch(p, grid, smem, st, f.pack.data(), f.L));
+    CU(s, models ? ke->models_launch(p, grid, smem, st, f.pack.data(), f.L, *models) : ke->launch(p, grid, smem, st, f.pack.data(), f.L));
     s->launches += 1;
     if (grid_out) *grid_out = grid;
     return TINYMPC_CUDA_OK;
@@ -465,10 +497,14 @@ int launch_exact_pair(tinympc_cuda_solver* s, DeviceCtx& d, const KernelEntry* k
 // Do the kernels that will serve the batch do compact I/O themselves (SolveParams::xref_const / u0, KernelEntry::compact_ok)?
 // Mirrors the kernel choice of enqueue(): the first-pass kernel and, in the exact-count mode, the fp64 kernel of the second pass.
 bool compact_in_kernel(const tinympc_cuda_solver* s, const DeviceCtx& d, bool ppb, bool refs, int batch, const KernelEntry** ke_out = nullptr,
-                       const KernelEntry** ke64_out = nullptr) {
+                       const KernelEntry** ke64_out = nullptr, bool models = false) {
     const Family& f = s->fam;
     if (ke_out) *ke_out = nullptr;
     if (ke64_out) *ke64_out = nullptr;
+    if (models) {
+        const KernelEntry* ke = model_kernel(s, f, ppb);
+        return s->compact_in_kernel && ke && ke->compact_ok;
+    }
     if (s->force_wpp) return false;
     const KernelEntry* ke = pick_kernel(s, d, f, s->precision, ppb, refs, batch);
     const bool mixed = s->mixed_band > 0 && s->precision == 32;
@@ -520,9 +556,9 @@ int build_order(tinympc_cuda_solver* s, DeviceCtx& d, const SolveParams& p, int 
 }
 
 // Enqueue the solve of `in`/`out` (device pointers) on `st`.  slot selects the work counters and scratch buffers
-// (one set per pipeline stream + one for the device-resident entry point).
+// (one set per pipeline stream + one for the device-resident entry point).  models (device pointers): a model batch.
 int enqueue(tinympc_cuda_solver* s, DeviceCtx& d, const tinympc_cuda_batch_in& in, const tinympc_cuda_batch_out& out, int counter_slot,
-            cudaStream_t st, int scratch_slot, int direct = 0) {
+            cudaStream_t st, int scratch_slot, int direct = 0, const tinympc_cuda_models* models = nullptr) {
     const Family& f = s->fam;
     const bool ppb = in.x_min || in.x_max || in.u_min || in.u_max;
     if (ppb && !(in.x_min && in.x_max && in.u_min && in.u_max))
@@ -537,7 +573,7 @@ int enqueue(tinympc_cuda_solver* s, DeviceCtx& d, const tinympc_cuda_batch_in& i
         // write the first control alone; for any other kernel the reference is replicated over the horizon first and the
         // trajectories go to this slot's device scratch, from which u0 is gathered.
         const size_t sx = (size_t)f.nx * f.N, su = (size_t)f.nu * (f.N - 1);
-        const bool in_kernel = compact_in_kernel(s, d, ppb, in.xref_const || in.Xref || in.Uref, in.batch);
+        const bool in_kernel = compact_in_kernel(s, d, ppb, in.xref_const || in.Xref || in.Uref, in.batch, nullptr, nullptr, models != nullptr);
         tinympc_cuda_batch_in in2 = in;
         tinympc_cuda_batch_out out2 = out;
         in2.xref_const = nullptr;
@@ -565,7 +601,7 @@ int enqueue(tinympc_cuda_solver* s, DeviceCtx& d, const tinympc_cuda_batch_in& i
             if (!out.u) { CU(s, d.exp_u[scratch_slot].reserve(sizeof(float) * su * in.batch)); out2.u = static_cast<float*>(d.exp_u[scratch_slot].p); }
         }
         if (dir == 0) dir = -1;   // plain trajectories from here on: do not come back into this branch
-        int rc = enqueue(s, d, in2, out2, counter_slot, st, scratch_slot, dir);
+        int rc = enqueue(s, d, in2, out2, counter_slot, st, scratch_slot, dir, models);
         if (rc) return rc;
         if (out.u0 && !u0_direct) {
             const size_t total = (size_t)f.nu * in.batch;
@@ -578,10 +614,10 @@ int enqueue(tinympc_cuda_solver* s, DeviceCtx& d, const tinympc_cuda_batch_in& i
     if (direct < 0) direct = 0;
     const bool refs = in.Xref || in.Uref;
     int bits = s->precision;
-    const KernelEntry* ke = s->force_wpp ? nullptr : pick_kernel(s, d, f, bits, ppb, refs, in.batch);
+    const KernelEntry* ke = models ? model_kernel(s, f, ppb) : s->force_wpp ? nullptr : pick_kernel(s, d, f, bits, ppb, refs, in.batch);
     // mixed mode needs the specialised kernels in both precisions; any other shape runs entirely in fp64 (exact as well)
     const KernelEntry* ke64 = nullptr;
-    const bool mixed = s->mixed_band > 0 && bits == 32;
+    const bool mixed = !models && s->mixed_band > 0 && bits == 32;   // model batches: refused by solve_batch_common
     if (mixed) {
         ke64 = s->force_wpp ? nullptr : find_kernel(f, 64, ppb, refs, 0);
         if (!ke || !ke64) { ke = nullptr; bits = 64; }
@@ -600,27 +636,27 @@ int enqueue(tinympc_cuda_solver* s, DeviceCtx& d, const tinympc_cuda_batch_in& i
         return fail(s, TINYMPC_CUDA_EUNSUPPORTED, "internal: compact I/O handed to a kernel that does not do it");
     if (!ke) {
         // no specialised thread-per-problem kernel for this shape / feature mix: general warp-per-problem kernel
-        const WppLayout W = WppLayout::make(f.nx, f.nu, f.N);
+        const WppLayout W = WppLayout::make(f.nx, f.nu, f.N, models != nullptr);
         const int warps = std::max(1, std::min(in.batch, d.sm_count * 16));
         const size_t esz = bits == 64 ? sizeof(double) : sizeof(float);
         DevBuf& sb = d.wpp_scratch[scratch_slot];
         CU(s, sb.reserve((size_t)warps * W.size * esz));
         const void* full_pack = bits == 64 ? d.pack64 : d.pack32;
-        if (bits == 64) CU(s, wpp_launch<double>(p, f.L, full_pack, W, sb.p, warps, 0, st));
-        else CU(s, wpp_launch<float>(p, f.L, full_pack, W, sb.p, warps, 0, st));
-        note_kernel(s, bits == 64 ? "wpp_f64_generic" : "wpp_f32_generic");
+        if (bits == 64) CU(s, wpp_launch<double>(p, f.L, full_pack, W, sb.p, warps, 0, st, models));
+        else CU(s, wpp_launch<float>(p, f.L, full_pack, W, sb.p, warps, 0, st, models));
+        note_kernel(s, models ? (bits == 64 ? "wpp_f64_mdl_generic" : "wpp_f32_mdl_generic") : (bits == 64 ? "wpp_f64_generic" : "wpp_f32_generic"));
         s->launches += 1;
         return TINYMPC_CUDA_OK;
     }
     int* const counter = d.counters + counter_slot;
     // device-resident batches of a few waves: the fp32 thread-per-problem kernels claim the hardest problems first (build_order)
-    if (s->order && scratch_slot == kStreams && bits == 32 && f.feat == kFeatBox && !ppb && f.shared_bounds_ok && p.en_input_bound &&
+    if (!models && s->order && scratch_slot == kStreams && bits == 32 && f.feat == kFeatBox && !ppb && f.shared_bounds_ok && p.en_input_bound &&
         ke->lanes_per_problem <= 1 && f.nx <= 16 && f.nu <= 8 && (long long)in.batch >= 2LL * d.sm_count * ke->block) {
         int rc = build_order(s, d, p, in.batch, st, &p.index_list);
         if (rc) return rc;
     }
     if (!mixed) {
-        int rc = launch_tpp(s, d, ke, p, d.ref_scratch[scratch_slot], bits, counter, st);
+        int rc = launch_tpp(s, d, ke, p, d.ref_scratch[scratch_slot], bits, counter, st, 0, nullptr, 0, models);
         if (rc) return rc;
         note_kernel(s, ke->name);
         return TINYMPC_CUDA_OK;
@@ -1053,9 +1089,10 @@ std::mutex& device_call_mutex(int device) {
     return mu[device & 63];
 }
 
-// One device's share of a host batch: chunked H2D -> kernel -> D2H pipeline over kStreams streams.
+// One device's share of a host batch: chunked H2D -> kernel -> D2H pipeline over kStreams streams.  models (host pointers): a model
+// batch, whose model arrays travel chunk by chunk with the inputs.
 int run_shard(tinympc_cuda_solver* s, DeviceCtx& d, const tinympc_cuda_batch_in& in, const tinympc_cuda_batch_out& out, int lo, int hi,
-              double* kernel_ms, int* nchunks_out, long long* marked_out) {
+              double* kernel_ms, int* nchunks_out, long long* marked_out, const tinympc_cuda_models* models) {
     const Family& f = s->fam;
     const int n = hi - lo;
     *kernel_ms = 0; *nchunks_out = 0; *marked_out = 0;
@@ -1079,11 +1116,17 @@ int run_shard(tinympc_cuda_solver* s, DeviceCtx& d, const tinympc_cuda_batch_in&
     CU(s, d.iter.reserve(sizeof(int) * (size_t)n)); CU(s, d.status.reserve(sizeof(int) * (size_t)n));
     if (out.residuals) CU(s, d.res.reserve(sizeof(float) * 4 * (size_t)n));
     if (out.rho) CU(s, d.rho.reserve(sizeof(float) * (size_t)n));
+    ModelField mf[kModelFields];
+    if (models) {
+        model_fields(f.nx, f.nu, f.base.adaptive_rho != 0, mf);
+        for (int k = 0; k < kModelFields; ++k)
+            if (models->*mf[k].field) CU(s, d.models[k].reserve(sizeof(double) * mf[k].per_problem * (size_t)n));
+    }
 
     // single-launch streamed pipeline: a thread-per-problem kernel that honours the watermark; in the exact-count mode the
     // concurrent producer / consumer pair (both count completions per chunk)
     const bool mixed = s->mixed_band > 0 && s->precision == 32;
-    if (s->streamed && !compact && !(mixed && s->fixer_sms == -1) && !s->force_wpp && stream_memops().ok) {
+    if (!models && s->streamed && !compact && !(mixed && s->fixer_sms == -1) && !s->force_wpp && stream_memops().ok) {
         const KernelEntry* ke = pick_kernel(s, d, f, s->precision, ppb, in.Xref || in.Uref, n);
         const KernelEntry* ke64 = mixed ? find_kernel(f, 64, ppb, in.Xref || in.Uref, 0) : nullptr;
         // auto (0): the ramped chunk layout for shards of >= 2^16 problems, else equal chunks of >= 2^14 problems
@@ -1093,7 +1136,7 @@ int run_shard(tinympc_cuda_solver* s, DeviceCtx& d, const tinympc_cuda_batch_in&
     }
     // compact I/O: one launch chain behind an arrival watermark, when the kernels of the batch wait for the watermark and read
     // the compact reference in place (chunks = 1 keeps the single chunked launch, fixer_sms >= 0 the concurrent exact-count pair)
-    if (compact && s->compact_streamed && !s->force_wpp && stream_memops().ok && !(mixed && s->fixer_sms >= 0) &&
+    if (!models && compact && s->compact_streamed && !s->force_wpp && stream_memops().ok && !(mixed && s->fixer_sms >= 0) &&
         (s->chunks >= 2 || (s->chunks <= 0 && n >= (1 << 16))) && (ppb || f.shared_bounds_ok)) {
         const KernelEntry *ke = nullptr, *ke64 = nullptr;
         const bool refs = in.xref_const || in.Xref || in.Uref;
@@ -1149,8 +1192,17 @@ int run_shard(tinympc_cuda_solver* s, DeviceCtx& d, const tinympc_cuda_batch_in&
         dout.iter = (int*)d.iter.p + c0; dout.status = (int*)d.status.p + c0;
         dout.residuals = out.residuals ? (float*)d.res.p + 4 * (size_t)c0 : nullptr;
         dout.rho = out.rho ? (float*)d.rho.p + c0 : nullptr;
+        tinympc_cuda_models dm{};
+        if (models)
+            for (int k = 0; k < kModelFields; ++k)
+                if (const double* src = models->*mf[k].field) {
+                    const size_t per_problem = mf[k].per_problem;
+                    double* dst = static_cast<double*>(d.models[k].p) + per_problem * c0;
+                    CU(s, cudaMemcpyAsync(dst, src + per_problem * g0, sizeof(double) * per_problem * cn, cudaMemcpyHostToDevice, st));
+                    dm.*mf[k].field = dst;
+                }
         CU(s, cudaEventRecord(d.k0[c], st));
-        int rc = enqueue(s, d, din, dout, c, st, c % kStreams);
+        int rc = enqueue(s, d, din, dout, c, st, c % kStreams, 0, models ? &dm : nullptr);
         if (rc) return rc;
         CU(s, cudaEventRecord(d.k1[c], st));
         if (out.x) CU(s, cudaMemcpyAsync(out.x + sx * g0, dout.x, sizeof(float) * sx * cn, cudaMemcpyDeviceToHost, st));
@@ -1275,6 +1327,7 @@ int tinympc_cuda_destroy(tinympc_cuda_solver* s) {
         if (d.ev_pass) cudaEventDestroy(d.ev_pass);
         if (d.ev_copied) cudaEventDestroy(d.ev_copied);
         for (DevBuf* b : {&d.x0, &d.Xref, &d.Uref, &d.xmin, &d.xmax, &d.umin, &d.umax, &d.x, &d.u, &d.iter, &d.status, &d.res, &d.rho, &d.xrc, &d.u0}) b->release();
+        for (auto& b : d.models) b.release();
         for (auto& b : d.exp_xref) b.release();
         for (auto& b : d.exp_x) b.release();
         for (auto& b : d.exp_u) b.release();
@@ -1414,8 +1467,29 @@ int tinympc_cuda_set_family(tinympc_cuda_solver* s, const tinympc_cuda_family* f
     return upload_family(s);
 }
 
-int tinympc_cuda_solve_batch_device(tinympc_cuda_solver* s, int dev_index, const tinympc_cuda_batch_in* in, const tinympc_cuda_batch_out* out,
-                                    void* stream) {
+}  // extern "C"
+
+namespace {
+
+// model batches: every required array present (adaptive rho: the two sensitivities too); device pointers 16-byte aligned
+int check_models(tinympc_cuda_solver* s, const tinympc_cuda_models* m, bool device) {
+    if (!m) return TINYMPC_CUDA_OK;
+    if (s->mixed_band > 0 && s->precision == 32)
+        return fail(s, TINYMPC_CUDA_EUNSUPPORTED, "model batches have no exact-count (\"mixed\") form: use \"precision\" 64, which is exact for them");
+    ModelField mf[kModelFields];
+    model_fields(s->fam.nx, s->fam.nu, s->fam.base.adaptive_rho != 0, mf);
+    for (int k = 0; k < kModelFields; ++k) {
+        const double* p = m->*mf[k].field;
+        if (mf[k].required && !p)
+            return fail(s, TINYMPC_CUDA_EINVAL, std::string("model batch: ") + mf[k].name + " is required" +
+                                                    (k >= 12 ? " (the family has adaptive_rho)" : ""));
+        if (device && check_ptr16(s, p, mf[k].name)) return TINYMPC_CUDA_EINVAL;
+    }
+    return TINYMPC_CUDA_OK;
+}
+
+int solve_batch_device_common(tinympc_cuda_solver* s, int dev_index, const tinympc_cuda_models* m, const tinympc_cuda_batch_in* in,
+                              const tinympc_cuda_batch_out* out, void* stream) {
     if (!s || !in || !out) return TINYMPC_CUDA_EINVAL;
     if (!s->fam.set) return fail(s, TINYMPC_CUDA_ENOTREADY, "tinympc_cuda_set_family has not been called");
     if (dev_index < 0 || dev_index >= (int)s->devs.size()) return fail(s, TINYMPC_CUDA_EINVAL, "dev_index out of range");
@@ -1423,7 +1497,8 @@ int tinympc_cuda_solve_batch_device(tinympc_cuda_solver* s, int dev_index, const
     if (in->batch == 0) return TINYMPC_CUDA_OK;
     if (!in->x0 || !out->iter || !out->status || !((out->x && out->u) || out->u0))
         return fail(s, TINYMPC_CUDA_EINVAL, "x0, iter, status and either (x, u) or u0 are required");
-    int rc = 0;
+    int rc = check_models(s, m, true);
+    if (rc) return rc;
     rc |= check_ptr16(s, in->xref_const, "xref_const"); rc |= check_ptr16(s, out->u0, "u0");
     rc |= check_ptr16(s, in->x0, "x0"); rc |= check_ptr16(s, in->Xref, "Xref"); rc |= check_ptr16(s, in->Uref, "Uref");
     rc |= check_ptr16(s, in->x_min, "x_min"); rc |= check_ptr16(s, in->x_max, "x_max"); rc |= check_ptr16(s, in->u_min, "u_min");
@@ -1434,18 +1509,18 @@ int tinympc_cuda_solve_batch_device(tinympc_cuda_solver* s, int dev_index, const
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     DeviceGuard guard;                 // restores the caller's current device on every return path
     CU(s, cudaSetDevice(d.device));
-    if (s->fam.base.max_iter <= 0) {
+    if (s->fam.base.max_iter <= 0 && !m) {   // a model batch runs the zero iterations in the kernel: every problem keeps its own rho
         rc = zero_iteration_result(s, s->fam, *out, in->batch, st, true);
     } else {
         // The last counter / scratch slot belongs to the device-resident entry point: ONE call in flight per device context
         // (include/tinympc_b200.h).  A second call on another stream would share the work counter and the scratch buffers.
-        rc = enqueue(s, d, *in, *out, kMaxChunks - 1, st, kStreams);
+        rc = enqueue(s, d, *in, *out, kMaxChunks - 1, st, kStreams, 0, m);
         s->mixed_pending_dev = (s->mixed_band > 0 && s->precision == 32) ? dev_index : -1;
     }
     return rc;
 }
 
-int tinympc_cuda_solve_batch(tinympc_cuda_solver* s, const tinympc_cuda_batch_in* in, const tinympc_cuda_batch_out* out) {
+int solve_batch_common(tinympc_cuda_solver* s, const tinympc_cuda_models* m, const tinympc_cuda_batch_in* in, const tinympc_cuda_batch_out* out) {
     if (!s || !in || !out) return TINYMPC_CUDA_EINVAL;
     if (!s->fam.set) return fail(s, TINYMPC_CUDA_ENOTREADY, "tinympc_cuda_set_family has not been called");
     if (in->batch < 0) return fail(s, TINYMPC_CUDA_EINVAL, "negative batch");
@@ -1456,7 +1531,8 @@ int tinympc_cuda_solve_batch(tinympc_cuda_solver* s, const tinympc_cuda_batch_in
     const bool ppb = in->x_min || in->x_max || in->u_min || in->u_max;
     if (ppb && !(in->x_min && in->x_max && in->u_min && in->u_max))
         return fail(s, TINYMPC_CUDA_EINVAL, "per-problem bounds need all four of x_min, x_max, u_min, u_max");
-    if (s->fam.base.max_iter <= 0) return zero_iteration_result(s, s->fam, *out, in->batch, nullptr, false);
+    if (int rc = check_models(s, m, false)) return rc;
+    if (s->fam.base.max_iter <= 0 && !m) return zero_iteration_result(s, s->fam, *out, in->batch, nullptr, false);
 
     const auto t0 = std::chrono::steady_clock::now();
     const int G = (int)s->devs.size();
@@ -1469,7 +1545,7 @@ int tinympc_cuda_solve_batch(tinympc_cuda_solver* s, const tinympc_cuda_batch_in
     int per = ((in->batch + G - 1) / G + 3) & ~3;
     auto work = [&](int g) {
         const int lo = std::min(in->batch, g * per), hi = (g == G - 1) ? in->batch : std::min(in->batch, lo + per);
-        rcs[g] = run_shard(s, s->devs[g], *in, *out, lo, hi, &kms[g], &nch[g], &marked[g]);
+        rcs[g] = run_shard(s, s->devs[g], *in, *out, lo, hi, &kms[g], &nch[g], &marked[g], m);
     };
     if (G == 1) {
         work(0);
@@ -1487,6 +1563,31 @@ int tinympc_cuda_solve_batch(tinympc_cuda_solver* s, const tinympc_cuda_batch_in
     s->t_chunks = *std::max_element(nch.begin(), nch.end());
     s->t_total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     return TINYMPC_CUDA_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tinympc_cuda_solve_batch_device(tinympc_cuda_solver* s, int dev_index, const tinympc_cuda_batch_in* in, const tinympc_cuda_batch_out* out,
+                                    void* stream) {
+    return solve_batch_device_common(s, dev_index, nullptr, in, out, stream);
+}
+
+int tinympc_cuda_solve_batch(tinympc_cuda_solver* s, const tinympc_cuda_batch_in* in, const tinympc_cuda_batch_out* out) {
+    return solve_batch_common(s, nullptr, in, out);
+}
+
+int tinympc_cuda_solve_batch_models_device(tinympc_cuda_solver* s, int dev_index, const tinympc_cuda_models* m, const tinympc_cuda_batch_in* in,
+                                           const tinympc_cuda_batch_out* out, void* stream) {
+    if (!m) return s ? fail(s, TINYMPC_CUDA_EINVAL, "model batch: models is NULL") : TINYMPC_CUDA_EINVAL;
+    return solve_batch_device_common(s, dev_index, m, in, out, stream);
+}
+
+int tinympc_cuda_solve_batch_models(tinympc_cuda_solver* s, const tinympc_cuda_models* m, const tinympc_cuda_batch_in* in,
+                                    const tinympc_cuda_batch_out* out) {
+    if (!m) return s ? fail(s, TINYMPC_CUDA_EINVAL, "model batch: models is NULL") : TINYMPC_CUDA_EINVAL;
+    return solve_batch_common(s, m, in, out);
 }
 
 int tinympc_cuda_solve_workspace(tinympc_cuda_solver* s, const tinympc_cuda_workspace* w) {

@@ -9,6 +9,8 @@
 #include <cstddef>
 #include <cstdint>
 
+#include "tinympc_b200.h"   // tinympc_cuda_models: the per-problem model arrays the model kernels read on the device
+
 namespace tmpc {
 
 constexpr int kMaxCones = 4;     // per family (state cones) and (input cones)

@@ -34,6 +34,8 @@
 //                       rolled time loops, because the unrolled form no longer fits the 32 KB instruction cache
 //   session (MODE 1)    persistent TinyWorkspace images iterated in place with the reference's warm-start semantics
 //   workspace (MODE 2)  the same for ONE live workspace, every member written back: tiny_solve
+//   models (MODE 3)     model batches (tinympc_cuda_solve_batch_models): a group that claims a problem loads its lanes' rows from that
+//                       problem's own model and forms the products on the device in the host's order (fill_gpp_tab); box only
 #pragma once
 #include "tmpc_tpp2.cuh"
 #include "tmpc_wpp.h"
@@ -164,6 +166,8 @@ struct GppSession {
     WppLayout W;
     int full;          // informational: the launcher instantiates MODE 2 (also write d, every column of p and the unused columns 0 and N-1
                        // of q: tiny_solve on ONE live workspace, whose owner may look at any member of TinyWorkspace afterwards) or MODE 1
+    tinympc_cuda_models models;   // MODE 3 (model batches): the per-problem model arrays, device pointers; the tables of `tab` other
+                                  // than the bounds are not read
 };
 
 // per-slot state of a lane: registers (statically indexed, unrolled time loops) or a shared-memory column [slot][thread]
@@ -189,12 +193,17 @@ __device__ __forceinline__ double gabsmax(double r, double a) {
 }
 __device__ __forceinline__ double gclamp(double t, double lo, double hi) { return gmin(hi, gmax(lo, t)); }   // admm.cpp:91-98 order
 
-template <class C, int MODE = 0>   // 0: batch; 1: sessions (what the next warm start reads is written back); 2: tiny_solve on one live workspace (every member)
+constexpr int kGppModels = 3;      // gpp_kernel MODE of model batches
+
+template <class C, int MODE = 0>   // 0: batch; 1: sessions (what the next warm start reads is written back); 2: tiny_solve on one live workspace (every member);
+                                   // 3: model batch (every problem brings its own matrices and cache, ses.models)
 __global__ void __launch_bounds__(C::BLOCK, C::MINB)
 gpp_kernel(const __grid_constant__ SolveParams prm, const __grid_constant__ GppTab<C::NX, C::NU, C::NH, C::GS, C::ADAPT> tab,
            const __grid_constant__ GppSession ses) {
-    constexpr bool SESSION = MODE != 0, FULLWS = MODE == 2;
+    // (model mode is tested as MODE == kGppModels: one more constexpr local here changes the machine code of the other modes)
+    constexpr bool SESSION = MODE == 1 || MODE == 2, FULLWS = MODE == 2;
     static_assert(!(SESSION && C::ADAPT), "adaptive-rho sessions keep a cache per problem: they stay on the warp-per-problem kernel");
+    static_assert(!(MODE == kGppModels && (C::ADAPT || C::CONSTR)), "model batches with adaptive rho, cones or rows stay on the warp-per-problem kernel");
     using T = double;
     constexpr int NX = C::NX, NU = C::NU, NH = C::NH, GS = C::GS, NXP = C::NXP, NUP = C::NUP, SXL = C::SX, SUL = C::SU;
     constexpr unsigned FULL = 0xffffffffu;
@@ -236,7 +245,7 @@ gpp_kernel(const __grid_constant__ SolveParams prm, const __grid_constant__ GppT
     for (int c = 0; c < NX; ++c) { cf1[c] = tab.CF1[lc][c]; cb1[c] = tab.CB1[lc][c]; }
 #pragma unroll
     for (int a = 0; a < NU; ++a) { cf2[a] = tab.CF2[lc][a]; cb2[a] = tab.CB2[lc][a]; }
-    const T cf0 = tab.cf0[lc], cb0 = tab.cb0[lc], wref = tab.wref[lc];
+    T cf0 = tab.cf0[lc], cb0 = tab.cb0[lc], wref = tab.wref[lc];
     const T rho0 = prm.rho, tol_pri = prm.abs_pri_tol, tol_dua = prm.abs_dua_tol;
     const bool adaptive = C::ADAPT && prm.adaptive_rho != 0;
     const int max_iter = prm.max_iter, check_every = prm.check_termination;
@@ -335,6 +344,49 @@ gpp_kernel(const __grid_constant__ SolveParams prm, const __grid_constant__ GppT
                 }
 #pragma unroll
                 for (int s = 0; s < NH; ++s) { G[s] = 0; V[s] = 0; RF[s] = 0.f; }
+                if constexpr (MODE == kGppModels) {
+                    // this lane's rows of the problem's own model (column-major: M(i, j) = M[j * rows + i]), formed exactly as fill_gpp_tab
+                    // forms them on the host: the same order, every product and sum rounded on its own (no contraction into an fma)
+                    const tinympc_cuda_models& M = ses.models;
+                    const size_t b = prob;
+                    const double* A = M.Adyn + b * NX * NX; const double* B = M.Bdyn + b * NX * NU; const double* K = M.Kinf + b * NU * NX;
+                    const double* Qi = M.Quu_inv + b * NU * NU;
+                    if (is_u) {   // input lane a = row
+#pragma unroll
+                        for (int c = 0; c < NX; ++c) {
+                            cf1[c] = -K[c * NU + row];
+                            T acc = 0.0;
+#pragma unroll
+                            for (int e = 0; e < NU; ++e) acc = __dadd_rn(acc, __dmul_rn(Qi[e * NU + row], B[e * NX + c]));   // (Quu_inv B')[a][c]
+                            cb1[c] = acc;
+                        }
+                        T acc = 0.0;
+#pragma unroll
+                        for (int e = 0; e < NU; ++e) {
+                            cf2[e] = (e == row) ? -1.0 : 0.0;
+                            cb2[e] = Qi[e * NU + row];
+                            acc = __dadd_rn(acc, __dmul_rn(Qi[e * NU + row], M.BPf ? M.BPf[b * NU + e] : 0.0));
+                        }
+                        cf0 = 0.0;
+                        cb0 = acc;
+                        wref = M.R[b * NU + row];
+                    } else {      // state lane r = row (idle lanes compute row 0's values, which nobody reads)
+#pragma unroll
+                        for (int c = 0; c < NX; ++c) {
+                            T acc = A[c * NX + row];
+#pragma unroll
+                            for (int e = 0; e < NU; ++e) acc = __dsub_rn(acc, __dmul_rn(B[e * NX + row], K[c * NU + e]));   // (A - B Kinf)[r][c]
+                            cf1[c] = acc;
+                            cb1[c] = M.AmBKt[b * NX * NX + c * NX + row];
+                        }
+#pragma unroll
+                        for (int e = 0; e < NU; ++e) { cf2[e] = -B[e * NX + row]; cb2[e] = -K[row * NU + e]; }
+                        cf0 = M.fdyn ? M.fdyn[b * NX + row] : 0.0;
+                        cb0 = M.APf ? M.APf[b * NX + row] : 0.0;
+                        wref = M.Q[b * NX + row];
+                    }
+                    rho = rho_lc = M.rho[b];
+                }
                 if constexpr (C::CONSTR) {
 #pragma unroll
                     for (int s = 0; s < NH; ++s) { GC[s] = 0; GL[s] = 0; EC[s] = 0; }
@@ -379,7 +431,8 @@ gpp_kernel(const __grid_constant__ SolveParams prm, const __grid_constant__ GppT
                     T acc = 0, acc1 = 0;
 #pragma unroll
                     for (int c = 0; c < NX; ++c) {
-                        acc = fma(xb[c], tab.Pinf[c][row], acc);
+                        if constexpr (MODE == kGppModels) acc = fma(xb[c], ses.models.Pinf[(size_t)prob * NX * NX + row * NX + c], acc);   // Pinf(c, row)
+                        else acc = fma(xb[c], tab.Pinf[c][row], acc);
                         if constexpr (C::ADAPT) acc1 = fma(xb[c], tab.dPinf[c][row], acc1);
                     }
                     PT = -acc; PT1 = -acc1;

@@ -46,6 +46,10 @@ struct KernelEntry {
     int compact_ok;
     // 1: honours SolveParams::order_from (a streamed batch whose later part is claimed through a list built meanwhile)
     int order_from_ok;
+    // 1: a model-batch instance (tinympc_cuda_solve_batch_models): launched through models_launch only, never for a family batch
+    int models;
+    cudaError_t (*models_launch)(const SolveParams& p, int grid, size_t smem, cudaStream_t st, const double* master_pack, const PackLayout& L,
+                                 const tinympc_cuda_models& m);
 };
 
 const KernelEntry* const* kernel_table(int* count);   // defined in gen/tmpc_table.cu
@@ -154,4 +158,30 @@ const KernelEntry* const* kernel_table(int* count);   // defined in gen/tmpc_tab
                                     0, 0, 1, CFG::BLOCK, VAR, 1, SYM##_smem, SYM##_prepare,                        \
                                     SYM##_occ, SYM##_launch, CFG::CONSTR ? 1 : 0, CFG::SCS, CFG::SCD, CFG::UCS, CFG::UCD, CFG::NSL, CFG::NIL, CFG::GS,     \
                                     (CFG::ADAPT || CFG::CONSTR) ? nullptr : SYM##_session, 1};                      \
+    }
+
+// model-batch form of the lane-group-per-problem fp64 kernel (gpp_kernel MODE 3): the shared bounds come from the family's table,
+// every other row from the claimed problem's model
+#define TMPC_DEFINE_GPP_MDL_ENTRY(SYM, CFG, VAR)                                                                    \
+    namespace tmpc {                                                                                                \
+    static_assert(!CFG::ADAPT && !CFG::CONSTR, "model batches: box families only");                                 \
+    static size_t SYM##_smem(int pe) { return gpp_smem_bytes<CFG>(pe); }                                            \
+    static cudaError_t SYM##_prepare(size_t smem) {                                                                 \
+        return cudaFuncSetAttribute(gpp_kernel<CFG, kGppModels>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);    \
+    }                                                                                                               \
+    static cudaError_t SYM##_occ(int* n, size_t smem) {                                                             \
+        return cudaOccupancyMaxActiveBlocksPerMultiprocessor(n, gpp_kernel<CFG, kGppModels>, CFG::BLOCK, smem);              \
+    }                                                                                                               \
+    static cudaError_t SYM##_launch(const SolveParams& p, int grid, size_t smem, cudaStream_t st, const double* mp, \
+                                    const PackLayout& L, const tinympc_cuda_models& m) {                            \
+        GppTab<CFG::NX, CFG::NU, CFG::NH, CFG::GS, false> tab;                                                      \
+        fill_gpp_tab(tab, mp, L, p);                                                                                \
+        GppSession ses{};                                                                                           \
+        ses.models = m;                                                                                             \
+        gpp_kernel<CFG, kGppModels><<<grid, CFG::BLOCK, smem, st>>>(p, tab, ses);                                            \
+        return cudaGetLastError();                                                                                  \
+    }                                                                                                               \
+    extern const KernelEntry SYM = {#SYM, KF_TPP, CFG::NX, CFG::NU, CFG::NH, 0 /* FEAT_BOX */, 64, 1, 0, 0, 1, CFG::BLOCK, VAR, 0, \
+                                    SYM##_smem, SYM##_prepare, SYM##_occ, nullptr, 0, 0, 0, 0, 0, 0, 0, CFG::GS, nullptr, 1, 0, \
+                                    1, SYM##_launch};                                                               \
     }

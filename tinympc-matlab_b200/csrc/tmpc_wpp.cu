@@ -82,240 +82,20 @@ template <typename T, int NXC, int NUC>
 __global__ void __launch_bounds__(128) wpp_kernel(const SolveParams prm, const PackLayout L, const T* __restrict__ pack,
                                                   const WppLayout W, T* __restrict__ scratch, const int explicit_workspace,
                                                   const int ws_in_smem) {
-    extern __shared__ __align__(16) unsigned char wpp_smem[];
-    const int lane = threadIdx.x & 31;
-    const int warp_global = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int n_warps = (gridDim.x * blockDim.x) >> 5;
-    const int nx = NXC > 0 ? NXC : L.nx, nu = NUC > 0 ? NUC : L.nu, N = L.N;
-    constexpr int UNR = NXC > 0 ? 16 : 1;   // compile-time shapes: every dot product fully unrolled
-    const int sx = nx * N, su = nu * (N - 1);
+    constexpr bool MODELS = false;
+    [[maybe_unused]] const tinympc_cuda_models M{};
+#include "tmpc_wpp_body.inc"
+}
 
-    const T* A = pack + L.A;   const T* B = pack + L.B;   const T* AK = pack + L.AmBKt; const T* Quu = pack + L.Quu_inv;
-    const T* f = pack + L.f;   const T* APf = pack + L.APf; const T* BPf = pack + L.BPf;
-    const T* Qd = pack + L.Qd; const T* Rd = pack + L.Rd;
-    const T* dK = pack + L.dKinf; const T* dP = pack + L.dPinf;
-    const T* Alx = pack + L.Alin_x; const T* blx = pack + L.blin_x; const T* nrx = pack + L.nrm_x;
-    const T* Alu = pack + L.Alin_u; const T* blu = pack + L.blin_u; const T* nru = pack + L.nrm_u;
-
-    const bool en_sb = prm.en_state_bound, en_ib = prm.en_input_bound;
-    const bool soc_x = prm.en_state_soc && prm.n_state_cones > 0, soc_u = prm.en_input_soc && prm.n_input_cones > 0;
-    const bool lin_x = prm.en_state_linear, lin_u = prm.en_input_linear;
-    const T tol_pri = static_cast<T>(prm.abs_pri_tol), tol_dua = static_cast<T>(prm.abs_dua_tol);
-
-    for (int prob = warp_global; prob < prm.batch; prob += n_warps) {
-        // explicit_workspace 0: one scratch workspace per warp, cold start per problem; 1: ONE live workspace (tiny_solve);
-        // 2: a persistent workspace per PROBLEM (a session of warm-started solvers), iterated in place
-        // The workspace is iterated in SHARED memory when the launcher says so (ws_in_smem): the lanes of the warp hand the columns
-        // of p, x, u and the scratch vector to each other at every time step.  Live workspaces (sessions) are copied in and out.
-        T* const gws = scratch ? scratch + (size_t)(explicit_workspace == 2 ? prob : warp_global) * W.size : nullptr;
-        T* const ws = ws_in_smem ? reinterpret_cast<T*>(wpp_smem) + (size_t)(threadIdx.x >> 5) * W.size : gws;
-        if (ws_in_smem && explicit_workspace) {
-            for (int e = lane; e < W.size; e += 32) ws[e] = gws[e];
-            __syncwarp();
-        }
-        T *x = ws + W.x, *u = ws + W.u, *q = ws + W.q, *r = ws + W.r, *p = ws + W.p, *d = ws + W.d;
-        T *v = ws + W.v, *vnew = ws + W.vnew, *z = ws + W.z, *znew = ws + W.znew, *g = ws + W.g, *y = ws + W.y;
-        T *vcnew = ws + W.vcnew, *zcnew = ws + W.zcnew, *gc = ws + W.gc, *yc = ws + W.yc;
-        T *vlnew = ws + W.vlnew, *zlnew = ws + W.zlnew, *gl = ws + W.gl, *yl = ws + W.yl;
-        T *Xref = ws + W.Xref, *Uref = ws + W.Uref;
-        T *xmin = ws + W.xmin, *xmax = ws + W.xmax, *umin = ws + W.umin, *umax = ws + W.umax;
-        T *K = ws + W.Kinf, *P = ws + W.Pinf;        // per-problem copies: adaptive rho mutates them
-        T *tmp = ws + W.tmp;                          // nu scratch
-        T *sc = ws + W.scalars;                       // [0] rho, [1] iter, [2] status, [3..6] residuals, [7] solved
-
-        if (!explicit_workspace) {
-            // ---- cold workspace (tiny_api.cpp:68-105) + this problem's inputs
-            for (int e = lane; e < W.zero_end; e += 32) ws[e] = 0;
-            __syncwarp();
-            for (int e = lane; e < nx; e += 32) x[e] = static_cast<T>(prm.x0[(size_t)prob * nx + e]);
-            for (int e = lane; e < sx; e += 32) {
-                Xref[e] = prm.Xref ? static_cast<T>(prm.Xref[(size_t)prob * sx + e]) : T(0);
-                xmin[e] = prm.x_min ? static_cast<T>(prm.x_min[(size_t)prob * sx + e]) : pack[L.xmin + e];
-                xmax[e] = prm.x_max ? static_cast<T>(prm.x_max[(size_t)prob * sx + e]) : pack[L.xmax + e];
-            }
-            for (int e = lane; e < su; e += 32) {
-                Uref[e] = prm.Uref ? static_cast<T>(prm.Uref[(size_t)prob * su + e]) : T(0);
-                umin[e] = prm.u_min ? static_cast<T>(prm.u_min[(size_t)prob * su + e]) : pack[L.umin + e];
-                umax[e] = prm.u_max ? static_cast<T>(prm.u_max[(size_t)prob * su + e]) : pack[L.umax + e];
-            }
-            for (int e = lane; e < nu * nx; e += 32) K[e] = pack[L.Kinf + e];
-            for (int e = lane; e < nx * nx; e += 32) P[e] = pack[L.Pinf + e];
-            if (lane == 0) sc[0] = static_cast<T>(prm.rho);
-            __syncwarp();
-        }
-        T rho = sc[0];
-        int iter = 0, status = 11, solved = 0;
-        T r_px = sc[3], r_dx = sc[4], r_pu = sc[5], r_du = sc[6];
-
-        // admm.cpp:295-310 (slack initialisation; overwritten by update_slack before any use)
-        if (soc_x) for (int e = lane; e < sx; e += 32) vcnew[e] = x[e];
-        if (soc_u) for (int e = lane; e < su; e += 32) zcnew[e] = u[e];
-        if (lin_x) for (int e = lane; e < sx; e += 32) vlnew[e] = x[e];
-        if (lin_u) for (int e = lane; e < su; e += 32) zlnew[e] = u[e];
-        __syncwarp();
-
-        for (int it = 0; it < prm.max_iter; ++it) {
-            // ---------------- backward_pass_grad, admm.cpp:13-20
-            for (int i = N - 2; i >= 0; --i) {
-                const T* pn = p + (i + 1) * nx;
-                for (int a = lane; a < nu; a += 32) tmp[a] = col_dot<T, UNR>(B, a, nx, nu, pn) + r[i * nu + a] + BPf[a];
-                __syncwarp();
-                for (int a = lane; a < nu; a += 32) d[i * nu + a] = row_dot<T, UNR>(Quu, a, nu, tmp);
-                for (int c = lane; c < nx; c += 32)
-                    p[i * nx + c] = q[i * nx + c] + row_dot<T, UNR>(AK, c, nx, pn) - col_dot<T, UNR>(K, c, nu, nx, r + i * nu) + APf[c];
-                __syncwarp();
-            }
-            // ---------------- forward_pass, admm.cpp:25-32
-            for (int i = 0; i < N - 1; ++i) {
-                for (int a = lane; a < nu; a += 32) u[i * nu + a] = -row_dot<T, UNR>(K, a, nx, x + i * nx) - d[i * nu + a];
-                __syncwarp();
-                for (int c = lane; c < nx; c += 32)
-                    x[(i + 1) * nx + c] = row_dot<T, UNR>(A, c, nx, x + i * nx) + row_dot<T, UNR>(B, c, nu, u + i * nu) + f[c];
-                __syncwarp();
-            }
-            // ---------------- update_slack, admm.cpp:81-175
-            for (int e = lane; e < sx; e += 32) {
-                T t = x[e] + g[e];
-                if (en_sb) t = tmin(xmax[e], tmax(xmin[e], t));
-                vnew[e] = t;
-                if (soc_x) vcnew[e] = x[e] + gc[e];
-                if (lin_x) vlnew[e] = x[e] + gl[e];
-            }
-            for (int e = lane; e < su; e += 32) {
-                T t = u[e] + y[e];
-                if (en_ib) t = tmin(umax[e], tmax(umin[e], t));
-                znew[e] = t;
-                if (soc_u) zcnew[e] = u[e] + yc[e];
-                if (lin_u) zlnew[e] = u[e] + yl[e];
-            }
-            __syncwarp();
-            if (prm.en_state_soc)
-                for (int i = lane; i < N; i += 32)
-                    for (int c = 0; c < prm.n_state_cones; ++c) project_soc(vcnew + i * nx + prm.Acx[c], prm.qcx[c], prm.cx[c]);
-            if (prm.en_input_soc)
-                for (int i = lane; i < N - 1; i += 32)
-                    for (int c = 0; c < prm.n_input_cones; ++c) project_soc(zcnew + i * nu + prm.Acu[c], prm.qcu[c], prm.cu[c]);
-            if (lin_x)
-                for (int i = lane; i < N; i += 32)
-                    for (int c = 0; c < L.nsl; ++c) {          // sequential in place per column, admm.cpp:149-157
-                        T* col = vlnew + i * nx;
-                        const T val = row_dot<T, UNR>(Alx, c, nx, col);
-                        if (val > blx[c]) {
-                            const T dist = (val - blx[c]) / nrx[c];
-                            for (int j = 0; j < nx; ++j) col[j] -= dist * Alx[c * nx + j];
-                        }
-                    }
-            if (lin_u)
-                for (int i = lane; i < N - 1; i += 32)
-                    for (int c = 0; c < L.nil; ++c) {
-                        T* col = zlnew + i * nu;
-                        const T val = row_dot<T, UNR>(Alu, c, nu, col);
-                        if (val > blu[c]) {
-                            const T dist = (val - blu[c]) / nru[c];
-                            for (int j = 0; j < nu; ++j) col[j] -= dist * Alu[c * nu + j];
-                        }
-                    }
-            __syncwarp();
-            // ---------------- update_dual (admm.cpp:181-208) + update_linear_cost (admm.cpp:214-247)
-            for (int e = lane; e < sx; e += 32) {
-                g[e] = g[e] + x[e] - vnew[e];
-                T qv = -(Xref[e] * Qd[e % nx]);
-                qv -= rho * (vnew[e] - g[e]);
-                if (soc_x) { gc[e] = gc[e] + x[e] - vcnew[e]; qv -= rho * (vcnew[e] - gc[e]); }
-                if (lin_x) { gl[e] = gl[e] + x[e] - vlnew[e]; qv -= rho * (vlnew[e] - gl[e]); }
-                q[e] = qv;
-            }
-            for (int e = lane; e < su; e += 32) {
-                y[e] = y[e] + u[e] - znew[e];
-                T rv = -(Uref[e] * Rd[e % nu]);
-                rv -= rho * (znew[e] - y[e]);
-                if (soc_u) { yc[e] = yc[e] + u[e] - zcnew[e]; rv -= rho * (zcnew[e] - yc[e]); }
-                if (lin_u) { yl[e] = yl[e] + u[e] - zlnew[e]; rv -= rho * (zlnew[e] - yl[e]); }
-                r[e] = rv;
-            }
-            __syncwarp();
-            {
-                const int o = (N - 1) * nx;
-                for (int c = lane; c < nx; c += 32) {           // p_N = -(xref_N' Pinf)' - rho (...)  admm.cpp:238-246
-                    T pv = -col_dot<T, UNR>(P, c, nx, nx, Xref + o);
-                    pv -= rho * (vnew[o + c] - g[o + c]);
-                    if (soc_x) pv -= rho * (vcnew[o + c] - gc[o + c]);
-                    if (lin_x) pv -= rho * (vlnew[o + c] - gl[o + c]);
-                    p[o + c] = pv;
-                }
-            }
-            iter += 1;
-            __syncwarp();
-            // ---------------- adaptive rho, admm.cpp:331-357 / rho_benchmark.cpp:44-250 in closed block form
-            if (prm.adaptive_rho && it > 0 && it % 5 == 0) {
-                T pri = 0, prin = 0, dua = 0, duan = 0;
-                for (int e = lane; e < su; e += 32) {            // input rows: Ax = u, z = znew
-                    pri = tmax(pri, tabs(u[e] - znew[e]));
-                    prin = tmax(prin, tmax(tabs(u[e]), tabs(znew[e])));
-                }
-                for (int e = lane; e < sx - nx; e += 32) {        // dynamics rows i: (A x_i + B u_i - x_{i+1}) - vnew_{i+1} = -f - vnew_{i+1}
-                    const T vv = vnew[nx + e], ff = f[e % nx];
-                    pri = tmax(pri, tabs(ff + vv));
-                    prin = tmax(prin, tmax(tabs(vv), tabs(ff)));
-                }
-                for (int e = lane; e < sx; e += 32) {             // x blocks of P x + q + A'y
-                    const int i = e / nx, c = e % nx;
-                    T px, aty = 0;
-                    const T qx = Qd[c] * x[e];
-                    if (i < N - 1) { px = qx; aty = col_dot<T, UNR>(A, c, nx, nx, g + (i + 1) * nx); } else { px = row_dot<T, UNR>(P, c, nx, x + i * nx); }
-                    if (i >= 1) aty -= g[e];
-                    dua = tmax(dua, tabs(px + qx + aty));
-                    duan = tmax(duan, tmax(tmax(tabs(px), tabs(qx)), tabs(aty)));
-                }
-                for (int e = lane; e < su; e += 32) {             // u blocks
-                    const int i = e / nu, a = e % nu;
-                    const T ru = Rd[a] * u[e];
-                    const T aty = y[e] + col_dot<T, UNR>(B, a, nx, nu, g + (i + 1) * nx);
-                    dua = tmax(dua, tabs(ru + ru + aty));
-                    duan = tmax(duan, tmax(tabs(ru), tabs(aty)));
-                }
-                pri = warp_max(pri); prin = warp_max(prin); dua = warp_max(dua); duan = warp_max(duan);
-                const T eps = T(1e-10);
-                T nr = rho * tsqrt((pri / (prin + eps)) / (dua / (duan + eps) + eps));
-                if (prm.rho_clip) nr = tmin(tmax(nr, static_cast<T>(prm.rho_min)), static_cast<T>(prm.rho_max));
-                const T dr = nr - rho;
-                __syncwarp();
-                for (int e = lane; e < nu * nx; e += 32) K[e] = K[e] + dr * dK[e];    // rho_benchmark.cpp:199-212
-                for (int e = lane; e < nx * nx; e += 32) P[e] = P[e] + dr * dP[e];
-                rho = nr;
-                __syncwarp();
-            }
-            // ---------------- termination_condition, admm.cpp:253-271
-            bool done = false;
-            if (iter % prm.check_termination == 0) {
-                T a = 0, b = 0, c2 = 0, dd = 0;
-                for (int e = lane; e < sx; e += 32) { a = tmax(a, tabs(x[e] - vnew[e])); b = tmax(b, tabs(v[e] - vnew[e])); }
-                for (int e = lane; e < su; e += 32) { c2 = tmax(c2, tabs(u[e] - znew[e])); dd = tmax(dd, tabs(z[e] - znew[e])); }
-                r_px = warp_max(a); r_dx = warp_max(b) * rho; r_pu = warp_max(c2); r_du = warp_max(dd) * rho;
-                done = r_px < tol_pri && r_pu < tol_pri && r_dx < tol_dua && r_du < tol_dua;
-            }
-            if (done) { status = 1; solved = 1; break; }
-            for (int e = lane; e < sx; e += 32) v[e] = vnew[e];      // admm.cpp:379-380
-            for (int e = lane; e < su; e += 32) z[e] = znew[e];
-            __syncwarp();
-        }
-        // ---------------- results
-        if (lane == 0) { sc[0] = rho; sc[1] = static_cast<T>(iter); sc[2] = static_cast<T>(status); sc[3] = r_px; sc[4] = r_dx; sc[5] = r_pu; sc[6] = r_du; sc[7] = static_cast<T>(solved); }
-        if (ws_in_smem && explicit_workspace) {
-            __syncwarp();
-            for (int e = lane; e < W.size; e += 32) gws[e] = ws[e];
-        }
-        if (explicit_workspace != 1 && prm.x) {
-            for (int e = lane; e < sx; e += 32) prm.x[(size_t)prob * sx + e] = static_cast<float>(vnew[e]);
-            for (int e = lane; e < su; e += 32) prm.u[(size_t)prob * su + e] = static_cast<float>(znew[e]);
-            if (lane == 0) {
-                prm.iter[prob] = iter; prm.status[prob] = status;
-                if (prm.residuals) { float* o = prm.residuals + 4 * (size_t)prob; o[0] = (float)r_px; o[1] = (float)r_dx; o[2] = (float)r_pu; o[3] = (float)r_du; }
-                if (prm.rho_out) prm.rho_out[prob] = static_cast<float>(rho);
-            }
-        }
-        __syncwarp();
-    }
+// model batches (tinympc_cuda_solve_batch_models): cold start per problem, one scratch workspace per warp with a model block
+// (WppLayout::make(..., true))
+template <typename T, int NXC, int NUC>
+__global__ void __launch_bounds__(128) wpp_mdl_kernel(const SolveParams prm, const PackLayout L, const T* __restrict__ pack,
+                                                      const WppLayout W, T* __restrict__ scratch, const int ws_in_smem,
+                                                      const tinympc_cuda_models M) {
+    constexpr bool MODELS = true;
+    constexpr int explicit_workspace = 0;
+#include "tmpc_wpp_body.inc"
 }
 
 // ---- session helpers (persistent per-problem workspaces) -------------------------------------------------------
@@ -372,7 +152,7 @@ template cudaError_t wpp_session_init<double>(const SolveParams&, const PackLayo
 template cudaError_t wpp_session_step<float>(const PackLayout&, const void*, const WppLayout&, void*, int, int, cudaStream_t);
 template cudaError_t wpp_session_step<double>(const PackLayout&, const void*, const WppLayout&, void*, int, int, cudaStream_t);
 
-WppLayout WppLayout::make(int nx, int nu, int N) {
+WppLayout WppLayout::make(int nx, int nu, int N, bool models) {
     WppLayout W{};
     const int sx = nx * N, su = nu * (N - 1);
     int o = 0;
@@ -388,13 +168,14 @@ WppLayout WppLayout::make(int nx, int nu, int N) {
     W.Xref = take(sx); W.Uref = take(su);
     W.xmin = take(sx); W.xmax = take(sx); W.umin = take(su); W.umax = take(su);
     W.Kinf = take(nu * nx); W.Pinf = take(nx * nx);
+    if (models) o = WppModelBlock::make(W, nx, nu).end;
     W.size = (o + 3) & ~3;
     return W;
 }
 
 template <typename T>
 cudaError_t wpp_launch(const SolveParams& p, const PackLayout& L, const void* pack, const WppLayout& W, void* scratch, int warps,
-                       int explicit_workspace, cudaStream_t st) {
+                       int explicit_workspace, cudaStream_t st, const tinympc_cuda_models* models) {
     const int block = 128;                       // 4 warps per CTA
     int grid = (warps * 32 + block - 1) / block;
     if (grid < 1) grid = 1;
@@ -406,20 +187,28 @@ cudaError_t wpp_launch(const SolveParams& p, const PackLayout& L, const void* pa
     // solves/s); fp64 ones stay in global memory, where the smaller footprint per CTA keeps more warps resident (13.2 M against
     // 9.2 M solves/s), and so do long horizons that do not fit
     const int in_smem = (sizeof(T) == 4 && smem <= 200 * 1024) ? 1 : 0;
-    auto go = [&](auto kernel) -> cudaError_t {
+    auto go = [&](auto kernel, auto... args) -> cudaError_t {
         if (in_smem && smem > 48 * 1024) {
             cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
             if (e != cudaSuccess) return e;
         }
-        kernel<<<grid, threads, in_smem ? smem : 0, st>>>(p, L, pk, W, sc, explicit_workspace, in_smem);
+        kernel<<<grid, threads, in_smem ? smem : 0, st>>>(p, L, pk, W, sc, args...);
         return cudaGetLastError();
     };
-    if (L.nx == 12 && L.nu == 4) return go(wpp_kernel<T, 12, 4>);
-    if (L.nx == 4 && L.nu == 1) return go(wpp_kernel<T, 4, 1>);
-    if (L.nx == 6 && L.nu == 3) return go(wpp_kernel<T, 6, 3>);
-    return go(wpp_kernel<T, 0, 0>);
+    if (models) {
+        if (L.nx == 12 && L.nu == 4) return go(wpp_mdl_kernel<T, 12, 4>, in_smem, *models);
+        if (L.nx == 4 && L.nu == 1) return go(wpp_mdl_kernel<T, 4, 1>, in_smem, *models);
+        if (L.nx == 6 && L.nu == 3) return go(wpp_mdl_kernel<T, 6, 3>, in_smem, *models);
+        return go(wpp_mdl_kernel<T, 0, 0>, in_smem, *models);
+    }
+    if (L.nx == 12 && L.nu == 4) return go(wpp_kernel<T, 12, 4>, explicit_workspace, in_smem);
+    if (L.nx == 4 && L.nu == 1) return go(wpp_kernel<T, 4, 1>, explicit_workspace, in_smem);
+    if (L.nx == 6 && L.nu == 3) return go(wpp_kernel<T, 6, 3>, explicit_workspace, in_smem);
+    return go(wpp_kernel<T, 0, 0>, explicit_workspace, in_smem);
 }
-template cudaError_t wpp_launch<float>(const SolveParams&, const PackLayout&, const void*, const WppLayout&, void*, int, int, cudaStream_t);
-template cudaError_t wpp_launch<double>(const SolveParams&, const PackLayout&, const void*, const WppLayout&, void*, int, int, cudaStream_t);
+template cudaError_t wpp_launch<float>(const SolveParams&, const PackLayout&, const void*, const WppLayout&, void*, int, int, cudaStream_t,
+                                       const tinympc_cuda_models*);
+template cudaError_t wpp_launch<double>(const SolveParams&, const PackLayout&, const void*, const WppLayout&, void*, int, int, cudaStream_t,
+                                        const tinympc_cuda_models*);
 
 }  // namespace tmpc

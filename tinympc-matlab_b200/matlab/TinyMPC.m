@@ -132,6 +132,32 @@ classdef TinyMPC < handle
             out = struct('states', xs, 'controls', us, 'iter', it, 'status', st, 'residuals', res, 'rho', rho_out);
         end
 
+        function out = solve_batch_models(obj, X0, Xref, Uref, models)
+            % out = solve_batch_models(X0, Xref, Uref, models)
+            % B independent problems that each bring their OWN model: what a loop of setup + solve over solvers with
+            % different dynamics and costs computes, in one GPU call.  This object supplies the horizon, the settings and
+            % the shared bounds and constraints; X0, Xref, Uref as for solve_batch.  models is a struct of double arrays,
+            % one page per problem:
+            %   A nx x nx x B, B nx x nu x B, Q nx x B, R nu x B (diag + rho, as setup stores them), rho 1 x B,
+            %   Kinf nu x nx x B, Pinf nx x nx x B, Quu_inv nu x nu x B, AmBKt nx x nx x B (the cache of each model),
+            %   optional f, APf (nx x B), BPf (nu x B), and dKinf, dPinf (required with adaptive rho).
+            % Returns the fields of solve_batch.
+            obj.require_setup();
+            B = size(X0, 2);
+            Xref = obj.batch_traj(Xref, obj.nx, obj.N, B);
+            Uref = obj.batch_traj(Uref, obj.nu, obj.N-1, B);
+            if ~isstruct(models)
+                error('TinyMPC:InvalidInput', 'models must be a struct of per-problem model arrays');
+            end
+            names = {'A', 'B', 'f', 'Q', 'R', 'rho', 'Kinf', 'Pinf', 'Quu_inv', 'AmBKt', 'APf', 'BPf', 'dKinf', 'dPinf'};
+            arrs = cell(1, numel(names));
+            for k = 1:numel(names)
+                if isfield(models, names{k}), arrs{k} = double(models.(names{k})); else, arrs{k} = []; end
+            end
+            [xs, us, it, st, res, rho_out] = tinympc_matlab('solve_batch_models', X0, Xref, Uref, arrs{:}, false);
+            out = struct('states', xs, 'controls', us, 'iter', it, 'status', st, 'residuals', res, 'rho', rho_out);
+        end
+
         function set_option(obj, name, value)
             % 'precision' 32 (fast, default for batches) | 64 (iteration counts identical to the CPU reference),
             % 'mixed' (band: fp32 pass + fp64 re-solve of the borderline problems), 'chunks', 'ctas_per_sm', 'force_wpp'

@@ -263,6 +263,49 @@ void cmd_solve_batch(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[])
     for (int k = 1; k < 6; ++k) { if (k < nlhs || k == 0) plhs[k] = outs[k]; else mxDestroyArray(outs[k]); }
     if (scalar_int(prhs[7])) mexPrintf("solve_batch: %d problems\n", (int)B);
 }
+// NEW.  [X, U, iter, status, residuals, rho] = tinympc_matlab('solve_batch_models', X0, Xref, Uref, A, B, f, Q, R, rho, Kinf, Pinf,
+//                                                                Quu_inv, AmBKt, APf, BPf, dKinf, dPinf, verbose)
+//   Problems that each bring their own model (tiny_solve_batch_models).  X0, Xref, Uref as for solve_batch; the model arrays are
+//   double, one MATLAB page per problem: A nx x nx x B, B nx x nu x B, Kinf nu x nx x B, Pinf / AmBKt nx x nx x B, Quu_inv nu x nu x B,
+//   Q nx x B, R nu x B (diag + rho, as setup stores them), rho B; f, APf, BPf (nx x B, nx x B, nu x B), dKinf, dPinf may be [].
+void cmd_solve_batch_models(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
+    need_args(nrhs, 18, "solve_batch_models"); need_solver();
+    const TinyWorkspace* w = g_solver->work;
+    const size_t nx = w->nx, nu = w->nu, N = w->N;
+    if (mxGetM(prhs[0]) != nx) fail("InvalidInput", "X0 must be nx x B");
+    const size_t B = mxGetN(prhs[0]);
+    const size_t sx = nx * N * B, su = nu * (N - 1) * B;
+    FloatView x0 = float_view(prhs[0], nx * B), Xr = float_view(prhs[1], sx), Ur = float_view(prhs[2], su);
+    const char* names[14] = {"A", "B", "f", "Q", "R", "rho", "Kinf", "Pinf", "Quu_inv", "AmBKt", "APf", "BPf", "dKinf", "dPinf"};
+    const size_t per[14] = {nx * nx, nx * nu, nx, nx, nu, 1, nu * nx, nx * nx, nu * nu, nx * nx, nx, nu, nu * nx, nx * nx};
+    const double* p[14];
+    for (int k = 0; k < 14; ++k) {
+        const mxArray* a = prhs[3 + k];
+        p[k] = nullptr;
+        if (mxGetNumberOfElements(a) == 0) continue;
+        if (!mxIsDouble(a) || mxIsComplex(a)) fail("InvalidInput", std::string(names[k]) + " must be a real double array");
+        if (mxGetNumberOfElements(a) != per[k] * B)
+            fail("InvalidInput", std::string(names[k]) + " must hold " + std::to_string(per[k]) + " x B values");
+        p[k] = mxGetPr(a);
+    }
+    TinyModelBatch m{p[0], p[1], p[2], p[3], p[4], p[5], p[6], p[7], p[8], p[9], p[10], p[11], p[12], p[13]};
+    const mwSize dx[3] = {(mwSize)nx, (mwSize)N, (mwSize)B}, du[3] = {(mwSize)nu, (mwSize)(N - 1), (mwSize)B};
+    plhs[0] = mxCreateNumericArray(3, dx, mxSINGLE_CLASS, mxREAL);
+    mxArray* U = mxCreateNumericArray(3, du, mxSINGLE_CLASS, mxREAL);
+    const mwSize d1[2] = {(mwSize)B, 1}, d4[2] = {4, (mwSize)B};
+    mxArray* it = mxCreateNumericArray(2, d1, mxINT32_CLASS, mxREAL);
+    mxArray* st = mxCreateNumericArray(2, d1, mxINT32_CLASS, mxREAL);
+    mxArray* rs = mxCreateNumericArray(2, d4, mxSINGLE_CLASS, mxREAL);
+    mxArray* rh = mxCreateNumericArray(2, d1, mxSINGLE_CLASS, mxREAL);
+    TinyBatchIn in{(int)B, x0.ptr, Xr.ptr, Ur.ptr, nullptr, nullptr, nullptr, nullptr};
+    TinyBatchOut out{static_cast<float*>(mxGetData(plhs[0])), static_cast<float*>(mxGetData(U)), static_cast<int*>(mxGetData(it)),
+                     static_cast<int*>(mxGetData(st)), static_cast<float*>(mxGetData(rs)), static_cast<float*>(mxGetData(rh))};
+    const int rc = tiny_solve_batch_models(g_solver, &m, &in, &out);
+    if (rc != 0) fail("SolveBatchFailed", std::string("tiny_solve_batch_models failed: ") + tiny_b200_last_error(g_solver));
+    mxArray* outs[6] = {plhs[0], U, it, st, rs, rh};
+    for (int k = 1; k < 6; ++k) { if (k < nlhs) plhs[k] = outs[k]; else mxDestroyArray(outs[k]); }
+    if (scalar_int(prhs[17])) mexPrintf("solve_batch_models: %d problems\n", (int)B);
+}
 // NEW.  tinympc_matlab('set_option', name, value): 'precision' 32|64, 'chunks', 'ctas_per_sm', 'force_wpp'
 void cmd_set_option(int, mxArray*[], int nrhs, const mxArray* prhs[]) {
     need_args(nrhs, 2, "set_option"); need_solver();
@@ -355,7 +398,7 @@ const Command kCommands[] = {
     {"set_bound_constraints", cmd_set_bound_constraints}, {"set_sensitivity_matrices", cmd_set_sensitivity_matrices},
     {"set_cache_terms", cmd_set_cache_terms}, {"codegen_with_sensitivity", cmd_codegen_with_sensitivity}, {"update_settings", cmd_update_settings},
     {"print_problem_data", cmd_print_problem_data}, {"set_linear_constraints", cmd_set_linear_constraints},
-    {"set_cone_constraints", cmd_set_cone_constraints}, {"solve_batch", cmd_solve_batch}, {"set_option", cmd_set_option},
+    {"set_cone_constraints", cmd_set_cone_constraints}, {"solve_batch", cmd_solve_batch}, {"solve_batch_models", cmd_solve_batch_models}, {"set_option", cmd_set_option},
     {"session_create", cmd_session_create}, {"session_destroy", cmd_session_destroy}, {"session_set_x0", cmd_session_set_x0},
     {"session_set_x_ref", cmd_session_set_x_ref}, {"session_set_u_ref", cmd_session_set_u_ref}, {"session_solve", cmd_session_solve},
     {"session_step", cmd_session_step}, {"session_read", cmd_session_read},
