@@ -248,7 +248,10 @@ int  tinympc_cuda_session_read(tinympc_cuda_session *ss, const char *field, doub
    chunked batches, the concurrent producer / consumer pair inside the streamed host pipeline; -1 always sequential; 0 always the
    pair with 13 % of the SMs left to the consumer; n > 0 the pair with n SMs),
    "variant" (kernel tuning variant, 0 = default; 7 = costate recursion instead of the impulse-response backward pass of the
-   fp32 quadrotor kernels, 5 = direct-form fp32 kernels, 6 = thread-per-problem fp64 kernels, 9 = plain state layout) */
+   fp32 quadrotor kernels, 5 = direct-form fp32 kernels, 6 = thread-per-problem fp64 kernels, 9 = plain state layout),
+   "dense_a" (0 [default]: a family whose float32 A is zero outside the nonzero pattern compiled into an fp32 kernel of its shape
+   -- the bundled quadrotor (12x4x10) and cartpole (4x1x20) families -- runs that sparse-A kernel, whose forward rollout skips the
+   zero coefficient pairs of A; same results up to the sign of an exact zero; 1: always the dense kernel) */
 int  tinympc_cuda_set_option(tinympc_cuda_solver *s, const char *name, double value);
 int  tinympc_cuda_device_count(void);
 int  tinympc_cuda_num_devices(const tinympc_cuda_solver *s);

@@ -63,9 +63,10 @@ def plan_hybrid(nx, nu, N, max_warps=24):
     return None
 
 
-def inst3(nx, nu, N, refs=True, ppb=False, fb=False, variant=0, max_warps=24, opq=False, tib=None, aff=None, feat=BOX, cones=(0, 0, 0, 0, 0, 0), hyb=False, conv=-1):
+def inst3(nx, nu, N, refs=True, ppb=False, fb=False, variant=0, max_warps=24, opq=False, tib=None, aff=None, feat=BOX, cones=(0, 0, 0, 0, 0, 0), hyb=False, conv=-1, sa=None):
     """incremental-form kernel (tmpc_tpp3.cuh): x and t in tensor memory (2 nx N columns per thread), u, u + y, -dd in shared memory;
-    with cones / linear rows (feat=CON) two more arrays of each kind (the pre-projection slacks of the two families)"""
+    with cones / linear rows (feat=CON) two more arrays of each kind (the pre-projection slacks of the two families);
+    sa: the nonzero pattern of A compiled into the forward rollout (a_pattern), None = dense"""
     sx, su = nx * N, nu * (N - 1)
     ntm, nsm = (4, 5) if feat == CON else (2, 3)
     warps = min(max_warps, 4 * (512 // (ntm * sx)), ((226 * 1024 - 1024 - pack_elems(nx, nu, N) * 4) // (nsm * su * 4 * 32) // 4) * 4)
@@ -79,7 +80,7 @@ def inst3(nx, nu, N, refs=True, ppb=False, fb=False, variant=0, max_warps=24, op
     # (quadrotor +3.3 %), unlike the direct form, where the hoisted bounds starved the coefficient stream of the quadrotor instance
     tib = True if tib is None else tib
     return dict(gen=3, bits=32, nx=nx, nu=nu, N=N, feat=feat, refs=3 if refs else 0, ppb=ppb, fb=fb, variant=variant, block=warps * 32, aff=aff,
-                opq=opq, tib=tib, tm=True, minb=1, ntm=ntm, cones=cones, ttm=ttm, conv=conv)
+                opq=opq, tib=tib, tm=True, minb=1, ntm=ntm, cones=cones, ttm=ttm, conv=conv, sa=sa)
 
 
 def inst4(nx, nu, N, refs=True, fb=False, variant=0, aff=None, cones=(0, 0, 0, 0, 0, 0)):
@@ -151,17 +152,49 @@ def plan_block(nx, nu, N, feat, bits, refs, budget_kb=226, tm=False, max_warps=1
     return best[0], best[1]
 
 
+# shapes whose fp32 box instances get a sparse-A twin, and the bundled family each one takes its pattern from
+SPARSE_A_FAMILIES = {(12, 4, 10): "quadrotor", (4, 1, 20): "cartpole"}
+
+
+def load_problems():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("tmpc_build_problems", HERE / "problems.py")
+    mod = importlib.util.module_from_spec(spec)
+    sys.modules[spec.name] = mod        # dataclasses resolve the module of their class through sys.modules
+    spec.loader.exec_module(mod)
+    return mod
+
+
+def a_pattern(A):
+    """nonzero pattern of the float32 conversion of A (the kernels' A) at row-pair granularity: one mask per column, bit j = rows
+    2j, 2j+1, bit nx // 2 = the odd tail row (SparsePairs, tmpc_tpp2.cuh; Family::a_pairs, tmpc_capi.cu)"""
+    import numpy as np
+    A32 = np.asarray(A, dtype=np.float32)
+    nx = A32.shape[0]
+    return tuple(sum(1 << j for j in {r // 2 for r in range(nx) if A32[r, c] != 0}) for c in range(nx))
+
+
+def sparse_a_patterns():
+    P = load_problems()
+    return {shape: a_pattern(getattr(P, fam)().A) for shape, fam in SPARSE_A_FAMILIES.items()}
+
+
 def default_instances():
     out = []
     shapes = [(12, 4, 10), (4, 1, 20), (4, 1, 10), (6, 3, 10)]
+    # sparse A (quadrotor: 26 of the 72 row pairs of A are nonzero, cartpole: 5 of 8): twins of the fp32 box instances whose forward
+    # rollout skips the zero pairs, placed before their dense twins; the dispatcher takes one for a family whose A fits the pattern
+    sparse = sparse_a_patterns()
+    twins = lambda shape: (sparse[shape], None) if shape in sparse else (None,)
     # fp32 box-constrained batches: the incremental ("delta") form, tmpc_tpp3.cuh -- the default (variant 0)
     for (nx, nu, N) in shapes:
         # hybrid state layout where it buys resident warps: the quadrotor shape goes from 8 to 12 warps per SM (+6.7 %)
         hyb = plan_hybrid(nx, nu, N) is not None and plan_hybrid(nx, nu, N)[0] > inst3(nx, nu, N)["block"] // 32
-        for fb in (True, False):      # fb: bounds constant over the horizon and containing 0 (the common case)
-            out.append(inst3(nx, nu, N, refs=True, fb=fb, hyb=hyb))
-            out.append(inst3(nx, nu, N, refs=False, fb=fb, hyb=hyb))
-        out.append(inst3(nx, nu, N, refs=True, ppb=True, hyb=hyb))
+        for sa in twins((nx, nu, N)):
+            for fb in (True, False):      # fb: bounds constant over the horizon and containing 0 (the common case)
+                out.append(inst3(nx, nu, N, refs=True, fb=fb, hyb=hyb, sa=sa))
+                out.append(inst3(nx, nu, N, refs=False, fb=fb, hyb=hyb, sa=sa))
+            out.append(inst3(nx, nu, N, refs=True, ppb=True, hyb=hyb, sa=sa))
     # box + second-order cones + linear inequalities (rocket landing, rocket_landing_constraints.m:40-55: one cone on the
     # first three states, one on the three inputs): the same form with two more slack families, cone blocks compiled in
     # (+ one linear row on each side, SURVEY G4; the last two numbers are the row counts)
@@ -201,10 +234,11 @@ def default_instances():
     # wave of it (tmpc_capi.cu, kLatencyVariant); option variant=9 forces it.
     for (nx, nu, N) in shapes:
         if plan_hybrid(nx, nu, N) is not None and plan_hybrid(nx, nu, N)[0] > inst3(nx, nu, N)["block"] // 32:
-            for fb in (True, False):
-                out.append(inst3(nx, nu, N, refs=True, fb=fb, variant=9))
-                out.append(inst3(nx, nu, N, refs=False, fb=fb, variant=9))
-            out.append(inst3(nx, nu, N, refs=True, ppb=True, variant=9))
+            for sa in twins((nx, nu, N)):
+                for fb in (True, False):
+                    out.append(inst3(nx, nu, N, refs=True, fb=fb, variant=9, sa=sa))
+                    out.append(inst3(nx, nu, N, refs=False, fb=fb, variant=9, sa=sa))
+                out.append(inst3(nx, nu, N, refs=True, ppb=True, variant=9, sa=sa))
     # A/B: the costate recursion instead of the impulse-response form of the backward pass (tmpc_tpp3.cuh, Tpp3Cfg::CONV), option variant=7
     out.append(inst3(12, 4, 10, refs=True, fb=True, hyb=True, variant=7, conv=0))
     # A/B: the direct-form fp32 box kernels (16 / 24 warps per SM, tensor-memory TV) on the headline shapes, option variant=5
@@ -227,7 +261,7 @@ def name_of(i):
     if i["gen"] == 3:
         cn = ("_c" + "".join(str(c) for c in i["cones"])) if i["feat"] == CON else ""
         return (f"tpp3_f32_{i['nx']}x{i['nu']}x{i['N']}_{FEAT_NAME[i['feat']]}{cn}{'' if i['refs'] else '_noref'}{'_ppb' if i['ppb'] else ''}{'_fb' if i['fb'] else ''}"
-                f"{'_aff' if i['aff'] else ''}_v{i['variant']}")
+                f"{'_aff' if i['aff'] else ''}{'_sa' if i.get('sa') else ''}_v{i['variant']}")
     return (f"tpp{'' if i['gen'] == 1 else '2'}_{t}_{i['nx']}x{i['nu']}x{i['N']}_{FEAT_NAME[i['feat']]}{['_noref', '_refsm', ''][i['refs']]}"
             f"{'_ppb' if i['ppb'] else ''}{'_fb' if i['fb'] else ''}{'_aff' if (i['aff'] and i['gen'] == 2) else ''}{'_tm' if i['tm'] else ''}_v{i['variant']}")
 
@@ -272,7 +306,8 @@ def gen_sources(instances):
                 "// generated by tinympc-matlab_b200/build.py -- do not edit\n"
                 '#include "../tmpc_tpp3.cuh"\n#include "../tmpc_registry.h"\nusing namespace tmpc;\n'
                 f"using Cfg_{n} = Tpp3Cfg<{i['nx']}, {i['nu']}, {i['N']}, {i['block']}, {b(i['refs'])}, {b(i['ppb'])}, {b(i['fb'])}, {b(i['aff'])}, "
-                f"{b(i['opq'])}, {b(i['tib'])}, {FEAT_ENUM[i['feat']]}, {', '.join(str(c) for c in i['cones'])}, {i['ttm']}, {i['conv']}>;\n"
+                f"{b(i['opq'])}, {b(i['tib'])}, {FEAT_ENUM[i['feat']]}, {', '.join(str(c) for c in i['cones'])}, {i['ttm']}, {i['conv']}"
+                + (f", SparsePairs<{', '.join(f'{m}u' for m in i['sa'])}>" if i.get("sa") else "") + ">;\n"
                 f"TMPC_DEFINE_TPP3_ENTRY({n}, Cfg_{n}, {i['feat']}, 32, {i['variant']})\n"
             )
         else:

@@ -336,6 +336,8 @@ class CudaSolver:
             pass
 
     def set_option(self, name: str, value: float):
+        """tinympc_cuda_set_option: the option names and values of include/tinympc_b200.h ("precision", "mixed", "variant",
+        "dense_a", ...)"""
         self._check(self.L.tinympc_cuda_set_option(self.h, name.encode(), float(value)))
 
     def set_family(self, fam: dict):

@@ -25,6 +25,7 @@
 
 #include "tmpc_common.h"
 #include "tmpc_registry.h"
+#include "tmpc_sparse_a.h"
 #include "tmpc_wpp.h"
 
 using namespace tmpc;
@@ -86,6 +87,7 @@ struct Family {
     bool shared_bounds_ok = false;     // every enabled bound has shared arrays
     bool fastbox = false;              // shared bounds are constant over the horizon and contain 0
     bool affine = false;               // fdyn (hence APf, BPf) is not identically zero
+    std::vector<unsigned> a_pairs;     // nonzero pattern of the float32 A, as KernelEntry::a_pairs (one row-pair mask per column)
     PackLayout L{};
     std::vector<double> pack;          // double master copy
     SolveParams base{};                // settings + cone specs, pointers empty
@@ -103,6 +105,7 @@ struct tinympc_cuda_solver {
     int variant = 0;
     int force_wpp = 0;                 // option "kernel": 0 auto, 1 always the warp-per-problem kernel
     int refill_min = 0;                // option "refill_min": free lanes a warp collects before it claims new problems (tmpc_tpp3.cuh); 0 = adaptive
+    int dense_a = 0;                   // option "dense_a": 1 = never the sparse-A instances (Tpp3Cfg::SA), always their dense twins
     int streamed = 1;                  // option "streamed": 1 = single-launch streamed host pipeline where it applies, 0 = chunked launches
     int compact_streamed = 1;          // option "compact_streamed": compact host I/O through one launch chain behind an arrival watermark
                                        // (run_shard_compact_streamed); 0 = the chunked pipeline
@@ -180,7 +183,8 @@ void put_vec(std::vector<double>& pk, int at, const double* src, int n) {
     for (int i = 0; i < n; ++i) pk[at + i] = src ? src[i] : 0.0;
 }
 
-const KernelEntry* find_kernel(const Family& f, int bits, bool ppb, bool refs, int variant) {
+// dense_a: skip the sparse-A instances (option "dense_a")
+const KernelEntry* find_kernel(const Family& f, int bits, bool ppb, bool refs, int variant, bool dense_a = false) {
     int n = 0;
     const KernelEntry* const* tab = kernel_table(&n);
     for (int pass = 0; pass < 2; ++pass) {   // pass 1: a reference-storing kernel also serves a reference-free batch
@@ -189,6 +193,8 @@ const KernelEntry* find_kernel(const Family& f, int bits, bool ppb, bool refs, i
             if (e->models) continue;                               // model-batch instances: model_kernel()
             if (e->fastbox && (!f.fastbox || ppb)) continue;      // table order puts the fast-box instances first
             if (f.affine && !e->affine) continue;
+            if (e->a_cols && (dense_a || !a_pattern_covers(e->a_pairs, e->a_cols, f.a_pairs.data(), (int)f.a_pairs.size())))
+                continue;                                          // table order puts the sparse-A instances before their dense twins
             if (e->cone_fixed) {   // cones compiled into the instance: the family's cone list must be exactly that
                 const SolveParams& b = f.base;
                 const bool fsx = b.en_state_soc && b.n_state_cones > 0, fsu = b.en_input_soc && b.n_input_cones > 0;
@@ -202,7 +208,7 @@ const KernelEntry* find_kernel(const Family& f, int bits, bool ppb, bool refs, i
                 return e;
         }
     }
-    if (variant != 0) return find_kernel(f, bits, ppb, refs, 0);
+    if (variant != 0) return find_kernel(f, bits, ppb, refs, 0, dense_a);
     return nullptr;
 }
 
@@ -415,9 +421,9 @@ int upload_family(tinympc_cuda_solver* s) {
 // find_kernel + the small-batch rule: where the default instance uses the hybrid state layout (more resident warps, more
 // instructions per iteration), a batch that fits one wave of the plain-layout instance is latency bound and runs that one.
 const KernelEntry* pick_kernel(const tinympc_cuda_solver* s, const DeviceCtx& d, const Family& f, int bits, bool ppb, bool refs, int batch) {
-    const KernelEntry* ke = find_kernel(f, bits, ppb, refs, s->variant);
+    const KernelEntry* ke = find_kernel(f, bits, ppb, refs, s->variant, s->dense_a);
     if (ke && s->variant == 0 && bits == 32) {
-        const KernelEntry* kl = find_kernel(f, bits, ppb, refs, kLatencyVariant);
+        const KernelEntry* kl = find_kernel(f, bits, ppb, refs, kLatencyVariant, s->dense_a);
         if (kl && kl->variant == kLatencyVariant && kl->block < ke->block && batch <= d.sm_count * kl->block) ke = kl;
     }
     return ke;
@@ -1419,6 +1425,8 @@ int tinympc_cuda_set_family(tinympc_cuda_solver* s, const tinympc_cuda_family* f
     f.shared_bounds_ok = (!sb || have_sb) && (!ib || have_ib);
     for (int r = 0; r < nx; ++r) f.affine = f.affine || f.pack[L.f + r] != 0.0 || f.pack[L.APf + r] != 0.0;
     for (int a = 0; a < nu; ++a) f.affine = f.affine || f.pack[L.BPf + a] != 0.0;
+    f.a_pairs.assign(nx, 0u);
+    a_pairs_of(f.pack.data() + L.A, nx, f.a_pairs.data());
     f.fastbox = true;
     for (int e = 0; e < nx * N && f.fastbox; ++e)
         f.fastbox = f.pack[L.xmin + e] == f.pack[L.xmin + e % nx] && f.pack[L.xmax + e] == f.pack[L.xmax + e % nx] &&
@@ -1900,6 +1908,8 @@ int tinympc_cuda_set_option(tinympc_cuda_solver* s, const char* name, double val
         s->compact_in_kernel = value != 0;
     } else if (n == "refill_min") {
         s->refill_min = (int)value;
+    } else if (n == "dense_a") {
+        s->dense_a = value != 0;
     } else {
         return fail(s, TINYMPC_CUDA_EINVAL, "unknown option " + n);
     }

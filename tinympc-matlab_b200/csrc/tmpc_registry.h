@@ -50,6 +50,10 @@ struct KernelEntry {
     int models;
     cudaError_t (*models_launch)(const SolveParams& p, int grid, size_t smem, cudaStream_t st, const double* master_pack, const PackLayout& L,
                                  const tinympc_cuda_models& m);
+    // sparse-A instances (Tpp3Cfg::SA): the compiled nonzero pattern of A, a_cols (= nx) column masks of row pairs (bit j: rows 2j,
+    // 2j+1; bit nx / 2: the odd tail row).  They serve only families whose float32 A is zero outside it.  a_cols = 0: dense.
+    int a_cols;
+    const unsigned* a_pairs;
 };
 
 const KernelEntry* const* kernel_table(int* count);   // defined in gen/tmpc_table.cu
@@ -99,7 +103,7 @@ const KernelEntry* const* kernel_table(int* count);   // defined in gen/tmpc_tab
     extern const KernelEntry SYM = {#SYM, KF_TPP, CFG::NX, CFG::NU, CFG::NH, FEATV, BITS, CFG::REFMODE,             \
                                     CFG::PPB ? 1 : 0, CFG::FB ? 1 : 0, CFG::AFF ? 1 : 0, CFG::BLOCK, VAR, 1, SYM##_smem, SYM##_prepare, \
                                     SYM##_occ, SYM##_launch, CFG::CONSTR ? 1 : 0, CFG::SCS, CFG::SCD, CFG::UCS, CFG::UCD, CFG::NSL, CFG::NIL, \
-                                    0, nullptr, 1, 1};                                                              \
+                                    0, nullptr, 1, 1, 0, nullptr, CFG::SA::NCOL, CFG::SA::kCols};                  \
     }
 
 // mixed-precision rocket-family kernel (tmpc_tpp4.cuh)

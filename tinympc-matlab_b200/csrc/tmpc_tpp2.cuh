@@ -275,6 +275,66 @@ __device__ __forceinline__ void mv_acc(const T* __restrict__ M0, int z, const Ve
     }
 }
 
+// Compile-time sparsity pattern of a square matrix at row-pair granularity: M = one mask per column, bit j = row pair (2j, 2j+1),
+// bit ROWS / 2 = the odd tail row; an empty list means dense.  A masked product skips the pairs whose coefficients are both zero.
+template <unsigned... M>
+struct SparsePairs {
+    static constexpr int NCOL = static_cast<int>(sizeof...(M));
+    static constexpr bool DENSE = NCOL == 0;
+    static constexpr unsigned kCols[NCOL + 1] = {M..., 0u};   // host side: the registry's copy of the pattern
+    __host__ __device__ static constexpr unsigned col(int c) {
+        unsigned r = 0;
+        int i = 0;
+        ((r |= (i++ == c ? M : 0u)), ...);
+        return r;
+    }
+    // packed coefficients (SparsePairs::pack): the masked pairs column by column, then the masked tail entries
+    __host__ __device__ static constexpr int pairs(int rows) {
+        int n = 0;
+        for (int c = 0; c < NCOL; ++c)
+            for (int j = 0; j < rows / 2; ++j) n += (col(c) >> j) & 1u;
+        return n;
+    }
+    __host__ __device__ static constexpr int packed(int rows) {
+        int n = 2 * pairs(rows);
+        if (rows & 1)
+            for (int c = 0; c < NCOL; ++c) n += (col(c) >> (rows / 2)) & 1u;
+        return n;
+    }
+    template <typename T>
+    static void pack(T* dst, const T* M0, int rows) {   // M0 column-major with stride pad2(rows), as mv_acc reads it
+        const int rp = pad2(rows);
+        int k = 0;
+        for (int c = 0; c < NCOL; ++c)
+            for (int j = 0; j < rows / 2; ++j)
+                if ((col(c) >> j) & 1u) { dst[k++] = M0[c * rp + 2 * j]; dst[k++] = M0[c * rp + 2 * j + 1]; }
+        if (rows & 1)
+            for (int c = 0; c < NCOL; ++c)
+                if ((col(c) >> (rows / 2)) & 1u) dst[k++] = M0[c * rp + rows - 1];
+    }
+};
+
+// acc += M x as mv_acc computes it, for a matrix with the nonzero pattern S, from its packed coefficients MP (SparsePairs::pack):
+// the products of the masked pairs in mv_acc's order, so that the result equals mv_acc's for finite x up to the sign of an
+// exact zero (fma(0, x, acc) = acc).
+template <class S, int ROWS, int COLS, typename T>
+__device__ __forceinline__ void mv_acc_masked(const T* __restrict__ MP, int z, const Vec<T, COLS>& x, Vec<T, ROWS>& acc) {
+    static_assert(S::NCOL == COLS, "pattern of another shape");
+    constexpr int NPAIR = S::pairs(ROWS);
+    const T* __restrict__ M = MP + z;
+    int k = 0, kt = 2 * NPAIR;
+#pragma unroll
+    for (int c = 0; c < COLS; ++c) {
+        const T xc = x.get(c);
+#pragma unroll
+        for (int j = 0; j < ROWS / 2; ++j)
+            if ((S::col(c) >> j) & 1u) { acc.p[j] = fmas(mk2(M[2 * k], M[2 * k + 1]), xc, acc.p[j]); ++k; }
+        if constexpr (ROWS & 1) {
+            if ((S::col(c) >> (ROWS / 2)) & 1u) { acc.t = fmas(M[kt], xc, acc.t); ++kt; }
+        }
+    }
+}
+
 // ----------------------------------------------------------------------------------------------
 // family tables in the kernel-parameter constant bank.  Every matrix is stored COLUMN-major with an
 // even (padded) column stride: the coefficient pair (M[2j][c], M[2j+1][c]) of one FFMA2 is adjacent.

@@ -17,6 +17,7 @@
 //
 // One iteration here (reference order: backward, forward, slack, dual, linear cost, check):
 //   forward : dx_0 = 0, du_i = -Kinf dx_i - dd_i, dx_{i+1} = A dx_i + B du_i;  X += dx, U += du          (admm.cpp:25-32)
+//             (sparse-A instances, Tpp3Cfg::SA: A dx over the compiled nonzero pairs of A only)
 //   sweep   : columns N-1 .. 0, fused: slack + dual + residuals of the column (admm.cpp:81-208, 253-260), the increment
 //             dw of (slack - dual), then the Riccati step on (-rho dw) giving dd for the next forward    (admm.cpp:13-20, 214-247)
 //   check   : admm.cpp:262-265, solution = (vnew, znew)
@@ -48,17 +49,22 @@ enum : int { REFS_STATE = 3 };   // registry "refs" code: reference terms parked
 // (coefficients row-major, offsets b, 1 / ||a||^2 for project_hyperplane, admm.cpp:70-73)
 // CONV: + the impulse-response tables of the backward pass (Tpp3Cfg::CONV): NG[k] = -Quu_inv B' AmBKt^k (k = 0 .. N-2, each NU x NX,
 // column-major like every other table) and NQ = -Quu_inv.
-template <int NX, int NU, int NH, int NSL, int NIL, bool CONV = false>
+// SA (sparse-A instances, Tpp3Cfg::SA): AS = the coefficients of A on SA's nonzero pairs, packed (SparsePairs::pack) for the
+// forward rollout's masked product.
+template <int NX, int NU, int NH, int NSL, int NIL, bool CONV = false, class SA = SparsePairs<>>
 struct alignas(16) ConstPack3 : ConstPack2<float, NX, NU, NH, false> {
     float Alx[NSL > 0 ? NSL * NX : 1], blx[NSL > 0 ? NSL : 1], inx[NSL > 0 ? NSL : 1];
     float Alu[NIL > 0 ? NIL * NU : 1], blu[NIL > 0 ? NIL : 1], inu[NIL > 0 ? NIL : 1];
     float NG[CONV ? (NH - 1) * NX * pad2(NU) : 2], NQ[CONV ? NU * pad2(NU) : 2];
+    float AS[SA::packed(NX) > 2 ? SA::packed(NX) : 2];
 };
-template <int NX, int NU, int NH, int NSL, int NIL, bool CONV>
-inline void fill_const_pack3(ConstPack3<NX, NU, NH, NSL, NIL, CONV>& c, const double* pk, const PackLayout& L) {
+template <int NX, int NU, int NH, int NSL, int NIL, bool CONV, class SA>
+inline void fill_const_pack3(ConstPack3<NX, NU, NH, NSL, NIL, CONV, SA>& c, const double* pk, const PackLayout& L) {
     fill_const_pack2(static_cast<ConstPack2<float, NX, NU, NH, false>&>(c), pk, L);
     c.Alx[0] = c.blx[0] = c.inx[0] = c.Alu[0] = c.blu[0] = c.inu[0] = 0.f;
     c.NG[0] = c.NG[1] = c.NQ[0] = c.NQ[1] = 0.f;
+    c.AS[0] = c.AS[1] = 0.f;
+    if constexpr (!SA::DENSE) SA::pack(c.AS, c.A, NX);
     if constexpr (CONV) {
         constexpr int NUP = pad2(NU);
         double G[NU * NX], Gn[NU * NX];                 // row-major NU x NX, double
@@ -93,7 +99,8 @@ inline void fill_const_pack3(ConstPack3<NX, NU, NH, NSL, NIL, CONV>& c, const do
 }
 
 template <int NX_, int NU_, int NH_, int BLOCK_, bool REFS_, bool PPB_, bool FB_, bool AFF_, bool OPQ_, bool TIB_, int FEAT_ = FEAT_BOX,
-          int SCS_ = 0, int SCD_ = 0, int UCS_ = 0, int UCD_ = 0, int NSL_ = 0, int NIL_ = 0, int TTM_ = -1, int CONV_ = -1>
+          int SCS_ = 0, int SCD_ = 0, int UCS_ = 0, int UCD_ = 0, int NSL_ = 0, int NIL_ = 0, int TTM_ = -1, int CONV_ = -1,
+          class SA_ = SparsePairs<>>
 struct Tpp3Cfg {
     using T = float;
     static_assert(FEAT_ == FEAT_BOX || FEAT_ == FEAT_CONSTR, "the incremental form covers box and box + cone + half-space families");
@@ -124,7 +131,12 @@ struct Tpp3Cfg {
     // scatters -G_k s_j into the -dd slots of the steps before it.  The cost grows with N^2 nu nx against N nx^2, so the form is
     // the default where it matters and is cheap (nx >= 6); the nx = 4 shapes keep the recursion, which is well conditioned there.
     static constexpr bool CONV = CONV_ < 0 ? (NX_ >= 12 && FEAT_ == FEAT_BOX) : (CONV_ != 0);
-    using CPack = ConstPack3<NX_, NU_, NH_, NSL_, NIL_, CONV>;
+    // SPARSE-A instances (SA_ non-empty): the nonzero pattern of A, at row-pair granularity, compiled in.  The forward rollout's
+    // product A dx then issues an FFMA2 only for the pairs of the pattern (26 of 72 on the quadrotor shape), fed from a packed table;
+    // the dispatcher (tmpc_capi.cu find_kernel) runs such an instance only for a family whose float32 A has no nonzero outside it.
+    using SA = SA_;
+    static_assert(SA_::DENSE || SA_::NCOL == NX_, "A pattern of another shape");
+    using CPack = ConstPack3<NX_, NU_, NH_, NSL_, NIL_, CONV, SA_>;
     // HYBRID state layout (TTM_ >= 0, box instances): the 2 nx N columns of x and t per thread cap the quadrotor shape at 8 warps
     // per SM (2 per scheduler, 61 % issue utilisation).  Three observations buy a third warp per scheduler:
     //   * x_0 is the problem's x0, which the lane holds in registers anyway -- column 0 of X is never stored;
@@ -575,7 +587,10 @@ tpp3_kernel(const __grid_constant__ SolveParams prm, const __grid_constant__ typ
                     } else {
                         dxn.fill(T(0));
                     }
-                    if (i > 0 || anyff) mv_acc<NX, NX>(cp.A, zf, dx, dxn);
+                    if (i > 0 || anyff) {
+                        if constexpr (C::SA::DENSE) mv_acc<NX, NX>(cp.A, zf, dx, dxn);
+                        else mv_acc_masked<typename C::SA, NX, NX>(cp.AS, zf, dx, dxn);
+                    }
                     mv_acc<NX, NU>(cp.B, zf, du, dxn);
                     dx = dxn;
                 }
