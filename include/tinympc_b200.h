@@ -218,6 +218,23 @@ int  tinympc_cuda_session_step(tinympc_cuda_session *ss, int use_solution);
  * "x0" batch*nx | "x", "sol_x" batch*nx*N (work->x, solution->x) | "u", "sol_u" batch*nu*(N-1) |
  * "iter", "status", "rho" batch | "residuals" batch*4 */
 int  tinympc_cuda_session_read(tinympc_cuda_session *ss, const char *field, double *host);
+/* Model sessions: `batch` solvers of the family, solver b with the model chunk b of `m` (HOST arrays, the tinympc_cuda_models
+ * layout and rules): the cold workspace and pristine cache of THAT model, i.e. a fresh tiny_setup(A_b, B_b, Q_b, R_b, rho_b) + the
+ * constraint setters.  The family still supplies the shape, the settings, the shared bounds, the cones, the linear rows and the
+ * adaptive-rho flags.  Every session call above works on a model session unchanged; session_step uses each solver's own model
+ * (x0 <- A_b x0 + B_b u0 + f_b) and read("rho") reports each solver's own rho.  Kernels: with "precision" 64 at creation, a box
+ * family without adaptive rho, shared bounds and a compiled shape, the session form of the lane-group kernel's model mode;
+ * otherwise the warp-per-problem kernel.  A missing required array or adaptive rho without the two sensitivities:
+ * TINYMPC_CUDA_EINVAL. */
+int  tinympc_cuda_session_create_models(tinympc_cuda_solver *s, int dev_index, int batch, const tinympc_cuda_models *m,
+                                        tinympc_cuda_session **out);
+/* Replace the model and cache of every solver of a model session (HOST arrays, as for create_models), as a reference user writes
+ * work->Adyn, Bdyn, fdyn, Q, R and the cache (rho, Kinf, Pinf, Quu_inv, AmBKt, APf, BPf, the sensitivities) of a live TinySolver
+ * between two tiny_solve calls: a Kinf, Pinf or rho that adaptive rho has moved is reset to the new model's.  The workspaces (x, u,
+ * q, r, p, d, slacks, duals, references, x0) are kept, so the next solve warm-starts from the previous one under the new model.
+ * One upload and one conversion kernel; no solve.  A session created without models, a missing required array or adaptive rho
+ * without the sensitivities: TINYMPC_CUDA_EINVAL, and the session is left as it was. */
+int  tinympc_cuda_session_set_models(tinympc_cuda_session *ss, const tinympc_cuda_models *m);
 
 /* ---- knobs and introspection ----------------------------------------------------------------- */
 /* option names: "precision" (32 = fp32 arithmetic [default], 64 = fp64 parity mode),

@@ -40,6 +40,7 @@ EXPORTS = [
     "tinympc_cuda_version", "tinympc_cuda_host_alloc", "tinympc_cuda_host_free",
     "tinympc_cuda_session_create", "tinympc_cuda_session_destroy", "tinympc_cuda_session_set_x0", "tinympc_cuda_session_set_x_ref",
     "tinympc_cuda_session_set_u_ref", "tinympc_cuda_session_solve", "tinympc_cuda_session_step", "tinympc_cuda_session_read",
+    "tinympc_cuda_session_create_models", "tinympc_cuda_session_set_models",
     "tinympc_cuda_precompute_batch", "tinympc_cuda_solve_batch_models", "tinympc_cuda_solve_batch_models_device",
 ]
 
@@ -204,6 +205,8 @@ def load():
         L.tinympc_cuda_session_solve.argtypes = [C.c_void_p]
         L.tinympc_cuda_session_step.argtypes = [C.c_void_p, C.c_int]
         L.tinympc_cuda_session_read.argtypes = [C.c_void_p, C.c_char_p, c_dp]
+        L.tinympc_cuda_session_create_models.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(CModels), C.POINTER(C.c_void_p)]
+        L.tinympc_cuda_session_set_models.argtypes = [C.c_void_p, C.POINTER(CModels)]
         L.tinympc_cuda_precompute_batch.argtypes = [C.POINTER(CPrecomputeIn), C.POINTER(CPrecomputeOut)]
         L.tinympc_cuda_solve_batch_models.argtypes = [C.c_void_p, C.POINTER(CModels), C.POINTER(CBatchIn), C.POINTER(CBatchOut)]
         L.tinympc_cuda_solve_batch_models_device.argtypes = [C.c_void_p, C.c_int, C.POINTER(CModels), C.POINTER(CBatchIn), C.POINTER(CBatchOut),
@@ -416,9 +419,10 @@ class CudaSolver:
         solve_batch."""
         return self.solve_batch(x0, models=models, **kw)
 
-    def session(self, batch: int, dev_index: int = 0) -> "CudaSession":
-        """`batch` warm-started solvers of the family, resident on the device (tinympc_cuda_session_*)."""
-        return CudaSession(self, batch, dev_index)
+    def session(self, batch: int, dev_index: int = 0, models: dict | None = None) -> "CudaSession":
+        """`batch` warm-started solvers of the family, resident on the device (tinympc_cuda_session_*).  models: every solver's own
+        model, in the math shapes pack_models takes (tinympc_cuda_session_create_models); None: the family's."""
+        return CudaSession(self, batch, dev_index, models)
 
     # ---- device buffers (raw pointers, e.g. torch.Tensor.data_ptr()) ---------------------------
     def solve_batch_device(self, batch: int, x0, Xref, Uref, x, u, iters, status, residuals=None, rho=None,
@@ -441,11 +445,22 @@ class CudaSession:
     """A batch of warm-started solvers on the device: the closed-loop pattern of the reference
     (tinympc/TinyMPC/examples/quadrotor_hovering.cpp:73-93) for `batch` independent systems at once."""
 
-    def __init__(self, solver: CudaSolver, batch: int, dev_index: int = 0):
+    def __init__(self, solver: CudaSolver, batch: int, dev_index: int = 0, models: dict | None = None):
         self.solver, self.L, self.batch = solver, solver.L, int(batch)
         self.nx, self.nu, self.N = solver.dims
         self.h = C.c_void_p()
-        solver._check(self.L.tinympc_cuda_session_create(solver.h, dev_index, self.batch, C.byref(self.h)))
+        if models is None:
+            solver._check(self.L.tinympc_cuda_session_create(solver.h, dev_index, self.batch, C.byref(self.h)))
+        else:
+            arrays = pack_models(models, self.batch, self.nx, self.nu)
+            solver._check(self.L.tinympc_cuda_session_create_models(solver.h, dev_index, self.batch, C.byref(models_struct(arrays)),
+                                                                    C.byref(self.h)))
+
+    def set_models(self, models: dict):
+        """Replace every solver's model and cache (tinympc_cuda_session_set_models); the workspaces are kept, so the next solve
+        warm-starts under the new models.  `models` as for pack_models."""
+        arrays = pack_models(models, self.batch, self.nx, self.nu)
+        self.solver._check(self.L.tinympc_cuda_session_set_models(self.h, C.byref(models_struct(arrays))))
 
     def close(self):
         if self.h:

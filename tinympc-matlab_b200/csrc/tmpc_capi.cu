@@ -145,6 +145,12 @@ struct tinympc_cuda_session {
     WppLayout W{};
     DevBuf ws, pack, x, u, iter, status;
     std::vector<unsigned char> stage;
+    // model sessions (tinympc_cuda_session_create_models): every solver's model, resident in double (one buffer per field of
+    // tinympc_cuda_models, model_fields), and `dm`, the device view of them; the warp-per-problem kernels read the copy that
+    // wpp_session_models writes into the model block of every workspace
+    bool models = false;
+    DevBuf mdl[14];
+    tinympc_cuda_models dm{};
 };
 
 namespace {
@@ -215,8 +221,8 @@ const KernelEntry* find_kernel(const Family& f, int bits, bool ppb, bool refs, i
 // Model batches (tinympc_cuda_solve_batch_models): the model form of the lane-group fp64 kernel where it applies -- precision 64, a box
 // family without adaptive rho, shared bounds, a compiled shape -- else nullptr: the warp-per-problem kernel in the solver's precision.
 // max_iter <= 0 also takes the warp-per-problem kernel, which runs the reference's zero iterations (the lane-group kernel runs one).
-const KernelEntry* model_kernel(const tinympc_cuda_solver* s, const Family& f, bool ppb) {
-    if (s->force_wpp || s->precision != 64 || f.feat != kFeatBox || ppb || !f.shared_bounds_ok || f.base.max_iter <= 0) return nullptr;
+const KernelEntry* model_kernel(const tinympc_cuda_solver* s, const Family& f, bool ppb, int bits) {
+    if (s->force_wpp || bits != 64 || f.feat != kFeatBox || ppb || !f.shared_bounds_ok || f.base.max_iter <= 0) return nullptr;
     int n = 0;
     const KernelEntry* const* tab = kernel_table(&n);
     for (int i = 0; i < n; ++i)
@@ -508,7 +514,7 @@ bool compact_in_kernel(const tinympc_cuda_solver* s, const DeviceCtx& d, bool pp
     if (ke_out) *ke_out = nullptr;
     if (ke64_out) *ke64_out = nullptr;
     if (models) {
-        const KernelEntry* ke = model_kernel(s, f, ppb);
+        const KernelEntry* ke = model_kernel(s, f, ppb, s->precision);
         return s->compact_in_kernel && ke && ke->compact_ok;
     }
     if (s->force_wpp) return false;
@@ -620,7 +626,7 @@ int enqueue(tinympc_cuda_solver* s, DeviceCtx& d, const tinympc_cuda_batch_in& i
     if (direct < 0) direct = 0;
     const bool refs = in.Xref || in.Uref;
     int bits = s->precision;
-    const KernelEntry* ke = models ? model_kernel(s, f, ppb) : s->force_wpp ? nullptr : pick_kernel(s, d, f, bits, ppb, refs, in.batch);
+    const KernelEntry* ke = models ? model_kernel(s, f, ppb, s->precision) : s->force_wpp ? nullptr : pick_kernel(s, d, f, bits, ppb, refs, in.batch);
     // mixed mode needs the specialised kernels in both precisions; any other shape runs entirely in fp64 (exact as well)
     const KernelEntry* ke64 = nullptr;
     const bool mixed = !models && s->mixed_band > 0 && bits == 32;   // model batches: refused by solve_batch_common
@@ -1312,6 +1318,7 @@ int tinympc_cuda_destroy(tinympc_cuda_solver* s) {
     for (tinympc_cuda_session* ss : s->sessions) {
         cudaSetDevice(s->devs[ss->dev].device);
         for (DevBuf* b : {&ss->ws, &ss->pack, &ss->x, &ss->u, &ss->iter, &ss->status}) b->release();
+        for (DevBuf& b : ss->mdl) b.release();
         ss->s = nullptr;
     }
     s->sessions.clear();
@@ -1479,21 +1486,25 @@ int tinympc_cuda_set_family(tinympc_cuda_solver* s, const tinympc_cuda_family* f
 
 namespace {
 
-// model batches: every required array present (adaptive rho: the two sensitivities too); device pointers 16-byte aligned
-int check_models(tinympc_cuda_solver* s, const tinympc_cuda_models* m, bool device) {
-    if (!m) return TINYMPC_CUDA_OK;
-    if (s->mixed_band > 0 && s->precision == 32)
-        return fail(s, TINYMPC_CUDA_EUNSUPPORTED, "model batches have no exact-count (\"mixed\") form: use \"precision\" 64, which is exact for them");
+// every required array of the family `f` present (adaptive rho: the two sensitivities too); device pointers 16-byte aligned
+int check_model_arrays(tinympc_cuda_solver* s, const Family& f, const tinympc_cuda_models* m, bool device, const char* what) {
     ModelField mf[kModelFields];
-    model_fields(s->fam.nx, s->fam.nu, s->fam.base.adaptive_rho != 0, mf);
+    model_fields(f.nx, f.nu, f.base.adaptive_rho != 0, mf);
     for (int k = 0; k < kModelFields; ++k) {
         const double* p = m->*mf[k].field;
         if (mf[k].required && !p)
-            return fail(s, TINYMPC_CUDA_EINVAL, std::string("model batch: ") + mf[k].name + " is required" +
+            return fail(s, TINYMPC_CUDA_EINVAL, std::string(what) + ": " + mf[k].name + " is required" +
                                                     (k >= 12 ? " (the family has adaptive_rho)" : ""));
         if (device && check_ptr16(s, p, mf[k].name)) return TINYMPC_CUDA_EINVAL;
     }
     return TINYMPC_CUDA_OK;
+}
+// model batches
+int check_models(tinympc_cuda_solver* s, const tinympc_cuda_models* m, bool device) {
+    if (!m) return TINYMPC_CUDA_OK;
+    if (s->mixed_band > 0 && s->precision == 32)
+        return fail(s, TINYMPC_CUDA_EUNSUPPORTED, "model batches have no exact-count (\"mixed\") form: use \"precision\" 64, which is exact for them");
+    return check_model_arrays(s, s->fam, m, device, "model batch");
 }
 
 int solve_batch_device_common(tinympc_cuda_solver* s, int dev_index, const tinympc_cuda_models* m, const tinympc_cuda_batch_in* in,
@@ -1681,17 +1692,47 @@ int tinympc_cuda_solve_workspace(tinympc_cuda_solver* s, const tinympc_cuda_work
 // sessions: persistent per-problem workspaces iterated in place by the warp-per-problem kernel (exact tiny_solve
 // warm-start semantics, tmpc_wpp.cu mode 2)
 // ---------------------------------------------------------------------------------------------------------------
-int tinympc_cuda_session_create(tinympc_cuda_solver* s, int dev_index, int batch, tinympc_cuda_session** out) {
+namespace {
+// host models (the tinympc_cuda_models layout, checked) -> the session's resident copy, then into every workspace's model block,
+// Kinf, Pinf and rho.  The rest of each workspace stays as it is.
+int session_upload_models(tinympc_cuda_session* ss, const tinympc_cuda_models* m) {
+    tinympc_cuda_solver* s = ss->s;
+    DeviceCtx& d = s->devs[ss->dev];
+    DeviceGuard guard;                       // restores the caller's current device on every return path
+    CU(s, cudaSetDevice(d.device));
+    ModelField mf[kModelFields];
+    model_fields(ss->fam.nx, ss->fam.nu, ss->fam.base.adaptive_rho != 0, mf);
+    for (int k = 0; k < kModelFields; ++k) {
+        const double* src = m->*mf[k].field;
+        const size_t bytes = sizeof(double) * mf[k].per_problem * (size_t)ss->batch;
+        if (src) {
+            CU(s, ss->mdl[k].reserve(bytes));
+            CU(s, cudaMemcpy(ss->mdl[k].p, src, bytes, cudaMemcpyHostToDevice));
+        }
+        ss->dm.*mf[k].field = src ? static_cast<const double*>(ss->mdl[k].p) : nullptr;
+    }
+    cudaStream_t st = d.streams[0];
+    const int adaptive = ss->fam.base.adaptive_rho != 0;
+    CU(s, ss->bits == 64 ? wpp_session_models<double>(ss->W, ss->ws.p, ss->batch, ss->fam.nx, ss->fam.nu, ss->dm, adaptive, st)
+                         : wpp_session_models<float>(ss->W, ss->ws.p, ss->batch, ss->fam.nx, ss->fam.nu, ss->dm, adaptive, st));
+    s->launches += 1;
+    CU(s, cudaStreamSynchronize(st));
+    return TINYMPC_CUDA_OK;
+}
+
+int session_create_common(tinympc_cuda_solver* s, int dev_index, int batch, const tinympc_cuda_models* m, tinympc_cuda_session** out) {
     if (!s || !out) return TINYMPC_CUDA_EINVAL;
     *out = nullptr;
     if (!s->fam.set) return fail(s, TINYMPC_CUDA_ENOTREADY, "tinympc_cuda_set_family has not been called");
     if (dev_index < 0 || dev_index >= (int)s->devs.size()) return fail(s, TINYMPC_CUDA_EINVAL, "dev_index out of range");
     if (batch < 1) return fail(s, TINYMPC_CUDA_EINVAL, "session batch must be >= 1");
     if (!s->fam.shared_bounds_ok) return fail(s, TINYMPC_CUDA_EINVAL, "bound constraints are enabled but the family has no bounds");
+    if (m) if (int rc = check_model_arrays(s, s->fam, m, false, "model session")) return rc;
     auto* ss = new tinympc_cuda_session();
     ss->s = s; ss->dev = dev_index; ss->batch = batch; ss->bits = s->precision;
     ss->fam = s->fam;
-    ss->W = WppLayout::make(ss->fam.nx, ss->fam.nu, ss->fam.N);
+    ss->models = m != nullptr;
+    ss->W = WppLayout::make(ss->fam.nx, ss->fam.nu, ss->fam.N, ss->models);
     DeviceCtx& d = s->devs[dev_index];
     int prev = 0;
     cudaGetDevice(&prev);
@@ -1723,8 +1764,33 @@ int tinympc_cuda_session_create(tinympc_cuda_solver* s, int dev_index, int batch
     s->launches += 1;
     cudaSetDevice(prev);
     s->sessions.push_back(ss);
+    if (m) {
+        if (int rc = session_upload_models(ss, m)) { tinympc_cuda_session_destroy(ss); return rc; }
+    }
     *out = ss;
     return TINYMPC_CUDA_OK;
+}
+}  // namespace
+
+int tinympc_cuda_session_create(tinympc_cuda_solver* s, int dev_index, int batch, tinympc_cuda_session** out) {
+    return session_create_common(s, dev_index, batch, nullptr, out);
+}
+
+int tinympc_cuda_session_create_models(tinympc_cuda_solver* s, int dev_index, int batch, const tinympc_cuda_models* m,
+                                       tinympc_cuda_session** out) {
+    if (out) *out = nullptr;
+    if (!m) return s ? fail(s, TINYMPC_CUDA_EINVAL, "model session: models is NULL") : TINYMPC_CUDA_EINVAL;
+    return session_create_common(s, dev_index, batch, m, out);
+}
+
+int tinympc_cuda_session_set_models(tinympc_cuda_session* ss, const tinympc_cuda_models* m) {
+    if (!ss) return TINYMPC_CUDA_EINVAL;
+    tinympc_cuda_solver* s = ss->s;
+    if (!s) return TINYMPC_CUDA_ENOTREADY;   // the solver was destroyed under the session
+    if (!m) return fail(s, TINYMPC_CUDA_EINVAL, "model session: models is NULL");
+    if (!ss->models) return fail(s, TINYMPC_CUDA_EINVAL, "set_models needs a session created with models (tinympc_cuda_session_create_models)");
+    if (int rc = check_model_arrays(s, ss->fam, m, false, "model session")) return rc;
+    return session_upload_models(ss, m);
 }
 
 int tinympc_cuda_session_destroy(tinympc_cuda_session* ss) {
@@ -1734,6 +1800,7 @@ int tinympc_cuda_session_destroy(tinympc_cuda_session* ss) {
         cudaGetDevice(&prev);
         cudaSetDevice(ss->s->devs[ss->dev].device);
         for (DevBuf* b : {&ss->ws, &ss->pack, &ss->x, &ss->u, &ss->iter, &ss->status}) b->release();
+        for (DevBuf& b : ss->mdl) b.release();
         cudaSetDevice(prev);
         auto& v = ss->s->sessions;
         v.erase(std::remove(v.begin(), v.end(), ss), v.end());
@@ -1810,8 +1877,10 @@ int tinympc_cuda_session_solve(tinympc_cuda_session* ss) {
     cudaStream_t st = d.streams[0];
     // fp64 sessions of a box family with a compiled shape run the lane-group kernel on the same workspaces (tmpc_gpp.cuh, session
     // mode): the reference's warm-start semantics at ~4x the rate of the warp-per-problem kernel; option "kernel" = 1 keeps the latter
-    const KernelEntry* kg = (ss->bits == 64 && !s->force_wpp && ss->fam.feat == kFeatBox && ss->fam.shared_bounds_ok) ? find_kernel(ss->fam, 64, false, true, 0) : nullptr;
-    if (kg && !kg->session_launch) kg = nullptr;
+    // Model sessions: the session form of the lane-group kernel's model mode where model batches take the model mode
+    const KernelEntry* kg = ss->models ? model_kernel(s, ss->fam, false, ss->bits)
+                          : (ss->bits == 64 && !s->force_wpp && ss->fam.feat == kFeatBox && ss->fam.shared_bounds_ok) ? find_kernel(ss->fam, 64, false, true, 0) : nullptr;
+    if (kg && !(ss->models ? kg->models_session_launch != nullptr : kg->session_launch != nullptr)) kg = nullptr;
     if (ss->fam.base.max_iter > 0 && kg) {
         const size_t smem = kg->smem_bytes(ss->fam.L.cold_size);
         int occ = 1;
@@ -1821,14 +1890,17 @@ int tinympc_cuda_session_solve(tinympc_cuda_session* ss) {
         const int grid = std::max(1, std::min(d.sm_count * std::max(1, occ), (ss->batch + per_cta - 1) / per_cta));
         p.work_counter = d.counters + kMaxChunks - 1;
         CU(s, cudaMemsetAsync(p.work_counter, 0, sizeof(int), st));
-        CU(s, kg->session_launch(p, grid, smem, st, ss->fam.pack.data(), ss->fam.L, static_cast<double*>(ss->ws.p), ss->W, 0));
+        if (ss->models) CU(s, kg->models_session_launch(p, grid, smem, st, ss->fam.pack.data(), ss->fam.L, static_cast<double*>(ss->ws.p), ss->W, ss->dm));
+        else CU(s, kg->session_launch(p, grid, smem, st, ss->fam.pack.data(), ss->fam.L, static_cast<double*>(ss->ws.p), ss->W, 0));
         s->launches += 1;
         note_kernel(s, std::string(kg->name) + "_session");
     } else if (ss->fam.base.max_iter > 0) {
-        CU(s, ss->bits == 64 ? wpp_launch<double>(p, ss->fam.L, ss->pack.p, ss->W, ss->ws.p, warps, 2, st)
-                             : wpp_launch<float>(p, ss->fam.L, ss->pack.p, ss->W, ss->ws.p, warps, 2, st));
+        const tinympc_cuda_models* mdl = ss->models ? &ss->dm : nullptr;
+        CU(s, ss->bits == 64 ? wpp_launch<double>(p, ss->fam.L, ss->pack.p, ss->W, ss->ws.p, warps, 2, st, mdl)
+                             : wpp_launch<float>(p, ss->fam.L, ss->pack.p, ss->W, ss->ws.p, warps, 2, st, mdl));
         s->launches += 1;
-        note_kernel(s, ss->bits == 64 ? "wpp_f64_session" : "wpp_f32_session");
+        note_kernel(s, ss->models ? (ss->bits == 64 ? "wpp_f64_mdl_session" : "wpp_f32_mdl_session")
+                                  : (ss->bits == 64 ? "wpp_f64_session" : "wpp_f32_session"));
     }
     CU(s, cudaStreamSynchronize(st));
     cudaSetDevice(prev);
@@ -1846,8 +1918,13 @@ int tinympc_cuda_session_step(tinympc_cuda_session* ss, int use_solution) {
     DeviceGuard guard;                       // restores the caller's current device on every return path
     CU(s, cudaSetDevice(d.device));
     cudaStream_t st = d.streams[0];
-    CU(s, ss->bits == 64 ? wpp_session_step<double>(ss->fam.L, ss->pack.p, ss->W, ss->ws.p, ss->batch, use_solution, st)
-                         : wpp_session_step<float>(ss->fam.L, ss->pack.p, ss->W, ss->ws.p, ss->batch, use_solution, st));
+    const int nx = ss->fam.nx, nu = ss->fam.nu;
+    if (ss->models)
+        CU(s, ss->bits == 64 ? wpp_session_step_models<double>(ss->W, ss->ws.p, ss->batch, nx, nu, use_solution, st)
+                             : wpp_session_step_models<float>(ss->W, ss->ws.p, ss->batch, nx, nu, use_solution, st));
+    else
+        CU(s, ss->bits == 64 ? wpp_session_step<double>(ss->fam.L, ss->pack.p, ss->W, ss->ws.p, ss->batch, use_solution, st)
+                             : wpp_session_step<float>(ss->fam.L, ss->pack.p, ss->W, ss->ws.p, ss->batch, use_solution, st));
     s->launches += 1;
     CU(s, cudaStreamSynchronize(st));
     return TINYMPC_CUDA_OK;

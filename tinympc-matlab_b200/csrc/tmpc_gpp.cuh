@@ -36,6 +36,8 @@
 //   workspace (MODE 2)  the same for ONE live workspace, every member written back: tiny_solve
 //   models (MODE 3)     model batches (tinympc_cuda_solve_batch_models): a group that claims a problem loads its lanes' rows from that
 //                       problem's own model and forms the products on the device in the host's order (fill_gpp_tab); box only
+//   model session (MODE 4)  MODE 1 on the workspaces of a model session (tinympc_cuda_session_create_models): the workspace as in
+//                       MODE 1, the lanes' rows from the solver's resident model as in MODE 3
 #pragma once
 #include "tmpc_tpp2.cuh"
 #include "tmpc_wpp.h"
@@ -194,16 +196,17 @@ __device__ __forceinline__ double gabsmax(double r, double a) {
 __device__ __forceinline__ double gclamp(double t, double lo, double hi) { return gmin(hi, gmax(lo, t)); }   // admm.cpp:91-98 order
 
 constexpr int kGppModels = 3;      // gpp_kernel MODE of model batches
+constexpr int kGppModelSession = 4;   // gpp_kernel MODE of model sessions
 
 template <class C, int MODE = 0>   // 0: batch; 1: sessions (what the next warm start reads is written back); 2: tiny_solve on one live workspace (every member);
-                                   // 3: model batch (every problem brings its own matrices and cache, ses.models)
+                                   // 3: model batch (every problem brings its own matrices and cache, ses.models); 4: model session (1 with the rows of 3)
 __global__ void __launch_bounds__(C::BLOCK, C::MINB)
 gpp_kernel(const __grid_constant__ SolveParams prm, const __grid_constant__ GppTab<C::NX, C::NU, C::NH, C::GS, C::ADAPT> tab,
            const __grid_constant__ GppSession ses) {
     // (model mode is tested as MODE == kGppModels: one more constexpr local here changes the machine code of the other modes)
-    constexpr bool SESSION = MODE == 1 || MODE == 2, FULLWS = MODE == 2;
+    constexpr bool SESSION = MODE == 1 || MODE == 2 || MODE == kGppModelSession, FULLWS = MODE == 2;
     static_assert(!(SESSION && C::ADAPT), "adaptive-rho sessions keep a cache per problem: they stay on the warp-per-problem kernel");
-    static_assert(!(MODE == kGppModels && (C::ADAPT || C::CONSTR)), "model batches with adaptive rho, cones or rows stay on the warp-per-problem kernel");
+    static_assert(!((MODE == kGppModels || MODE == kGppModelSession) && (C::ADAPT || C::CONSTR)), "model batches with adaptive rho, cones or rows stay on the warp-per-problem kernel");
     using T = double;
     constexpr int NX = C::NX, NU = C::NU, NH = C::NH, GS = C::GS, NXP = C::NXP, NUP = C::NUP, SXL = C::SX, SUL = C::SU;
     constexpr unsigned FULL = 0xffffffffu;
@@ -344,7 +347,7 @@ gpp_kernel(const __grid_constant__ SolveParams prm, const __grid_constant__ GppT
                 }
 #pragma unroll
                 for (int s = 0; s < NH; ++s) { G[s] = 0; V[s] = 0; RF[s] = 0.f; }
-                if constexpr (MODE == kGppModels) {
+                if constexpr (MODE == kGppModels || MODE == kGppModelSession) {
                     // this lane's rows of the problem's own model (column-major: M(i, j) = M[j * rows + i]), formed exactly as fill_gpp_tab
                     // forms them on the host: the same order, every product and sum rounded on its own (no contraction into an fma)
                     const tinympc_cuda_models& M = ses.models;
@@ -431,7 +434,7 @@ gpp_kernel(const __grid_constant__ SolveParams prm, const __grid_constant__ GppT
                     T acc = 0, acc1 = 0;
 #pragma unroll
                     for (int c = 0; c < NX; ++c) {
-                        if constexpr (MODE == kGppModels) acc = fma(xb[c], ses.models.Pinf[(size_t)prob * NX * NX + row * NX + c], acc);   // Pinf(c, row)
+                        if constexpr (MODE == kGppModels || MODE == kGppModelSession) acc = fma(xb[c], ses.models.Pinf[(size_t)prob * NX * NX + row * NX + c], acc);   // Pinf(c, row)
                         else acc = fma(xb[c], tab.Pinf[c][row], acc);
                         if constexpr (C::ADAPT) acc1 = fma(xb[c], tab.dPinf[c][row], acc1);
                     }

@@ -54,6 +54,10 @@ struct KernelEntry {
     // 2j+1; bit nx / 2: the odd tail row).  They serve only families whose float32 A is zero outside it.  a_cols = 0: dense.
     int a_cols;
     const unsigned* a_pairs;
+    // model sessions (tinympc_cuda_session_create_models): session_launch on workspaces whose solvers each carry their own model, m
+    // (device pointers, every solver's model resident); NULL = the warp-per-problem kernel serves them
+    cudaError_t (*models_session_launch)(const SolveParams& p, int grid, size_t smem, cudaStream_t st, const double* master_pack,
+                                         const PackLayout& L, double* ws, const WppLayout& W, const tinympc_cuda_models& m);
 };
 
 const KernelEntry* const* kernel_table(int* count);   // defined in gen/tmpc_table.cu
@@ -165,7 +169,7 @@ const KernelEntry* const* kernel_table(int* count);   // defined in gen/tmpc_tab
     }
 
 // model-batch form of the lane-group-per-problem fp64 kernel (gpp_kernel MODE 3): the shared bounds come from the family's table,
-// every other row from the claimed problem's model
+// every other row from the claimed problem's model; and its session form (MODE 4, reported as SYM_session)
 #define TMPC_DEFINE_GPP_MDL_ENTRY(SYM, CFG, VAR)                                                                    \
     namespace tmpc {                                                                                                \
     static_assert(!CFG::ADAPT && !CFG::CONSTR, "model batches: box families only");                                 \
@@ -185,7 +189,18 @@ const KernelEntry* const* kernel_table(int* count);   // defined in gen/tmpc_tab
         gpp_kernel<CFG, kGppModels><<<grid, CFG::BLOCK, smem, st>>>(p, tab, ses);                                            \
         return cudaGetLastError();                                                                                  \
     }                                                                                                               \
+    static cudaError_t SYM##_session(const SolveParams& p, int grid, size_t smem, cudaStream_t st, const double* mp,\
+                                     const PackLayout& L, double* ws, const WppLayout& W, const tinympc_cuda_models& m) { \
+        GppTab<CFG::NX, CFG::NU, CFG::NH, CFG::GS, false> tab;                                                      \
+        fill_gpp_tab(tab, mp, L, p);                                                                                \
+        cudaError_t e = cudaFuncSetAttribute(gpp_kernel<CFG, kGppModelSession>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+        if (e != cudaSuccess) return e;                                                                             \
+        GppSession ses{ws, W, 0};                                                                                   \
+        ses.models = m;                                                                                             \
+        gpp_kernel<CFG, kGppModelSession><<<grid, CFG::BLOCK, smem, st>>>(p, tab, ses);                             \
+        return cudaGetLastError();                                                                                  \
+    }                                                                                                               \
     extern const KernelEntry SYM = {#SYM, KF_TPP, CFG::NX, CFG::NU, CFG::NH, 0 /* FEAT_BOX */, 64, 1, 0, 0, 1, CFG::BLOCK, VAR, 0, \
                                     SYM##_smem, SYM##_prepare, SYM##_occ, nullptr, 0, 0, 0, 0, 0, 0, 0, CFG::GS, nullptr, 1, 0, \
-                                    1, SYM##_launch};                                                               \
+                                    1, SYM##_launch, 0, nullptr, SYM##_session};                                    \
     }

@@ -98,6 +98,17 @@ __global__ void __launch_bounds__(128) wpp_mdl_kernel(const SolveParams prm, con
 #include "tmpc_wpp_body.inc"
 }
 
+// model sessions (tinympc_cuda_session_create_models): a persistent workspace per solver (WppLayout::make(..., true)), iterated in
+// place, whose model block holds the solver's own model
+template <typename T, int NXC, int NUC>
+__global__ void __launch_bounds__(128) wpp_mdl_session_kernel(const SolveParams prm, const PackLayout L, const T* __restrict__ pack,
+                                                              const WppLayout W, T* __restrict__ scratch, const int ws_in_smem) {
+    constexpr bool MODELS = true;
+    constexpr int explicit_workspace = 2;
+    [[maybe_unused]] const tinympc_cuda_models M{};
+#include "tmpc_wpp_body.inc"
+}
+
 // ---- session helpers (persistent per-problem workspaces) -------------------------------------------------------
 // cold workspaces as tiny_setup + the constraint setters leave them (tiny_api.cpp:68-105) with the pristine cache
 template <typename T>
@@ -135,6 +146,62 @@ __global__ void wpp_session_step_kernel(const PackLayout L, const T* __restrict_
     __syncwarp();
     if (lane < nx) ws[W.x + lane] = xn;
 }
+
+// every solver's model (column-major double, device) -> the model block, Kinf, Pinf and rho of its workspace, row-major T as
+// set_family packs a family (the conversion wpp_mdl_kernel makes at claim); one warp per solver
+template <typename T>
+__global__ void wpp_session_models_kernel(const WppLayout W, T* __restrict__ wsp, int batch, int nx, int nu, const tinympc_cuda_models M,
+                                          int adaptive) {
+    const int lane = threadIdx.x & 31;
+    const WppModelBlock MB = WppModelBlock::make(W, nx, nu);
+    for (int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; b < batch; b += (gridDim.x * blockDim.x) >> 5) {
+        T* ws = wsp + (size_t)b * W.size;
+        auto cm = [&](int at, const double* src, int rows, int cols) {
+            for (int e = lane; e < rows * cols; e += 32)
+                ws[at + e] = static_cast<T>(src[(size_t)b * rows * cols + (size_t)(e % cols) * rows + e / cols]);
+        };
+        auto vec = [&](int at, const double* src, int n) {
+            for (int e = lane; e < n; e += 32) ws[at + e] = src ? static_cast<T>(src[(size_t)b * n + e]) : T(0);
+        };
+        cm(MB.A, M.Adyn, nx, nx); cm(MB.B, M.Bdyn, nx, nu); cm(W.Kinf, M.Kinf, nu, nx); cm(W.Pinf, M.Pinf, nx, nx);
+        cm(MB.AmBKt, M.AmBKt, nx, nx); cm(MB.Quu_inv, M.Quu_inv, nu, nu);
+        vec(MB.f, M.fdyn, nx); vec(MB.APf, M.APf, nx); vec(MB.BPf, M.BPf, nu); vec(MB.Qd, M.Q, nx); vec(MB.Rd, M.R, nu);
+        if (adaptive) { cm(MB.dKinf, M.dKinf_drho, nu, nx); cm(MB.dPinf, M.dPinf_drho, nx, nx); }
+        if (lane == 0) ws[W.scalars] = static_cast<T>(M.rho[b]);
+    }
+}
+// x0 <- A_b x0 + B_b u0 + f_b with every solver's own model (the model block)
+template <typename T>
+__global__ void wpp_session_step_models_kernel(const WppLayout W, T* __restrict__ wsp, int batch, int nx, int nu, int use_solution) {
+    constexpr int UNR = 1;
+    const int prob = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (prob >= batch) return;
+    T* ws = wsp + (size_t)prob * W.size;
+    const WppModelBlock MB = WppModelBlock::make(W, nx, nu);
+    const T* x0 = ws + W.x;
+    const T* u0 = ws + (use_solution ? W.znew : W.u);
+    T xn = 0;
+    if (lane < nx) xn = row_dot<T, UNR>(ws + MB.A, lane, nx, x0) + row_dot<T, UNR>(ws + MB.B, lane, nu, u0) + ws[MB.f + lane];
+    __syncwarp();
+    if (lane < nx) ws[W.x + lane] = xn;
+}
+
+template <typename T>
+cudaError_t wpp_session_models(const WppLayout& W, void* wsp, int batch, int nx, int nu, const tinympc_cuda_models& m, int adaptive,
+                               cudaStream_t st) {
+    wpp_session_models_kernel<T><<<592, 256, 0, st>>>(W, static_cast<T*>(wsp), batch, nx, nu, m, adaptive);
+    return cudaGetLastError();
+}
+template <typename T>
+cudaError_t wpp_session_step_models(const WppLayout& W, void* wsp, int batch, int nx, int nu, int use_solution, cudaStream_t st) {
+    if (nx > 32) return cudaErrorInvalidValue;
+    wpp_session_step_models_kernel<T><<<(batch + 3) / 4, 128, 0, st>>>(W, static_cast<T*>(wsp), batch, nx, nu, use_solution);
+    return cudaGetLastError();
+}
+template cudaError_t wpp_session_models<float>(const WppLayout&, void*, int, int, int, const tinympc_cuda_models&, int, cudaStream_t);
+template cudaError_t wpp_session_models<double>(const WppLayout&, void*, int, int, int, const tinympc_cuda_models&, int, cudaStream_t);
+template cudaError_t wpp_session_step_models<float>(const WppLayout&, void*, int, int, int, int, cudaStream_t);
+template cudaError_t wpp_session_step_models<double>(const WppLayout&, void*, int, int, int, int, cudaStream_t);
 
 template <typename T>
 cudaError_t wpp_session_init(const SolveParams& p, const PackLayout& L, const void* pack, const WppLayout& W, void* wsp, int batch, cudaStream_t st) {
@@ -195,6 +262,12 @@ cudaError_t wpp_launch(const SolveParams& p, const PackLayout& L, const void* pa
         kernel<<<grid, threads, in_smem ? smem : 0, st>>>(p, L, pk, W, sc, args...);
         return cudaGetLastError();
     };
+    if (models && explicit_workspace == 2) {
+        if (L.nx == 12 && L.nu == 4) return go(wpp_mdl_session_kernel<T, 12, 4>, in_smem);
+        if (L.nx == 4 && L.nu == 1) return go(wpp_mdl_session_kernel<T, 4, 1>, in_smem);
+        if (L.nx == 6 && L.nu == 3) return go(wpp_mdl_session_kernel<T, 6, 3>, in_smem);
+        return go(wpp_mdl_session_kernel<T, 0, 0>, in_smem);
+    }
     if (models) {
         if (L.nx == 12 && L.nu == 4) return go(wpp_mdl_kernel<T, 12, 4>, in_smem, *models);
         if (L.nx == 4 && L.nu == 1) return go(wpp_mdl_kernel<T, 4, 1>, in_smem, *models);

@@ -38,8 +38,10 @@ struct WppModelBlock {
 // explicit_workspace = 1: `scratch` holds ONE fully initialised workspace that is iterated in place
 // (tiny_solve semantics); 0: cold start per problem from p.x0/Xref/Uref, `warps` scratch workspaces;
 // 2: `scratch` holds p.batch persistent workspaces (a session of warm-started solvers), each iterated in place.
-// models (device pointers, explicit_workspace 0 only): every problem iterates with its own model, copied into the model block of
-// the warp's workspace (W made with models = true) when the warp claims it; the family pack then supplies the bounds and rows only
+// models (device pointers, explicit_workspace 0): every problem iterates with its own model, copied into the model block of
+// the warp's workspace (W made with models = true) when the warp claims it; the family pack then supplies the bounds and rows only.
+// explicit_workspace 2 with models non-NULL: a model session, every solver's model already in the model block of its workspace
+// (wpp_session_models; the pointers are not read)
 template <typename T>
 cudaError_t wpp_launch(const SolveParams& p, const PackLayout& L, const void* pack, const WppLayout& W, void* scratch, int warps,
                        int explicit_workspace, cudaStream_t st, const tinympc_cuda_models* models = nullptr);
@@ -49,5 +51,12 @@ template <typename T>
 cudaError_t wpp_session_init(const SolveParams& p, const PackLayout& L, const void* pack, const WppLayout& W, void* wsp, int batch, cudaStream_t st);
 template <typename T>
 cudaError_t wpp_session_step(const PackLayout& L, const void* pack, const WppLayout& W, void* wsp, int batch, int use_solution, cudaStream_t st);
+// model sessions (W made with models = true): every solver's model m (device pointers, column-major double) -> the model block,
+// Kinf, Pinf and rho of its workspace; x0 <- A_b x0 + B_b u0 + f_b with the model block
+template <typename T>
+cudaError_t wpp_session_models(const WppLayout& W, void* wsp, int batch, int nx, int nu, const tinympc_cuda_models& m, int adaptive,
+                               cudaStream_t st);
+template <typename T>
+cudaError_t wpp_session_step_models(const WppLayout& W, void* wsp, int batch, int nx, int nu, int use_solution, cudaStream_t st);
 
 }  // namespace tmpc

@@ -146,14 +146,7 @@ classdef TinyMPC < handle
             B = size(X0, 2);
             Xref = obj.batch_traj(Xref, obj.nx, obj.N, B);
             Uref = obj.batch_traj(Uref, obj.nu, obj.N-1, B);
-            if ~isstruct(models)
-                error('TinyMPC:InvalidInput', 'models must be a struct of per-problem model arrays');
-            end
-            names = {'A', 'B', 'f', 'Q', 'R', 'rho', 'Kinf', 'Pinf', 'Quu_inv', 'AmBKt', 'APf', 'BPf', 'dKinf', 'dPinf'};
-            arrs = cell(1, numel(names));
-            for k = 1:numel(names)
-                if isfield(models, names{k}), arrs{k} = double(models.(names{k})); else, arrs{k} = []; end
-            end
+            arrs = obj.model_arrays(models);
             [xs, us, it, st, res, rho_out] = tinympc_matlab('solve_batch_models', X0, Xref, Uref, arrs{:}, false);
             out = struct('states', xs, 'controls', us, 'iter', it, 'status', st, 'residuals', res, 'rho', rho_out);
         end
@@ -167,10 +160,25 @@ classdef TinyMPC < handle
 
         % ---- sessions: B warm-started copies of this solver on the GPU (closed loops, examples/cartpole_example_mpc.m:36-44,
         % for B systems at once).  Constraints, settings and options are taken as they are when the session is created.
-        function session_create(obj, B)
+        function session_create(obj, B, models)
+            % session_create(B): B copies of this solver.  session_create(B, models): copy b with its own model, page b of
+            % the arrays of models (the struct solve_batch_models takes): the cold workspace and pristine cache of that model.
             obj.require_setup();
-            tinympc_matlab('session_create', B);
+            if nargin < 3
+                tinympc_matlab('session_create', B);
+            else
+                arrs = obj.model_arrays(models);
+                tinympc_matlab('session_create_models', B, arrs{:});
+            end
             obj.session_size = B;
+        end
+
+        function session_set_models(obj, models)
+            % Replace every copy's model and cache (a session created with models); the workspaces are kept, so the next
+            % session_solve warm-starts from the previous one under the new models.
+            obj.require_session();
+            arrs = obj.model_arrays(models);
+            tinympc_matlab('session_set_models', arrs{:});
         end
 
         function session_set_x0(obj, X0)
@@ -314,6 +322,18 @@ classdef TinyMPC < handle
             obj.require_setup();
             if obj.session_size < 1
                 error('TinyMPC:NotSetup', 'No session. Call session_create(B) first.');
+            end
+        end
+
+        function arrs = model_arrays(~, models)
+            % the 14 arrays of a models struct in the order of 'solve_batch_models' ([] for an absent field)
+            if ~isstruct(models)
+                error('TinyMPC:InvalidInput', 'models must be a struct of per-problem model arrays');
+            end
+            names = {'A', 'B', 'f', 'Q', 'R', 'rho', 'Kinf', 'Pinf', 'Quu_inv', 'AmBKt', 'APf', 'BPf', 'dKinf', 'dPinf'};
+            arrs = cell(1, numel(names));
+            for k = 1:numel(names)
+                if isfield(models, names{k}), arrs{k} = double(models.(names{k})); else, arrs{k} = []; end
             end
         end
 

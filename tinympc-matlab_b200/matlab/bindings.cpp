@@ -268,6 +268,21 @@ void cmd_solve_batch(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[])
 //   Problems that each bring their own model (tiny_solve_batch_models).  X0, Xref, Uref as for solve_batch; the model arrays are
 //   double, one MATLAB page per problem: A nx x nx x B, B nx x nu x B, Kinf nu x nx x B, Pinf / AmBKt nx x nx x B, Quu_inv nu x nu x B,
 //   Q nx x B, R nu x B (diag + rho, as setup stores them), rho B; f, APf, BPf (nx x B, nx x B, nu x B), dKinf, dPinf may be [].
+// the 14 model arrays A, B, f, Q, R, rho, Kinf, Pinf, Quu_inv, AmBKt, APf, BPf, dKinf, dPinf at prhs[0..13], B problems; [] = NULL
+void model_arrays(const mxArray* const* a, size_t B, const double* p[14]) {
+    const TinyWorkspace* w = g_solver->work;
+    const size_t nx = w->nx, nu = w->nu;
+    const char* names[14] = {"A", "B", "f", "Q", "R", "rho", "Kinf", "Pinf", "Quu_inv", "AmBKt", "APf", "BPf", "dKinf", "dPinf"};
+    const size_t per[14] = {nx * nx, nx * nu, nx, nx, nu, 1, nu * nx, nx * nx, nu * nu, nx * nx, nx, nu, nu * nx, nx * nx};
+    for (int k = 0; k < 14; ++k) {
+        p[k] = nullptr;
+        if (mxGetNumberOfElements(a[k]) == 0) continue;
+        if (!mxIsDouble(a[k]) || mxIsComplex(a[k])) fail("InvalidInput", std::string(names[k]) + " must be a real double array");
+        if (mxGetNumberOfElements(a[k]) != per[k] * B)
+            fail("InvalidInput", std::string(names[k]) + " must hold " + std::to_string(per[k]) + " x B values");
+        p[k] = mxGetPr(a[k]);
+    }
+}
 void cmd_solve_batch_models(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     need_args(nrhs, 18, "solve_batch_models"); need_solver();
     const TinyWorkspace* w = g_solver->work;
@@ -276,18 +291,8 @@ void cmd_solve_batch_models(int nlhs, mxArray* plhs[], int nrhs, const mxArray* 
     const size_t B = mxGetN(prhs[0]);
     const size_t sx = nx * N * B, su = nu * (N - 1) * B;
     FloatView x0 = float_view(prhs[0], nx * B), Xr = float_view(prhs[1], sx), Ur = float_view(prhs[2], su);
-    const char* names[14] = {"A", "B", "f", "Q", "R", "rho", "Kinf", "Pinf", "Quu_inv", "AmBKt", "APf", "BPf", "dKinf", "dPinf"};
-    const size_t per[14] = {nx * nx, nx * nu, nx, nx, nu, 1, nu * nx, nx * nx, nu * nu, nx * nx, nx, nu, nu * nx, nx * nx};
     const double* p[14];
-    for (int k = 0; k < 14; ++k) {
-        const mxArray* a = prhs[3 + k];
-        p[k] = nullptr;
-        if (mxGetNumberOfElements(a) == 0) continue;
-        if (!mxIsDouble(a) || mxIsComplex(a)) fail("InvalidInput", std::string(names[k]) + " must be a real double array");
-        if (mxGetNumberOfElements(a) != per[k] * B)
-            fail("InvalidInput", std::string(names[k]) + " must hold " + std::to_string(per[k]) + " x B values");
-        p[k] = mxGetPr(a);
-    }
+    model_arrays(prhs + 3, B, p);
     TinyModelBatch m{p[0], p[1], p[2], p[3], p[4], p[5], p[6], p[7], p[8], p[9], p[10], p[11], p[12], p[13]};
     const mwSize dx[3] = {(mwSize)nx, (mwSize)N, (mwSize)B}, du[3] = {(mwSize)nu, (mwSize)(N - 1), (mwSize)B};
     plhs[0] = mxCreateNumericArray(3, dx, mxSINGLE_CLASS, mxREAL);
@@ -326,6 +331,11 @@ void cmd_set_option(int, mxArray*[], int nrhs, const mxArray* prhs[]) {
 //   v = tinympc_matlab('session_read', field)      'x0' nx x B | 'x','sol_x' nx x N x B | 'u','sol_u' nu x (N-1) x B |
 //                                                  'iter','status','rho' B x 1 | 'residuals' 4 x B      (doubles)
 //   tinympc_matlab('session_destroy')
+//   tinympc_matlab('session_create_models', B, A, B, f, Q, R, rho, Kinf, Pinf, Quu_inv, AmBKt, APf, BPf, dKinf, dPinf)
+//                                                  B copies, copy b with its own model (the arrays of 'solve_batch_models'):
+//                                                  cold workspace + pristine cache of that model (tinympc_cuda_session_create_models)
+//   tinympc_matlab('session_set_models', A, B, f, Q, R, rho, Kinf, Pinf, Quu_inv, AmBKt, APf, BPf, dKinf, dPinf)
+//                                                  replace every copy's model and cache, keep the workspaces (warm start)
 void need_session() { if (!g_session) fail("NotInitialized", "No session: call session_create first"); }
 void session_check(int rc, const char* what) {
     if (rc != 0) fail("SessionFailed", std::string(what) + ": " + tinympc_cuda_last_error(static_cast<tinympc_cuda_solver*>(tiny_b200_cuda_handle(g_solver))));
@@ -348,6 +358,27 @@ void cmd_session_create(int, mxArray*[], int nrhs, const mxArray* prhs[]) {
     const int rc = tinympc_cuda_session_create(h, 0, B, &g_session);
     if (rc != 0) { g_session = nullptr; fail("SessionFailed", std::string("session_create: ") + tinympc_cuda_last_error(h)); }
     g_session_batch = B;
+}
+void cmd_session_create_models(int, mxArray*[], int nrhs, const mxArray* prhs[]) {
+    need_args(nrhs, 15, "session_create_models"); need_solver();
+    const int B = scalar_int(prhs[0]);
+    if (B < 1) fail("InvalidInput", "session_create_models requires a positive number of problems");
+    const double* p[14];
+    model_arrays(prhs + 1, (size_t)B, p);
+    drop_session();
+    auto* h = static_cast<tinympc_cuda_solver*>(tiny_b200_cuda_handle(g_solver));
+    if (!h) fail("SessionFailed", std::string("no GPU backend: ") + tiny_b200_last_error(g_solver));
+    const tinympc_cuda_models m{p[0], p[1], p[2], p[3], p[4], p[5], p[6], p[7], p[8], p[9], p[10], p[11], p[12], p[13]};
+    const int rc = tinympc_cuda_session_create_models(h, 0, B, &m, &g_session);
+    if (rc != 0) { g_session = nullptr; fail("SessionFailed", std::string("session_create_models: ") + tinympc_cuda_last_error(h)); }
+    g_session_batch = B;
+}
+void cmd_session_set_models(int, mxArray*[], int nrhs, const mxArray* prhs[]) {
+    need_args(nrhs, 14, "session_set_models"); need_solver(); need_session();
+    const double* p[14];
+    model_arrays(prhs, (size_t)g_session_batch, p);
+    const tinympc_cuda_models m{p[0], p[1], p[2], p[3], p[4], p[5], p[6], p[7], p[8], p[9], p[10], p[11], p[12], p[13]};
+    session_check(tinympc_cuda_session_set_models(g_session, &m), "session_set_models");
 }
 void cmd_session_destroy(int, mxArray*[], int, const mxArray*[]) { drop_session(); }
 void cmd_session_set_x0(int, mxArray*[], int nrhs, const mxArray* prhs[]) {
@@ -399,7 +430,8 @@ const Command kCommands[] = {
     {"set_cache_terms", cmd_set_cache_terms}, {"codegen_with_sensitivity", cmd_codegen_with_sensitivity}, {"update_settings", cmd_update_settings},
     {"print_problem_data", cmd_print_problem_data}, {"set_linear_constraints", cmd_set_linear_constraints},
     {"set_cone_constraints", cmd_set_cone_constraints}, {"solve_batch", cmd_solve_batch}, {"solve_batch_models", cmd_solve_batch_models}, {"set_option", cmd_set_option},
-    {"session_create", cmd_session_create}, {"session_destroy", cmd_session_destroy}, {"session_set_x0", cmd_session_set_x0},
+    {"session_create", cmd_session_create}, {"session_create_models", cmd_session_create_models},
+    {"session_set_models", cmd_session_set_models}, {"session_destroy", cmd_session_destroy}, {"session_set_x0", cmd_session_set_x0},
     {"session_set_x_ref", cmd_session_set_x_ref}, {"session_set_u_ref", cmd_session_set_u_ref}, {"session_solve", cmd_session_solve},
     {"session_step", cmd_session_step}, {"session_read", cmd_session_read},
 };
