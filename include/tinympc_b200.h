@@ -177,8 +177,11 @@ int  tinympc_cuda_solve_workspace(tinympc_cuda_solver *s, const tinympc_cuda_wor
 /* ---- batched cache precompute + rho-sensitivities on the device ------------------------------------ */
 /* replaces tiny_precompute_and_set_cache (tinympc/TinyMPC/src/tinympc/tiny_api.cpp:244-318) looped over problems that each
  * bring their OWN dynamics and costs, and TinyMPC.compute_sensitivity_autograd (src/TinyMPC.m:223-241: forward difference in rho,
- * h = 1e-6, both ends solved to 1e-10) for the derivatives adaptive rho needs.  All arrays are HOST, double, one contiguous
- * column-major chunk per problem (Eigen's layout); Q and R are the user's diagonals (before "+ rho").  Runs on the current device. */
+ * h = 1e-6, both ends solved to 1e-10) for the derivatives adaptive rho needs.  All arrays are double, one contiguous column-major
+ * chunk per problem (Eigen's layout, and the layout of tinympc_cuda_models: the outputs serve as the model arrays unchanged).  Q and R
+ * are the diagonals tiny_precompute_and_set_cache receives, to which it adds rho.  tiny_setup hands it work->Q = diag(Q) + rho
+ * (quirk Q1 of the reference: rho is added twice), so the cache of a model whose tinympc_cuda_models Q and R are diag + rho, as
+ * tiny_setup stores them, comes from passing THOSE arrays here as Q and R.  Runs on the current device. */
 typedef struct {
     int batch, nx, nu;                 /* nx <= 16, nu <= 8 */
     const double *Adyn, *Bdyn;         /* batch*nx*nx, batch*nx*nu */
@@ -191,7 +194,12 @@ typedef struct {
     double *dKinf_drho, *dPinf_drho, *dC1_drho, *dC2_drho;   /* optional (give the first two to get any); C1 = Quu_inv, C2 = AmBKt */
     int *iters;                        /* batch or NULL: Riccati iterations until max|Kinf - Kprev| < 1e-5 (at most 1000) */
 } tinympc_cuda_precompute_out;
+/* HOST arrays: upload, kernel, download; returns when the results are on the host */
 int  tinympc_cuda_precompute_batch(const tinympc_cuda_precompute_in *in, const tinympc_cuda_precompute_out *out);
+/* DEVICE arrays of the current device (16-byte aligned), e.g. the model arrays of a tinympc_cuda_models: the same kernel, enqueued
+ * on `stream` (a cudaStream_t, NULL = the default stream); no allocation, copy or synchronisation.  A missing required array, or
+ * an array that is not aligned device (or managed) memory of the current device: TINYMPC_CUDA_EINVAL, nothing queued. */
+int  tinympc_cuda_precompute_batch_device(const tinympc_cuda_precompute_in *in, const tinympc_cuda_precompute_out *out, void *stream);
 
 /* ---- sessions: a batch of warm-started solvers resident on the device ------------------------- */
 /* The closed-loop pattern of the reference (tinympc/TinyMPC/examples/quadrotor_hovering.cpp:73-93,
@@ -199,7 +207,8 @@ int  tinympc_cuda_precompute_batch(const tinympc_cuda_precompute_in *in, const t
  * workspace persists between solves (admm.cpp starts from the q, r, p, d, duals and slacks of the previous solve).
  * A session is `batch` such solvers of the family, each with its own complete TinyWorkspace and cache copy
  * (types.hpp:43-187) in device memory; every call below acts on all of them.  Arithmetic follows the "precision" option
- * at creation (64 reproduces the reference's iteration counts exactly).  All array arguments are HOST pointers. */
+ * at creation (64 reproduces the reference's iteration counts exactly).  All array arguments are HOST pointers (the _device entries
+ * further down take device pointers). */
 typedef struct tinympc_cuda_session tinympc_cuda_session;
 /* `batch` solvers as tiny_setup + the constraint setters leave them (cold workspaces, pristine cache), on device `dev_index` */
 int  tinympc_cuda_session_create(tinympc_cuda_solver *s, int dev_index, int batch, tinympc_cuda_session **out);
@@ -235,6 +244,28 @@ int  tinympc_cuda_session_create_models(tinympc_cuda_solver *s, int dev_index, i
  * One upload and one conversion kernel; no solve.  A session created without models, a missing required array or adaptive rho
  * without the sensitivities: TINYMPC_CUDA_EINVAL, and the session is left as it was. */
 int  tinympc_cuda_session_set_models(tinympc_cuda_session *ss, const tinympc_cuda_models *m);
+
+/* ---- sessions fed from device memory ----------------------------------------------------------------------------------------------
+ * The closed loop of a simulator or a linearisation that keeps its data on the GPU: relinearise every solver about its state,
+ * compute the caches (tinympc_cuda_precompute_batch_device writes them straight into the model arrays), set_models_device, solve,
+ * step, read_device.  All arrays are DEVICE pointers: 16-byte aligned device (or managed) memory of the session's device, doubles.
+ * Stream contract of the entries below: each runs after all work the caller queued on `stream` (a cudaStream_t, NULL = the default
+ * stream) before the call, and work the caller queues on `stream` after the call runs after it.  The host is not blocked, except by
+ * a first-time buffer allocation (create_models_device, and a model field set for the first time).  The work runs on the session's
+ * own stream, ordered by events; every host-pointer session call, tinympc_cuda_session_destroy and tinympc_cuda_destroy first
+ * waits for it.  session_solve and session_step stay host-synchronous.  Failed validation (a NULL required array, a misaligned
+ * pointer or one that is not device memory of the session's device, an unknown field, set_models_device on a session created
+ * without models): TINYMPC_CUDA_EINVAL before anything is queued, the session left as it was. */
+/* tinympc_cuda_session_create_models / _set_models with the model arrays of `m` on the device (device-to-device copies into the
+   session's resident model buffers, then the conversion into the workspaces) */
+int  tinympc_cuda_session_create_models_device(tinympc_cuda_solver *s, int dev_index, int batch, const tinympc_cuda_models *m,
+                                               void *stream, tinympc_cuda_session **out);
+int  tinympc_cuda_session_set_models_device(tinympc_cuda_session *ss, const tinympc_cuda_models *m, void *stream);
+/* the setters from device memory: field "x0" (batch*nx), "Xref" (batch*nx*N) or "Uref" (batch*nu*(N-1)); broadcast 1: src is ONE
+   solver's array, shared by all, as for the host setters.  src is required. */
+int  tinympc_cuda_session_write_device(tinympc_cuda_session *ss, const char *field, const double *src, int broadcast, void *stream);
+/* session_read into device memory: every field session_read accepts, the same layout, doubles */
+int  tinympc_cuda_session_read_device(tinympc_cuda_session *ss, const char *field, double *dst, void *stream);
 
 /* ---- knobs and introspection ----------------------------------------------------------------- */
 /* option names: "precision" (32 = fp32 arithmetic [default], 64 = fp64 parity mode),

@@ -41,6 +41,8 @@ EXPORTS = [
     "tinympc_cuda_session_create", "tinympc_cuda_session_destroy", "tinympc_cuda_session_set_x0", "tinympc_cuda_session_set_x_ref",
     "tinympc_cuda_session_set_u_ref", "tinympc_cuda_session_solve", "tinympc_cuda_session_step", "tinympc_cuda_session_read",
     "tinympc_cuda_session_create_models", "tinympc_cuda_session_set_models",
+    "tinympc_cuda_session_create_models_device", "tinympc_cuda_session_set_models_device", "tinympc_cuda_session_write_device",
+    "tinympc_cuda_session_read_device", "tinympc_cuda_precompute_batch_device",
     "tinympc_cuda_precompute_batch", "tinympc_cuda_solve_batch_models", "tinympc_cuda_solve_batch_models_device",
 ]
 
@@ -166,6 +168,23 @@ def precompute_batch(A, B, Q, R, rho, f=None, sensitivities=False) -> dict:
     return o
 
 
+PRECOMPUTE_OUT_FIELDS = ("Kinf", "Pinf", "Quu_inv", "AmBKt", "APf", "BPf", "dKinf_drho", "dPinf_drho", "dC1_drho", "dC2_drho", "iters")
+
+
+def precompute_batch_device(batch: int, nx: int, nu: int, A, B, Q, R, rho, out: dict, f=None, stream=None):
+    """tinympc_cuda_precompute_batch_device: device pointers (ints, e.g. torch.Tensor.data_ptr()) of float64 arrays on the current
+    device, column-major per problem (pack_models' layout).  A, B, Q, R, rho, f as for precompute_batch (f may be None); out maps
+    PRECOMPUTE_OUT_FIELDS names to pointers (Kinf .. BPf required; dKinf_drho and dPinf_drho to get the sensitivities; iters is
+    int32).  Enqueued on `stream` (cudaStream_t as an int, None = the default stream); returns without waiting."""
+    L = load()
+    dp = lambda v: None if v is None else C.cast(C.c_void_p(v), c_dp)
+    cin = CPrecomputeIn(batch, nx, nu, dp(A), dp(B), dp(f), dp(Q), dp(R), dp(rho))
+    co = CPrecomputeOut(*[dp(out.get(k)) for k in PRECOMPUTE_OUT_FIELDS[:-1]], C.cast(C.c_void_p(out["iters"]), c_ip) if out.get("iters") else None)
+    rc = L.tinympc_cuda_precompute_batch_device(C.byref(cin), C.byref(co), stream)
+    if rc:
+        raise TinympcCudaError(rc, "tinympc_cuda_precompute_batch_device failed")
+
+
 def load():
     """Load the in-tree CUDA library; raises if it has not been built (no fallback)."""
     global _lib
@@ -208,6 +227,12 @@ def load():
         L.tinympc_cuda_session_create_models.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(CModels), C.POINTER(C.c_void_p)]
         L.tinympc_cuda_session_set_models.argtypes = [C.c_void_p, C.POINTER(CModels)]
         L.tinympc_cuda_precompute_batch.argtypes = [C.POINTER(CPrecomputeIn), C.POINTER(CPrecomputeOut)]
+        L.tinympc_cuda_precompute_batch_device.argtypes = [C.POINTER(CPrecomputeIn), C.POINTER(CPrecomputeOut), C.c_void_p]
+        L.tinympc_cuda_session_create_models_device.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(CModels), C.c_void_p,
+                                                                C.POINTER(C.c_void_p)]
+        L.tinympc_cuda_session_set_models_device.argtypes = [C.c_void_p, C.POINTER(CModels), C.c_void_p]
+        L.tinympc_cuda_session_write_device.argtypes = [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int, C.c_void_p]
+        L.tinympc_cuda_session_read_device.argtypes = [C.c_void_p, C.c_char_p, C.c_void_p, C.c_void_p]
         L.tinympc_cuda_solve_batch_models.argtypes = [C.c_void_p, C.POINTER(CModels), C.POINTER(CBatchIn), C.POINTER(CBatchOut)]
         L.tinympc_cuda_solve_batch_models_device.argtypes = [C.c_void_p, C.c_int, C.POINTER(CModels), C.POINTER(CBatchIn), C.POINTER(CBatchOut),
                                                              C.c_void_p]
@@ -419,10 +444,13 @@ class CudaSolver:
         solve_batch."""
         return self.solve_batch(x0, models=models, **kw)
 
-    def session(self, batch: int, dev_index: int = 0, models: dict | None = None) -> "CudaSession":
+    def session(self, batch: int, dev_index: int = 0, models: dict | None = None, models_device: dict | None = None,
+                stream=None) -> "CudaSession":
         """`batch` warm-started solvers of the family, resident on the device (tinympc_cuda_session_*).  models: every solver's own
-        model, in the math shapes pack_models takes (tinympc_cuda_session_create_models); None: the family's."""
-        return CudaSession(self, batch, dev_index, models)
+        model, in the math shapes pack_models takes (tinympc_cuda_session_create_models); models_device: the same as device pointers
+        by CModels field name, as for solve_batch_models_device (tinympc_cuda_session_create_models_device, enqueued on `stream`);
+        neither: the family's."""
+        return CudaSession(self, batch, dev_index, models, models_device, stream)
 
     # ---- device buffers (raw pointers, e.g. torch.Tensor.data_ptr()) ---------------------------
     def solve_batch_device(self, batch: int, x0, Xref, Uref, x, u, iters, status, residuals=None, rho=None,
@@ -445,11 +473,15 @@ class CudaSession:
     """A batch of warm-started solvers on the device: the closed-loop pattern of the reference
     (tinympc/TinyMPC/examples/quadrotor_hovering.cpp:73-93) for `batch` independent systems at once."""
 
-    def __init__(self, solver: CudaSolver, batch: int, dev_index: int = 0, models: dict | None = None):
+    def __init__(self, solver: CudaSolver, batch: int, dev_index: int = 0, models: dict | None = None, models_device: dict | None = None,
+                 stream=None):
         self.solver, self.L, self.batch = solver, solver.L, int(batch)
         self.nx, self.nu, self.N = solver.dims
         self.h = C.c_void_p()
-        if models is None:
+        if models_device is not None:
+            solver._check(self.L.tinympc_cuda_session_create_models_device(solver.h, dev_index, self.batch,
+                                                                           C.byref(models_struct(models_device)), stream, C.byref(self.h)))
+        elif models is None:
             solver._check(self.L.tinympc_cuda_session_create(solver.h, dev_index, self.batch, C.byref(self.h)))
         else:
             arrays = pack_models(models, self.batch, self.nx, self.nu)
@@ -461,6 +493,21 @@ class CudaSession:
         warm-starts under the new models.  `models` as for pack_models."""
         arrays = pack_models(models, self.batch, self.nx, self.nu)
         self.solver._check(self.L.tinympc_cuda_session_set_models(self.h, C.byref(models_struct(arrays))))
+
+    # ---- device buffers (raw pointers of float64 arrays on the session's device); enqueued on `stream`, see the header's stream
+    # contract --------------------------------------------------------------------------------------------------------------------
+    def set_models_device(self, models: dict, stream=None):
+        """tinympc_cuda_session_set_models_device: models maps CModels field names to device pointers (pack_models' layout)"""
+        self.solver._check(self.L.tinympc_cuda_session_set_models_device(self.h, C.byref(models_struct(models)), stream))
+
+    def write_device(self, field: str, src: int, broadcast: bool = False, stream=None):
+        """tinympc_cuda_session_write_device: field "x0" (B, nx), "Xref" (B, N, nx) or "Uref" (B, N-1, nu); broadcast: src holds one
+        solver's array, shared by all"""
+        self.solver._check(self.L.tinympc_cuda_session_write_device(self.h, field.encode(), src, 1 if broadcast else 0, stream))
+
+    def read_device(self, field: str, dst: int, stream=None):
+        """tinympc_cuda_session_read_device: any field read() takes, as doubles in read()'s shape (iter and status too)"""
+        self.solver._check(self.L.tinympc_cuda_session_read_device(self.h, field.encode(), dst, stream))
 
     def close(self):
         if self.h:

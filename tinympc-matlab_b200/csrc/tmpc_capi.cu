@@ -24,6 +24,7 @@
 #include <vector>
 
 #include "tmpc_common.h"
+#include "tmpc_devptr.h"
 #include "tmpc_registry.h"
 #include "tmpc_sparse_a.h"
 #include "tmpc_wpp.h"
@@ -151,6 +152,9 @@ struct tinympc_cuda_session {
     bool models = false;
     DevBuf mdl[14];
     tinympc_cuda_models dm{};
+    // the device-resident entries (tinympc_cuda_session_*_device) order their work on streams[0] against the caller's stream with
+    // these: ev_in recorded on the caller's stream, ev_out on streams[0]
+    cudaEvent_t ev_in = nullptr, ev_out = nullptr;
 };
 
 namespace {
@@ -1317,8 +1321,10 @@ int tinympc_cuda_destroy(tinympc_cuda_solver* s) {
     // TINYMPC_CUDA_ENOTREADY instead of dereferencing the freed solver, and session_destroy still releases the handle
     for (tinympc_cuda_session* ss : s->sessions) {
         cudaSetDevice(s->devs[ss->dev].device);
+        cudaStreamSynchronize(s->devs[ss->dev].streams[0]);   // work a device-resident session entry left queued
         for (DevBuf* b : {&ss->ws, &ss->pack, &ss->x, &ss->u, &ss->iter, &ss->status}) b->release();
         for (DevBuf& b : ss->mdl) b.release();
+        for (cudaEvent_t* ev : {&ss->ev_in, &ss->ev_out}) if (*ev) { cudaEventDestroy(*ev); *ev = nullptr; }
         ss->s = nullptr;
     }
     s->sessions.clear();
@@ -1693,41 +1699,76 @@ int tinympc_cuda_solve_workspace(tinympc_cuda_solver* s, const tinympc_cuda_work
 // warm-start semantics, tmpc_wpp.cu mode 2)
 // ---------------------------------------------------------------------------------------------------------------
 namespace {
-// host models (the tinympc_cuda_models layout, checked) -> the session's resident copy, then into every workspace's model block,
-// Kinf, Pinf and rho.  The rest of each workspace stays as it is.
-int session_upload_models(tinympc_cuda_session* ss, const tinympc_cuda_models* m) {
+// Stream contract of the device-resident session entries (include/tinympc_b200.h): the session's stream waits for the work the
+// caller queued on `caller` before the call; after the entry has queued its own work there, `caller` waits for that.  The host
+// entries copy on the legacy stream, which does not order against the non-blocking streams[0]: they call session_wait first.
+cudaError_t session_begin(tinympc_cuda_session* ss, cudaStream_t caller) {
+    cudaError_t e = cudaEventRecord(ss->ev_in, caller);
+    return e == cudaSuccess ? cudaStreamWaitEvent(ss->s->devs[ss->dev].streams[0], ss->ev_in, 0) : e;
+}
+cudaError_t session_end(tinympc_cuda_session* ss, cudaStream_t caller) {
+    cudaError_t e = cudaEventRecord(ss->ev_out, ss->s->devs[ss->dev].streams[0]);
+    return e == cudaSuccess ? cudaStreamWaitEvent(caller, ss->ev_out, 0) : e;
+}
+// host entries: whatever a device-resident entry left queued on the session's stream has finished (the session's device is current)
+cudaError_t session_wait(tinympc_cuda_session* ss) { return cudaStreamSynchronize(ss->s->devs[ss->dev].streams[0]); }
+
+// device entries: every array of `m` is 16-byte aligned device (or managed) memory of `device`, on top of check_model_arrays
+int check_device_models(tinympc_cuda_solver* s, const Family& f, const tinympc_cuda_models* m, int device, const char* what) {
+    if (int rc = check_model_arrays(s, f, m, true, what)) return rc;
+    ModelField mf[kModelFields];
+    model_fields(f.nx, f.nu, f.base.adaptive_rho != 0, mf);
+    for (int k = 0; k < kModelFields; ++k) {
+        const double* p = m->*mf[k].field;
+        if (p && !device_ptr_on(p, device))
+            return fail(s, TINYMPC_CUDA_EINVAL, std::string(what) + ": " + mf[k].name + " is not device memory of device " + std::to_string(device));
+    }
+    return TINYMPC_CUDA_OK;
+}
+
+// models (the tinympc_cuda_models layout, checked; host arrays, or device arrays with `device`) -> the session's resident copy,
+// then into every workspace's model block, Kinf, Pinf and rho.  The rest of each workspace stays as it is.  The host form copies
+// and waits; the device form copies device to device on the session's stream under the stream contract and does not wait.
+int session_upload_models(tinympc_cuda_session* ss, const tinympc_cuda_models* m, bool device = false, cudaStream_t caller = nullptr) {
     tinympc_cuda_solver* s = ss->s;
     DeviceCtx& d = s->devs[ss->dev];
     DeviceGuard guard;                       // restores the caller's current device on every return path
     CU(s, cudaSetDevice(d.device));
+    cudaStream_t st = d.streams[0];
+    if (!device) CU(s, session_wait(ss));
     ModelField mf[kModelFields];
     model_fields(ss->fam.nx, ss->fam.nu, ss->fam.base.adaptive_rho != 0, mf);
+    for (int k = 0; k < kModelFields; ++k)   // the buffers exist from the first upload of each field on
+        if (m->*mf[k].field) CU(s, ss->mdl[k].reserve(sizeof(double) * mf[k].per_problem * (size_t)ss->batch));
+    if (device) CU(s, session_begin(ss, caller));
     for (int k = 0; k < kModelFields; ++k) {
         const double* src = m->*mf[k].field;
         const size_t bytes = sizeof(double) * mf[k].per_problem * (size_t)ss->batch;
         if (src) {
-            CU(s, ss->mdl[k].reserve(bytes));
-            CU(s, cudaMemcpy(ss->mdl[k].p, src, bytes, cudaMemcpyHostToDevice));
+            if (device) CU(s, cudaMemcpyAsync(ss->mdl[k].p, src, bytes, cudaMemcpyDeviceToDevice, st));
+            else CU(s, cudaMemcpy(ss->mdl[k].p, src, bytes, cudaMemcpyHostToDevice));
         }
         ss->dm.*mf[k].field = src ? static_cast<const double*>(ss->mdl[k].p) : nullptr;
     }
-    cudaStream_t st = d.streams[0];
     const int adaptive = ss->fam.base.adaptive_rho != 0;
     CU(s, ss->bits == 64 ? wpp_session_models<double>(ss->W, ss->ws.p, ss->batch, ss->fam.nx, ss->fam.nu, ss->dm, adaptive, st)
                          : wpp_session_models<float>(ss->W, ss->ws.p, ss->batch, ss->fam.nx, ss->fam.nu, ss->dm, adaptive, st));
     s->launches += 1;
-    CU(s, cudaStreamSynchronize(st));
+    if (device) CU(s, session_end(ss, caller));
+    else CU(s, cudaStreamSynchronize(st));
     return TINYMPC_CUDA_OK;
 }
 
-int session_create_common(tinympc_cuda_solver* s, int dev_index, int batch, const tinympc_cuda_models* m, tinympc_cuda_session** out) {
+int session_create_common(tinympc_cuda_solver* s, int dev_index, int batch, const tinympc_cuda_models* m, tinympc_cuda_session** out,
+                          bool device = false, cudaStream_t caller = nullptr) {
     if (!s || !out) return TINYMPC_CUDA_EINVAL;
     *out = nullptr;
     if (!s->fam.set) return fail(s, TINYMPC_CUDA_ENOTREADY, "tinympc_cuda_set_family has not been called");
     if (dev_index < 0 || dev_index >= (int)s->devs.size()) return fail(s, TINYMPC_CUDA_EINVAL, "dev_index out of range");
     if (batch < 1) return fail(s, TINYMPC_CUDA_EINVAL, "session batch must be >= 1");
     if (!s->fam.shared_bounds_ok) return fail(s, TINYMPC_CUDA_EINVAL, "bound constraints are enabled but the family has no bounds");
-    if (m) if (int rc = check_model_arrays(s, s->fam, m, false, "model session")) return rc;
+    if (m && !device) if (int rc = check_model_arrays(s, s->fam, m, false, "model session")) return rc;
+    if (m && device) if (int rc = check_device_models(s, s->fam, m, s->devs[dev_index].device, "model session")) return rc;
     auto* ss = new tinympc_cuda_session();
     ss->s = s; ss->dev = dev_index; ss->batch = batch; ss->bits = s->precision;
     ss->fam = s->fam;
@@ -1739,6 +1780,8 @@ int session_create_common(tinympc_cuda_solver* s, int dev_index, int batch, cons
     auto bail = [&](cudaError_t e, const char* what) { cudaSetDevice(prev); tinympc_cuda_session_destroy(ss); return cuda_fail(s, e, what); };
     cudaError_t e = cudaSetDevice(d.device);
     if (e != cudaSuccess) return bail(e, "cudaSetDevice");
+    if ((e = cudaEventCreateWithFlags(&ss->ev_in, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "session event");
+    if ((e = cudaEventCreateWithFlags(&ss->ev_out, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "session event");
     const size_t esz = ss->bits == 64 ? sizeof(double) : sizeof(float);
     const size_t sx = (size_t)ss->fam.nx * ss->fam.N, su = (size_t)ss->fam.nu * (ss->fam.N - 1);
     if ((e = ss->ws.reserve((size_t)batch * ss->W.size * esz)) != cudaSuccess) return bail(e, "session workspace allocation");
@@ -1765,10 +1808,27 @@ int session_create_common(tinympc_cuda_solver* s, int dev_index, int batch, cons
     cudaSetDevice(prev);
     s->sessions.push_back(ss);
     if (m) {
-        if (int rc = session_upload_models(ss, m)) { tinympc_cuda_session_destroy(ss); return rc; }
+        if (int rc = session_upload_models(ss, m, device, caller)) { tinympc_cuda_session_destroy(ss); return rc; }
     }
     *out = ss;
     return TINYMPC_CUDA_OK;
+}
+
+// the workspace member (WppLayout offset) and width per solver of a session field: with `write` the fields the setters write, else
+// the fields session_read reads.  false for an unknown name.
+bool session_field(const tinympc_cuda_session* ss, const std::string& f, bool write, int* at, int* width) {
+    const WppLayout& W = ss->W;
+    const int nx = ss->fam.nx, nu = ss->fam.nu, N = ss->fam.N;
+    struct F { const char* name; int at, width; bool read, write; };
+    const F fields[] = {
+        {"x0", W.x, nx, true, true}, {"Xref", W.Xref, nx * N, false, true}, {"Uref", W.Uref, nu * (N - 1), false, true},
+        {"x", W.x, nx * N, true, false}, {"u", W.u, nu * (N - 1), true, false},
+        {"sol_x", W.vnew, nx * N, true, false}, {"sol_u", W.znew, nu * (N - 1), true, false},   // solution->x = work->vnew, admm.cpp:370, 386
+        {"rho", W.scalars + 0, 1, true, false}, {"iter", W.scalars + 1, 1, true, false}, {"status", W.scalars + 2, 1, true, false},
+        {"residuals", W.scalars + 3, 4, true, false}};
+    for (const F& x : fields)
+        if (f == x.name && (write ? x.write : x.read)) { *at = x.at; *width = x.width; return true; }
+    return false;
 }
 }  // namespace
 
@@ -1783,6 +1843,13 @@ int tinympc_cuda_session_create_models(tinympc_cuda_solver* s, int dev_index, in
     return session_create_common(s, dev_index, batch, m, out);
 }
 
+int tinympc_cuda_session_create_models_device(tinympc_cuda_solver* s, int dev_index, int batch, const tinympc_cuda_models* m, void* stream,
+                                              tinympc_cuda_session** out) {
+    if (out) *out = nullptr;
+    if (!m) return s ? fail(s, TINYMPC_CUDA_EINVAL, "model session: models is NULL") : TINYMPC_CUDA_EINVAL;
+    return session_create_common(s, dev_index, batch, m, out, true, static_cast<cudaStream_t>(stream));
+}
+
 int tinympc_cuda_session_set_models(tinympc_cuda_session* ss, const tinympc_cuda_models* m) {
     if (!ss) return TINYMPC_CUDA_EINVAL;
     tinympc_cuda_solver* s = ss->s;
@@ -1793,14 +1860,26 @@ int tinympc_cuda_session_set_models(tinympc_cuda_session* ss, const tinympc_cuda
     return session_upload_models(ss, m);
 }
 
+int tinympc_cuda_session_set_models_device(tinympc_cuda_session* ss, const tinympc_cuda_models* m, void* stream) {
+    if (!ss) return TINYMPC_CUDA_EINVAL;
+    tinympc_cuda_solver* s = ss->s;
+    if (!s) return TINYMPC_CUDA_ENOTREADY;   // the solver was destroyed under the session
+    if (!m) return fail(s, TINYMPC_CUDA_EINVAL, "model session: models is NULL");
+    if (!ss->models) return fail(s, TINYMPC_CUDA_EINVAL, "set_models needs a session created with models (tinympc_cuda_session_create_models)");
+    if (int rc = check_device_models(s, ss->fam, m, s->devs[ss->dev].device, "model session")) return rc;
+    return session_upload_models(ss, m, true, static_cast<cudaStream_t>(stream));
+}
+
 int tinympc_cuda_session_destroy(tinympc_cuda_session* ss) {
     if (!ss) return TINYMPC_CUDA_OK;
     if (ss->s) {   // (an orphan's buffers went with its solver)
         int prev = 0;
         cudaGetDevice(&prev);
         cudaSetDevice(ss->s->devs[ss->dev].device);
+        if (ss->ev_in) session_wait(ss);     // (a session that failed in creation may have no events and nothing queued)
         for (DevBuf* b : {&ss->ws, &ss->pack, &ss->x, &ss->u, &ss->iter, &ss->status}) b->release();
         for (DevBuf& b : ss->mdl) b.release();
+        for (cudaEvent_t ev : {ss->ev_in, ss->ev_out}) if (ev) cudaEventDestroy(ev);
         cudaSetDevice(prev);
         auto& v = ss->s->sessions;
         v.erase(std::remove(v.begin(), v.end(), ss), v.end());
@@ -1825,6 +1904,7 @@ int session_scatter(tinympc_cuda_session* ss, int at, int width, const double* s
     int prev = 0;
     cudaGetDevice(&prev);
     CU(s, cudaSetDevice(s->devs[ss->dev].device));
+    CU(s, session_wait(ss));
     CU(s, cudaMemcpy2D(static_cast<char*>(ss->ws.p) + (size_t)at * esz, (size_t)ss->W.size * esz, ss->stage.data(), (size_t)width * esz,
                        (size_t)width * esz, ss->batch, cudaMemcpyHostToDevice));
     cudaSetDevice(prev);
@@ -1839,6 +1919,7 @@ int session_gather(tinympc_cuda_session* ss, int at, int width, double* dst) {
     int prev = 0;
     cudaGetDevice(&prev);
     CU(s, cudaSetDevice(s->devs[ss->dev].device));
+    CU(s, session_wait(ss));
     CU(s, cudaMemcpy2D(ss->stage.data(), (size_t)width * esz, static_cast<char*>(ss->ws.p) + (size_t)at * esz, (size_t)ss->W.size * esz,
                        (size_t)width * esz, ss->batch, cudaMemcpyDeviceToHost));
     cudaSetDevice(prev);
@@ -1933,19 +2014,46 @@ int tinympc_cuda_session_step(tinympc_cuda_session* ss, int use_solution) {
 int tinympc_cuda_session_read(tinympc_cuda_session* ss, const char* field, double* host) {
     if (!ss || !field || !host) return TINYMPC_CUDA_EINVAL;
     if (!ss->s) return TINYMPC_CUDA_ENOTREADY;
-    const std::string f(field);
-    const WppLayout& W = ss->W;
-    const int nx = ss->fam.nx, nu = ss->fam.nu, N = ss->fam.N;
-    if (f == "x0") return session_gather(ss, W.x, nx, host);
-    if (f == "x") return session_gather(ss, W.x, nx * N, host);
-    if (f == "u") return session_gather(ss, W.u, nu * (N - 1), host);
-    if (f == "sol_x") return session_gather(ss, W.vnew, nx * N, host);       // solution->x = work->vnew, admm.cpp:370, 386
-    if (f == "sol_u") return session_gather(ss, W.znew, nu * (N - 1), host);
-    if (f == "rho") return session_gather(ss, W.scalars + 0, 1, host);
-    if (f == "iter") return session_gather(ss, W.scalars + 1, 1, host);
-    if (f == "status") return session_gather(ss, W.scalars + 2, 1, host);
-    if (f == "residuals") return session_gather(ss, W.scalars + 3, 4, host);
-    return fail(ss->s, TINYMPC_CUDA_EINVAL, "unknown session field " + f);
+    int at = 0, width = 0;
+    if (!session_field(ss, field, false, &at, &width)) return fail(ss->s, TINYMPC_CUDA_EINVAL, std::string("unknown session field ") + field);
+    return session_gather(ss, at, width, host);
+}
+
+namespace {
+// the two device-resident I/O entries: `p` (16-byte aligned device memory of the session's device), a packed [batch][width] array of
+// doubles (or one row, write with broadcast) <-> member `at` of every workspace, under the stream contract
+int session_io_device(tinympc_cuda_session* ss, const char* field, bool write, const double* src, double* dst, int broadcast, void* stream) {
+    if (!ss || !field) return TINYMPC_CUDA_EINVAL;
+    tinympc_cuda_solver* s = ss->s;
+    if (!s) return TINYMPC_CUDA_ENOTREADY;   // the solver was destroyed under the session
+    DeviceCtx& d = s->devs[ss->dev];
+    int at = 0, width = 0;
+    if (!session_field(ss, field, write, &at, &width))
+        return fail(s, TINYMPC_CUDA_EINVAL, std::string("unknown session field for ") + (write ? "write_device: " : "read_device: ") + field);
+    const void* p = write ? static_cast<const void*>(src) : static_cast<const void*>(dst);
+    if (!p || !device_ptr_on(p, d.device))
+        return fail(s, TINYMPC_CUDA_EINVAL, std::string(field) + ": the array must be 16-byte aligned device memory of device " + std::to_string(d.device));
+    const cudaStream_t caller = static_cast<cudaStream_t>(stream);
+    DeviceGuard guard;                       // restores the caller's current device on every return path
+    CU(s, cudaSetDevice(d.device));
+    CU(s, session_begin(ss, caller));
+    if (write)
+        CU(s, ss->bits == 64 ? wpp_session_scatter<double>(ss->W, ss->ws.p, ss->batch, at, width, src, broadcast != 0, d.streams[0])
+                             : wpp_session_scatter<float>(ss->W, ss->ws.p, ss->batch, at, width, src, broadcast != 0, d.streams[0]));
+    else
+        CU(s, ss->bits == 64 ? wpp_session_gather<double>(ss->W, ss->ws.p, ss->batch, at, width, dst, d.streams[0])
+                             : wpp_session_gather<float>(ss->W, ss->ws.p, ss->batch, at, width, dst, d.streams[0]));
+    s->launches += 1;
+    CU(s, session_end(ss, caller));
+    return TINYMPC_CUDA_OK;
+}
+}  // namespace
+
+int tinympc_cuda_session_write_device(tinympc_cuda_session* ss, const char* field, const double* src, int broadcast, void* stream) {
+    return session_io_device(ss, field, true, src, nullptr, broadcast, stream);
+}
+int tinympc_cuda_session_read_device(tinympc_cuda_session* ss, const char* field, double* dst, void* stream) {
+    return session_io_device(ss, field, false, nullptr, dst, 0, stream);
 }
 
 int tinympc_cuda_set_option(tinympc_cuda_solver* s, const char* name, double value) {

@@ -12,6 +12,7 @@
 #include <algorithm>
 
 #include "../../include/tinympc_b200.h"
+#include "tmpc_devptr.h"
 
 namespace {
 
@@ -21,8 +22,8 @@ constexpr int kMaxNx = 16, kMaxNu = 8;
 struct PreParams {
     int batch, nx, nu, max_iter, want_sens;
     double tol, h;
-    const double *A, *B, *f, *Q, *R, *rho;           // per problem: nx*nx, nx*nu (row-major), nx, nx (diagonal), nu (diagonal), 1
-    double *Kinf, *Pinf, *Quu_inv, *AmBKt, *APf, *BPf;   // per problem, row-major
+    const double *A, *B, *f, *Q, *R, *rho;           // per problem: nx*nx, nx*nu (column-major), nx, nx (diagonal), nu (diagonal), 1
+    double *Kinf, *Pinf, *Quu_inv, *AmBKt, *APf, *BPf;   // per problem, column-major (the tinympc_cuda_models layout)
     double *dKinf, *dPinf, *dC1, *dC2;                // per problem or NULL
     int* iters;                                       // per problem or NULL: Riccati iterations used
 };
@@ -128,6 +129,19 @@ __device__ int riccati(const WarpMem& m, int nx, int nu, double rho, const doubl
     return it;
 }
 
+// Between the column-major arrays of one problem in global memory (element e = row e % rows, column e / rows) and the row-major
+// matrices the recursion keeps in shared memory; lanes walk the global side contiguously.
+__device__ __forceinline__ void load_cm(double* S, const double* G, int rows, int cols, int lane) {
+    for (int e = lane; e < rows * cols; e += 32) S[(e % rows) * cols + e / rows] = G[e];
+}
+__device__ __forceinline__ void store_cm(double* G, const double* S, int rows, int cols, int lane) {
+    for (int e = lane; e < rows * cols; e += 32) G[e] = S[(e % rows) * cols + e / rows];
+}
+// G <- (S - G) / h, the forward difference of the sensitivities over the base point G holds
+__device__ __forceinline__ void diff_cm(double* G, const double* S, int rows, int cols, double ih, int lane) {
+    for (int e = lane; e < rows * cols; e += 32) G[e] = (S[(e % rows) * cols + e / rows] - G[e]) * ih;
+}
+
 __global__ void __launch_bounds__(128) precompute_kernel(const PreParams p) {
     extern __shared__ __align__(16) double pre_smem[];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -135,8 +149,8 @@ __global__ void __launch_bounds__(128) precompute_kernel(const PreParams p) {
     const WarpMem m(pre_smem + (size_t)wib * WarpMem::size(nx, nu), nx, nu);
     const int nwarps = (gridDim.x * blockDim.x) >> 5;
     for (int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; b < p.batch; b += nwarps) {
-        for (int e = lane; e < nx * nx; e += 32) m.A[e] = p.A[(size_t)b * nx * nx + e];
-        for (int e = lane; e < nx * nu; e += 32) m.B[e] = p.B[(size_t)b * nx * nu + e];
+        load_cm(m.A, p.A + (size_t)b * nx * nx, nx, nx, lane);
+        load_cm(m.B, p.B + (size_t)b * nx * nu, nx, nu, lane);
         for (int e = lane; e < nx; e += 32) m.f[e] = p.f ? p.f[(size_t)b * nx + e] : 0.0;
         __syncwarp();
         const double rho = p.rho[b];
@@ -146,9 +160,10 @@ __global__ void __launch_bounds__(128) precompute_kernel(const PreParams p) {
         if (p.iters && lane == 0) p.iters[b] = it;
         double* oK = p.Kinf + (size_t)b * nu * nx; double* oP = p.Pinf + (size_t)b * nx * nx;
         double* oQ = p.Quu_inv + (size_t)b * nu * nu; double* oA = p.AmBKt + (size_t)b * nx * nx;
-        for (int e = lane; e < nu * nx; e += 32) oK[e] = m.K[e];
-        for (int e = lane; e < nx * nx; e += 32) { oP[e] = m.Pn[e]; oA[e] = m.M[(e % nx) * nx + e / nx]; }     // AmBKt = (A - B K)'
-        for (int e = lane; e < nu * nu; e += 32) oQ[e] = m.Gi[e];
+        store_cm(oK, m.K, nu, nx, lane);
+        store_cm(oP, m.Pn, nx, nx, lane);
+        for (int e = lane; e < nx * nx; e += 32) oA[e] = m.M[e];     // AmBKt = (A - B K)': column-major AmBKt is row-major A - B K
+        store_cm(oQ, m.Gi, nu, nu, lane);
         // APf = AmBKt Pinf f, BPf = B' Pinf f   (tiny_api.cpp:290-291)
         for (int r = lane; r < nx; r += 32) { double acc = 0; for (int c = 0; c < nx; ++c) acc = fma(m.Pn[r * nx + c], m.f[c], acc); m.T3[r] = acc; }
         __syncwarp();
@@ -162,15 +177,17 @@ __global__ void __launch_bounds__(128) precompute_kernel(const PreParams p) {
             double* dK = p.dKinf + (size_t)b * nu * nx; double* dP = p.dPinf + (size_t)b * nx * nx;
             double* d1 = p.dC1 ? p.dC1 + (size_t)b * nu * nu : nullptr; double* d2 = p.dC2 ? p.dC2 + (size_t)b * nx * nx : nullptr;
             riccati(m, nx, nu, rho, Qd, Rd, 5000, 1e-10, lane);
-            for (int e = lane; e < nu * nx; e += 32) dK[e] = m.K[e];
-            for (int e = lane; e < nx * nx; e += 32) { dP[e] = m.Pn[e]; if (d2) d2[e] = m.M[(e % nx) * nx + e / nx]; }
-            for (int e = lane; e < nu * nu; e += 32) if (d1) d1[e] = m.Gi[e];
+            store_cm(dK, m.K, nu, nx, lane);
+            store_cm(dP, m.Pn, nx, nx, lane);
+            if (d2) for (int e = lane; e < nx * nx; e += 32) d2[e] = m.M[e];
+            if (d1) store_cm(d1, m.Gi, nu, nu, lane);
             __syncwarp();
             riccati(m, nx, nu, rho + p.h, Qd, Rd, 5000, 1e-10, lane);
             const double ih = 1.0 / p.h;
-            for (int e = lane; e < nu * nx; e += 32) dK[e] = (m.K[e] - dK[e]) * ih;
-            for (int e = lane; e < nx * nx; e += 32) { dP[e] = (m.Pn[e] - dP[e]) * ih; if (d2) d2[e] = (m.M[(e % nx) * nx + e / nx] - d2[e]) * ih; }
-            for (int e = lane; e < nu * nu; e += 32) if (d1) d1[e] = (m.Gi[e] - d1[e]) * ih;
+            diff_cm(dK, m.K, nu, nx, ih, lane);
+            diff_cm(dP, m.Pn, nx, nx, ih, lane);
+            if (d2) for (int e = lane; e < nx * nx; e += 32) d2[e] = (m.M[e] - d2[e]) * ih;
+            if (d1) diff_cm(d1, m.Gi, nu, nu, ih, lane);
             __syncwarp();
         }
     }
@@ -186,38 +203,56 @@ struct Dev {
     ~Dev() { if (p) cudaFree(p); }
 };
 
+// shape and required arrays, the same for both entries
+int check_args(const tinympc_cuda_precompute_in* in, const tinympc_cuda_precompute_out* out) {
+    if (!in || !out) return TINYMPC_CUDA_EINVAL;
+    if (in->batch < 0 || in->nx < 1 || in->nu < 1 || in->nx > kMaxNx || in->nu > kMaxNu) return TINYMPC_CUDA_EINVAL;
+    if (in->batch == 0) return TINYMPC_CUDA_OK;
+    if (!in->Adyn || !in->Bdyn || !in->Q || !in->R || !in->rho) return TINYMPC_CUDA_EINVAL;
+    if (!out->Kinf || !out->Pinf || !out->Quu_inv || !out->AmBKt || !out->APf || !out->BPf) return TINYMPC_CUDA_EINVAL;
+    return TINYMPC_CUDA_OK;
+}
+
+PreParams params_of(const tinympc_cuda_precompute_in* in, const tinympc_cuda_precompute_out* out) {
+    PreParams p{};
+    p.batch = in->batch; p.nx = in->nx; p.nu = in->nu; p.max_iter = 1000; p.tol = 1e-5; p.h = 1e-6;
+    p.want_sens = out->dKinf_drho && out->dPinf_drho ? 1 : 0;
+    p.A = in->Adyn; p.B = in->Bdyn; p.f = in->fdyn; p.Q = in->Q; p.R = in->R; p.rho = in->rho;
+    p.Kinf = out->Kinf; p.Pinf = out->Pinf; p.Quu_inv = out->Quu_inv; p.AmBKt = out->AmBKt; p.APf = out->APf; p.BPf = out->BPf;
+    if (p.want_sens) { p.dKinf = out->dKinf_drho; p.dPinf = out->dPinf_drho; p.dC1 = out->dC1_drho; p.dC2 = out->dC2_drho; }
+    p.iters = out->iters;
+    return p;
+}
+
+// the kernel on `stream` over device arrays (p's pointers); no allocation, copy or synchronisation
+cudaError_t enqueue(const PreParams& p, cudaStream_t stream) {
+    const int warps_per_cta = 4;
+    const size_t smem = sizeof(double) * WarpMem::size(p.nx, p.nu) * warps_per_cta;
+    cudaError_t e = cudaFuncSetAttribute(precompute_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    int sms = 0, dev = 0;
+    if (e == cudaSuccess) e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (e != cudaSuccess) return e;
+    const int grid = std::max(1, std::min((p.batch + warps_per_cta - 1) / warps_per_cta, sms * 4));
+    precompute_kernel<<<grid, warps_per_cta * 32, smem, stream>>>(p);
+    return cudaGetLastError();
+}
+
 }  // namespace
 
 extern "C" int tinympc_cuda_precompute_batch(const tinympc_cuda_precompute_in* in, const tinympc_cuda_precompute_out* out) {
-    if (!in || !out) return TINYMPC_CUDA_EINVAL;
+    if (int rc = check_args(in, out)) return rc;
     const int B = in->batch, nx = in->nx, nu = in->nu;
-    if (B < 0 || nx < 1 || nu < 1 || nx > kMaxNx || nu > kMaxNu) return TINYMPC_CUDA_EINVAL;
     if (B == 0) return TINYMPC_CUDA_OK;
-    if (!in->Adyn || !in->Bdyn || !in->Q || !in->R || !in->rho) return TINYMPC_CUDA_EINVAL;
-    if (!out->Kinf || !out->Pinf || !out->Quu_inv || !out->AmBKt || !out->APf || !out->BPf) return TINYMPC_CUDA_EINVAL;
-    const bool sens = out->dKinf_drho && out->dPinf_drho;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) { cudaGetLastError(); return TINYMPC_CUDA_ENODEVICE; }
     const size_t nxx = (size_t)nx * nx, nxu = (size_t)nx * nu, nuu = (size_t)nu * nu;
-    // host arrays are column-major per problem (the reference's Eigen layout); the kernel works row-major: transpose on the way
-    auto to_rowmajor = [&](const double* src, int rows, int cols, double* dst) {
-        for (int b = 0; b < B; ++b)
-            for (int r = 0; r < rows; ++r)
-                for (int c = 0; c < cols; ++c) dst[(size_t)b * rows * cols + r * cols + c] = src[(size_t)b * rows * cols + (size_t)c * rows + r];
-    };
-    auto to_colmajor = [&](const double* src, int rows, int cols, double* dst) {
-        for (int b = 0; b < B; ++b)
-            for (int r = 0; r < rows; ++r)
-                for (int c = 0; c < cols; ++c) dst[(size_t)b * rows * cols + (size_t)c * rows + r] = src[(size_t)b * rows * cols + r * cols + c];
-    };
-    double* hA = new double[B * nxx]; double* hB = new double[B * nxu];
-    to_rowmajor(in->Adyn, nx, nx, hA);
-    to_rowmajor(in->Bdyn, nx, nu, hB);
+    const bool sens = out->dKinf_drho && out->dPinf_drho;
+    // the kernel reads and writes the host entry's column-major layout as it is: upload, kernel, download
     Dev dA, dB, df, dQ, dR, drho, oK, oP, oQ, oA, oAPf, oBPf, sK, sP, s1, s2, dit;
     cudaError_t e = cudaSuccess;
     auto ok = [&](cudaError_t r) { if (e == cudaSuccess) e = r; };
-    ok(dA.put(hA, sizeof(double) * B * nxx)); ok(dB.put(hB, sizeof(double) * B * nxu));
-    delete[] hA; delete[] hB;
+    ok(dA.put(in->Adyn, sizeof(double) * B * nxx)); ok(dB.put(in->Bdyn, sizeof(double) * B * nxu));
     if (in->fdyn) ok(df.put(in->fdyn, sizeof(double) * B * nx));
     ok(dQ.put(in->Q, sizeof(double) * B * nx)); ok(dR.put(in->R, sizeof(double) * B * nu)); ok(drho.put(in->rho, sizeof(double) * B));
     ok(oK.put(nullptr, sizeof(double) * B * nxu)); ok(oP.put(nullptr, sizeof(double) * B * nxx)); ok(oQ.put(nullptr, sizeof(double) * B * nuu));
@@ -225,41 +260,41 @@ extern "C" int tinympc_cuda_precompute_batch(const tinympc_cuda_precompute_in* i
     ok(dit.put(nullptr, sizeof(int) * B));
     if (sens) {
         ok(sK.put(nullptr, sizeof(double) * B * nxu)); ok(sP.put(nullptr, sizeof(double) * B * nxx));
-        ok(s1.put(nullptr, sizeof(double) * B * nuu)); ok(s2.put(nullptr, sizeof(double) * B * nxx));
+        if (out->dC1_drho) ok(s1.put(nullptr, sizeof(double) * B * nuu));
+        if (out->dC2_drho) ok(s2.put(nullptr, sizeof(double) * B * nxx));
     }
     if (e != cudaSuccess) return TINYMPC_CUDA_ECUDA;
-    PreParams p{};
-    p.batch = B; p.nx = nx; p.nu = nu; p.max_iter = 1000; p.tol = 1e-5; p.h = 1e-6; p.want_sens = sens ? 1 : 0;
-    p.A = (const double*)dA.p; p.B = (const double*)dB.p; p.f = (const double*)df.p; p.Q = (const double*)dQ.p; p.R = (const double*)dR.p;
-    p.rho = (const double*)drho.p;
-    p.Kinf = (double*)oK.p; p.Pinf = (double*)oP.p; p.Quu_inv = (double*)oQ.p; p.AmBKt = (double*)oA.p; p.APf = (double*)oAPf.p; p.BPf = (double*)oBPf.p;
-    p.dKinf = (double*)sK.p; p.dPinf = (double*)sP.p; p.dC1 = (double*)s1.p; p.dC2 = (double*)s2.p; p.iters = (int*)dit.p;
-    const int warps_per_cta = 4;
-    const size_t smem = sizeof(double) * WarpMem::size(nx, nu) * warps_per_cta;
-    cudaFuncSetAttribute(precompute_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    int sms = 0;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int grid = std::max(1, std::min((B + warps_per_cta - 1) / warps_per_cta, sms * 4));
-    precompute_kernel<<<grid, warps_per_cta * 32, smem>>>(p);
-    ok(cudaGetLastError());
+    const tinympc_cuda_precompute_in din{B, nx, nu, (const double*)dA.p, (const double*)dB.p, (const double*)df.p, (const double*)dQ.p,
+                                         (const double*)dR.p, (const double*)drho.p};
+    const tinympc_cuda_precompute_out dout{(double*)oK.p, (double*)oP.p, (double*)oQ.p, (double*)oA.p, (double*)oAPf.p, (double*)oBPf.p,
+                                           (double*)sK.p, (double*)sP.p, (double*)s1.p, (double*)s2.p, (int*)dit.p};
+    ok(enqueue(params_of(&din, &dout), nullptr));
     ok(cudaDeviceSynchronize());
     if (e != cudaSuccess) return TINYMPC_CUDA_ECUDA;
-    // back to the host, column-major per problem; the staging buffer holds the largest block fetched (nu x nx or nu x nu when nu > nx)
-    double* h = new double[B * std::max({nxx, nxu, nuu})];
-    auto fetch = [&](const Dev& d, double* dst, int rows, int cols) {
-        if (!dst) return;
-        ok(cudaMemcpy(h, d.p, sizeof(double) * B * rows * cols, cudaMemcpyDeviceToHost));
-        to_colmajor(h, rows, cols, dst);
-    };
-    fetch(oK, out->Kinf, nu, nx); fetch(oP, out->Pinf, nx, nx); fetch(oQ, out->Quu_inv, nu, nu); fetch(oA, out->AmBKt, nx, nx);
-    ok(cudaMemcpy(out->APf, oAPf.p, sizeof(double) * B * nx, cudaMemcpyDeviceToHost));
-    ok(cudaMemcpy(out->BPf, oBPf.p, sizeof(double) * B * nu, cudaMemcpyDeviceToHost));
-    if (out->iters) ok(cudaMemcpy(out->iters, dit.p, sizeof(int) * B, cudaMemcpyDeviceToHost));
+    auto fetch = [&](const Dev& d, void* dst, size_t bytes) { if (dst) ok(cudaMemcpy(dst, d.p, bytes, cudaMemcpyDeviceToHost)); };
+    fetch(oK, out->Kinf, sizeof(double) * B * nxu); fetch(oP, out->Pinf, sizeof(double) * B * nxx);
+    fetch(oQ, out->Quu_inv, sizeof(double) * B * nuu); fetch(oA, out->AmBKt, sizeof(double) * B * nxx);
+    fetch(oAPf, out->APf, sizeof(double) * B * nx); fetch(oBPf, out->BPf, sizeof(double) * B * nu);
+    fetch(dit, out->iters, sizeof(int) * B);
     if (sens) {
-        fetch(sK, out->dKinf_drho, nu, nx); fetch(sP, out->dPinf_drho, nx, nx); fetch(s1, out->dC1_drho, nu, nu); fetch(s2, out->dC2_drho, nx, nx);
+        fetch(sK, out->dKinf_drho, sizeof(double) * B * nxu); fetch(sP, out->dPinf_drho, sizeof(double) * B * nxx);
+        fetch(s1, out->dC1_drho, sizeof(double) * B * nuu); fetch(s2, out->dC2_drho, sizeof(double) * B * nxx);
     }
-    delete[] h;
     return e == cudaSuccess ? TINYMPC_CUDA_OK : TINYMPC_CUDA_ECUDA;
+}
+
+extern "C" int tinympc_cuda_precompute_batch_device(const tinympc_cuda_precompute_in* in, const tinympc_cuda_precompute_out* out,
+                                                    void* stream) {
+    if (int rc = check_args(in, out)) return rc;
+    if (in->batch == 0) return TINYMPC_CUDA_OK;
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) { cudaGetLastError(); return TINYMPC_CUDA_ENODEVICE; }
+    const PreParams p = params_of(in, out);
+    // every array the kernel will touch: 16-byte aligned device memory of the current device
+    for (const void* a : {(const void*)p.A, (const void*)p.B, (const void*)p.f, (const void*)p.Q, (const void*)p.R, (const void*)p.rho,
+                          (const void*)p.Kinf, (const void*)p.Pinf, (const void*)p.Quu_inv, (const void*)p.AmBKt, (const void*)p.APf,
+                          (const void*)p.BPf, (const void*)p.dKinf, (const void*)p.dPinf, (const void*)p.dC1, (const void*)p.dC2,
+                          (const void*)p.iters})
+        if (a && !tmpc::device_ptr_on(a, dev)) return TINYMPC_CUDA_EINVAL;
+    return enqueue(p, static_cast<cudaStream_t>(stream)) == cudaSuccess ? TINYMPC_CUDA_OK : TINYMPC_CUDA_ECUDA;
 }

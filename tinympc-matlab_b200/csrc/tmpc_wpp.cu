@@ -186,6 +186,25 @@ __global__ void wpp_session_step_models_kernel(const WppLayout W, T* __restrict_
     if (lane < nx) ws[W.x + lane] = xn;
 }
 
+// packed doubles [batch][width] (or ONE broadcast row) -> member `at` of every workspace, converted to T (the device form of the
+// host session setters' conversion loop)
+template <typename T>
+__global__ void wpp_session_scatter_kernel(const WppLayout W, T* __restrict__ wsp, int batch, int at, int width, const double* __restrict__ src,
+                                           int broadcast) {
+    for (size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x; k < (size_t)batch * width; k += (size_t)gridDim.x * blockDim.x) {
+        const size_t b = k / width, e = k - b * width;
+        wsp[b * W.size + at + e] = static_cast<T>(src[broadcast ? e : k]);
+    }
+}
+// member `at` of every workspace -> packed doubles [batch][width] (the device form of session_read's conversion loop)
+template <typename T>
+__global__ void wpp_session_gather_kernel(const WppLayout W, const T* __restrict__ wsp, int batch, int at, int width, double* __restrict__ dst) {
+    for (size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x; k < (size_t)batch * width; k += (size_t)gridDim.x * blockDim.x) {
+        const size_t b = k / width, e = k - b * width;
+        dst[k] = static_cast<double>(wsp[b * W.size + at + e]);
+    }
+}
+
 template <typename T>
 cudaError_t wpp_session_models(const WppLayout& W, void* wsp, int batch, int nx, int nu, const tinympc_cuda_models& m, int adaptive,
                                cudaStream_t st) {
@@ -202,6 +221,21 @@ template cudaError_t wpp_session_models<float>(const WppLayout&, void*, int, int
 template cudaError_t wpp_session_models<double>(const WppLayout&, void*, int, int, int, const tinympc_cuda_models&, int, cudaStream_t);
 template cudaError_t wpp_session_step_models<float>(const WppLayout&, void*, int, int, int, int, cudaStream_t);
 template cudaError_t wpp_session_step_models<double>(const WppLayout&, void*, int, int, int, int, cudaStream_t);
+
+template <typename T>
+cudaError_t wpp_session_scatter(const WppLayout& W, void* wsp, int batch, int at, int width, const double* src, int broadcast, cudaStream_t st) {
+    wpp_session_scatter_kernel<T><<<592, 256, 0, st>>>(W, static_cast<T*>(wsp), batch, at, width, src, broadcast);
+    return cudaGetLastError();
+}
+template <typename T>
+cudaError_t wpp_session_gather(const WppLayout& W, const void* wsp, int batch, int at, int width, double* dst, cudaStream_t st) {
+    wpp_session_gather_kernel<T><<<592, 256, 0, st>>>(W, static_cast<const T*>(wsp), batch, at, width, dst);
+    return cudaGetLastError();
+}
+template cudaError_t wpp_session_scatter<float>(const WppLayout&, void*, int, int, int, const double*, int, cudaStream_t);
+template cudaError_t wpp_session_scatter<double>(const WppLayout&, void*, int, int, int, const double*, int, cudaStream_t);
+template cudaError_t wpp_session_gather<float>(const WppLayout&, const void*, int, int, int, double*, cudaStream_t);
+template cudaError_t wpp_session_gather<double>(const WppLayout&, const void*, int, int, int, double*, cudaStream_t);
 
 template <typename T>
 cudaError_t wpp_session_init(const SolveParams& p, const PackLayout& L, const void* pack, const WppLayout& W, void* wsp, int batch, cudaStream_t st) {

@@ -59,4 +59,11 @@ cudaError_t wpp_session_models(const WppLayout& W, void* wsp, int batch, int nx,
 template <typename T>
 cudaError_t wpp_session_step_models(const WppLayout& W, void* wsp, int batch, int nx, int nu, int use_solution, cudaStream_t st);
 
+// device-resident session I/O: packed doubles [batch][width] (src: or one row shared by all, broadcast 1) <-> member `at` (a WppLayout
+// offset) of every workspace, in the workspace's type T
+template <typename T>
+cudaError_t wpp_session_scatter(const WppLayout& W, void* wsp, int batch, int at, int width, const double* src, int broadcast, cudaStream_t st);
+template <typename T>
+cudaError_t wpp_session_gather(const WppLayout& W, const void* wsp, int batch, int at, int width, double* dst, cudaStream_t st);
+
 }  // namespace tmpc
